@@ -2,6 +2,7 @@
 """bench.py -- RAFT correlation hot path: build + 12-iteration lookup, frame pairs/s at 1920x1088.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--volume-dtype fp32|bf16]
+                    [--dump-outputs DIR]
 
 One "step" = one synthetic frame pair (BASELINE.json configs[1]): correlation volume + 4-level
 pyramid from two (1, 256, 136, 240) feature maps, then 12 radius-4 lookups with drifting
@@ -23,6 +24,11 @@ coordinates.  Prints ONE JSON line (rank 0).  See DESIGN.md section "Measurement
 --impl reference times the reference's own CPU implementation as its own arm (rank 0 only): every step is one FULL
 1920x1088 pair through torchvision's CorrBlock.build_pyramid + 12 x index_pyramid, warm-up included.
 No number here is taken under a profiler.
+
+--dump-outputs DIR (ours, rank 0) writes what the timed loop computed in its last step, as float32 .npy files, so that
+two builds can be compared output for output (the inputs are seeded, identical from run to run):
+  lookup.npy            the last of the step's 12 lookups, (1, 324, 136, 240), in full
+  pyramid_level<l>.npy  the pyramid rows of DUMP_ROWS query pixels drawn with a fixed seed, (DUMP_ROWS, 1, h_l, w_l)
 """
 from __future__ import annotations
 
@@ -47,6 +53,7 @@ N = H8 * W8
 RING = 4                                   # distinct input sets rotated through (268 MB > 126 MB L2)
 WORKLOAD = ("1 frame pair 1920x1088 per step per GPU: corr volume + 4-level pyramid + 12 radius-4 lookups "
             "(BASELINE.json configs[1])")
+DUMP_ROWS = 64                             # --dump-outputs: 42.3 MB of lookup + 11.1 MB of pyramid rows
 
 
 # ----------------------------------------------------------------------------- workload maths
@@ -215,6 +222,19 @@ def run_reference(args):
 
 
 # ----------------------------------------------------------------------------- our arm
+def dump_outputs(out_dir: str, pyr, lookup):
+    """Write the last step's lookup and a fixed sample of its pyramid (see --dump-outputs) as float32 .npy."""
+    import numpy as np
+    import torch
+    os.makedirs(out_dir, exist_ok=True)
+    rows = torch.randperm(B * N, generator=torch.Generator().manual_seed(0))[:DUMP_ROWS].sort().values
+    arrays = {"lookup": lookup}
+    for l in range(LEVELS):
+        arrays[f"pyramid_level{l}"] = pyr.level(l, rows.to(lookup.device))
+    for name, t in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), t.float().cpu().numpy())
+
+
 def run_ours(args):
     import numpy as np
     import torch
@@ -290,6 +310,8 @@ def run_ours(args):
     launches = lib.rdvc_corr_launch_count() - launches0
     build_ms = [a.elapsed_time(b_) for a, b_, _ in kev]
     lookup_ms = [b_.elapsed_time(c_) for _, b_, c_ in kev]
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, blk._pyr, out)
 
     # ---- the same timed loop with the other pyramid storage type (reported beside the headline: the
     # reference's own GPU default is an fp16 volume under autocast, R:codec_processing.py:1436)
@@ -489,7 +511,11 @@ def main():
     ap.add_argument("--no-gop", action="store_true", help="skip the GOP-sharded motion-branch run (configs 3 / 4)")
     ap.add_argument("--gop-frames", type=int, default=600, help="frames of the GOP-sharded run (config 4: 600)")
     ap.add_argument("--gop-fp32", action="store_true", help="run the GOP-sharded RAFT in fp32 / TF32 instead of fp16 autocast")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the last timed step's lookup and a fixed sample of its pyramid to DIR as .npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs dumps the CUDA path: use it with --impl ours")
     if args.warmup < 3 and args.impl == "ours":
         args.warmup = 3   # timing rule: at least 3 warm-up steps
     return run_reference(args) if args.impl == "reference" else run_ours(args)
