@@ -99,6 +99,10 @@ def run_sharded(args, own_process_group=True):
     torch.manual_seed(0)
     vol = torch.float32 if args.volume == "fp32" else torch.bfloat16
     model = raft_large(weights=None, corr_block=rc.TVCorrBlock(volume_dtype=vol)).eval().to(dev)
+    if getattr(args, "b200_recurrent_block", False):      # same weights, the SepConvGRU as this library's kernels
+        rb = rc.RecurrentBlock(input_size=256, hidden_size=model.update_block.recurrent_block.hidden_size)
+        rb.load_state_dict(model.update_block.recurrent_block.state_dict())
+        model.update_block.recurrent_block = rb.to(dev)
     h, w = args.height, args.width
     g = torch.Generator(device=dev).manual_seed(0)
     base = torch.rand(1, 3, h // 16 + 8, w // 16 + 8, device=dev, generator=g)
@@ -310,6 +314,8 @@ def run_sharded(args, own_process_group=True):
             "rank0_p_frames_per_s": (sum(1 for t in spans[0] if not gs.is_iframe(t, args.gop)) if by_frames
                                      else sum(g_.num_pframes for g_ in mine)) / max(t_local, 1e-9),
         }
+        if getattr(args, "b200_recurrent_block", False):
+            line["config"]["b200_recurrent_block"] = True
         # flow end-point error of this configuration against STOCK torchvision RAFT (same weights, same autocast
         # setting) on one frame pair of the sequence -- outside the timed region
         a, b = frame_at(big, 3, h, w), frame_at(big, 4, h, w)
@@ -389,6 +395,8 @@ def main():
     ap.add_argument("--no-entropy", dest="entropy", action="store_false",
                     help="config 4: raw int8 motion payload instead of the range coder stand-in")
     ap.add_argument("--cpu-baseline", action="store_true", help="also time stock RAFT on the host cores for 1 P-frame")
+    ap.add_argument("--b200-recurrent-block", action="store_true",
+                    help="config 4: swap rc.RecurrentBlock (the SepConvGRU as fused tcgen05 convolutions) into the model")
     args = ap.parse_args()
     if args.cudnn_benchmark:
         torch.backends.cudnn.benchmark = True

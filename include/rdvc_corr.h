@@ -280,6 +280,34 @@ int rdvc_mcn_forward(const float* warped, const float* flow, const float* ref, i
                      const unsigned long long* kmasks, const float* biases, void* workspace,
                      size_t workspace_bytes, float* out, void* stream);
 
+/* ---- RAFT's recurrent block: the SepConvGRU of every refinement iteration ---------------------------------- *
+ * rdvc_corr_convgru replaces ONE ConvGRU.forward (TV:raft.py:223-229) of torchvision's RecurrentBlock (TV:raft.py:238-270;
+ * raft_large: hidden size 128, input 256 = [context | motion features], kernels (1, 5) then (5, 1)):
+ *   z = sigmoid(convz([h | x])), r = sigmoid(convr([h | x])), q = tanh(convq([r * h | x])), out = (1 - z) h + z q
+ * as two tcgen05 implicit GEMMs (csrc/convgru_sm100.cuh): 16-bit operands (op_dtype), fp32 accumulation, fp32
+ * epilogue; z and r * h pass through the workspace in op_dtype; the blend uses h as given (act_dtype).
+ *
+ * rdvc_corr_convgru_pack_weights (HOST, no GPU needed): convz / convr / convq weights, each (128, 384, 1, 5) or
+ *   (128, 384, 5, 1) contiguous fp32 (both are w[co][ci][tap]) -> rdvc_corr_convgru_packed_weight_bytes() bytes of 16-bit
+ *   tap matrices: z|r [k-block 0..5][tap 0..4][256: convz rows, then convr rows][64 channels], then q
+ *   [k-block][tap][128][64]; input channel = 64 * k-block + column, tap t multiplies the pixel at offset t - 2 along
+ *   the tap axis.  Copy them to the device (16-byte aligned).
+ * rdvc_corr_convgru: h, context, motion: DEVICE, NHWC (B, H, W, >= 128), act_dtype F32 | F16 | BF16, channel stride 1 and
+ *   the given pixel strides in ELEMENTS (a multiple of 16 bytes; e.g. 256 for a channel slice of a 256-channel
+ *   channels_last tensor); base pointers 16-byte aligned.  op_dtype F16 | BF16; 16-bit activations must be op_dtype
+ *   (read in place), fp32 activations are rounded into the workspace first.  axis: the tap axis of the pass.
+ *   bias_z / bias_r / bias_q: 128 DEVICE floats each.  workspace: DEVICE, rdvc_corr_convgru_workspace_bytes(...), 256-byte
+ *   aligned.  out: DEVICE, (B, H, W, 128) contiguous act_dtype, not one of the inputs.  2 launches (3 for F32).      */
+#define RDVC_GRU_HORIZONTAL 0 /* 1 x 5 kernel, padding (0, 2): convgru1 */
+#define RDVC_GRU_VERTICAL 1   /* 5 x 1 kernel, padding (2, 0): convgru2 */
+size_t rdvc_corr_convgru_packed_weight_bytes(void);
+int rdvc_corr_convgru_pack_weights(const float* wz, const float* wr, const float* wq, int op_dtype, void* packed_host);
+size_t rdvc_corr_convgru_workspace_bytes(int B, int H, int W, int act_dtype);
+int rdvc_corr_convgru(const void* h, long long h_pixel_stride, const void* context, long long context_pixel_stride,
+                 const void* motion, long long motion_pixel_stride, int act_dtype, int op_dtype, int axis, int B, int H,
+                 int W, const void* packed_w, const float* bias_z, const float* bias_r, const float* bias_q,
+                 void* workspace, size_t workspace_bytes, void* out, void* stream);
+
 /* ---- next row f-4 (last piece): entropy-coder stand-in (HOST functions) ---- *
  * Stands in for the range coder behind EntropyBottleneck.compress / .decompress (R:codec_processing.py:433,447
  * construction, :488-497 compress, :509-536 decompress; compressai's RansEncoder.encode_with_indexes /

@@ -14,6 +14,7 @@ RDVC_DT_BF16, RDVC_DT_F32, RDVC_DT_F16 = 0, 1, 2
 RDVC_LAYOUT_ROWMAJOR, RDVC_LAYOUT_TILED = 0, 1
 RDVC_OUT_NCHW, RDVC_OUT_KMAJOR = 0, 1
 RDVC_ACT_NONE, RDVC_ACT_RELU = 0, 1
+RDVC_GRU_HORIZONTAL, RDVC_GRU_VERTICAL = 0, 1
 
 RDVC_E = {
     -1: "RDVC_E_NULL", -2: "RDVC_E_SHAPE", -3: "RDVC_E_TOO_SMALL", -4: "RDVC_E_DTYPE",
@@ -79,6 +80,11 @@ SYMBOLS = {
                                      _c.c_void_p, _c.c_void_p, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p]),
     "rdvc_mcn_forward": (_c.c_int, [_c.c_void_p] * 3 + [_c.c_int] * 4 + [_c.c_void_p, _c.c_void_p, _c.c_void_p,
                                     _c.c_void_p, _c.c_size_t, _c.c_void_p, _c.c_void_p]),
+    "rdvc_corr_convgru_packed_weight_bytes": (_c.c_size_t, []),
+    "rdvc_corr_convgru_pack_weights": (_c.c_int, [_c.c_void_p] * 3 + [_c.c_int, _c.c_void_p]),
+    "rdvc_corr_convgru_workspace_bytes": (_c.c_size_t, [_c.c_int] * 4),
+    "rdvc_corr_convgru": (_c.c_int, [_c.c_void_p, _c.c_longlong] * 3 + [_c.c_int] * 6 +
+                     [_c.c_void_p] * 5 + [_c.c_size_t, _c.c_void_p, _c.c_void_p]),
     "rdvc_corr_pair_host_submit": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p] +
                                    [_c.c_int] * 9),
     "rdvc_corr_pair_host_wait": (_c.c_int, [_c.c_int]),

@@ -22,6 +22,7 @@
 #include "corr_encoder_tail_sm100.cuh"
 #include "corr_lookup.cuh"
 #include "corr_pack.cuh"
+#include "convgru_sm100.cuh"
 #include "entropy_coder.h"
 #include "mcn_conv_sm100.cuh"
 #include "mcn_convx_sm100.cuh"
@@ -1592,6 +1593,188 @@ int rdvc_mcn_forward(const float* warped, const float* flow, const float* ref, i
     }
     return rdvc_mcn_conv_out(x, packed_weights[n_layers - 1], kmasks[n_layers - 1], biases + (n_layers - 1) * 32, 5, 3,
                              warped, out, B, H, W, stream);
+}
+
+}  // extern "C"
+
+// ---- RAFT's recurrent block: one ConvGRU pass as two tcgen05 implicit GEMMs ------------------------------------
+namespace {
+
+size_t gru_plane_bytes(int B, int H, int W) {
+    return align_up(static_cast<size_t>(B) * H * W * rdvc::GRU_C * 2, 256);
+}
+
+// {128 channels, across, along, B} over an NHWC tensor with pixel stride `ps` (16-bit elements); `horiz` lists y
+// before x so that the tap axis (x) is the map's third dimension (convgru_sm100.cuh, "Tile geometry")
+int gru_act_map(CUtensorMap* m, CUtensorMapDataType dt, const void* base, long long ps, int B, int H, int W, int horiz) {
+    const cuuint64_t px = static_cast<cuuint64_t>(ps) * 2, row = px * W;
+    const cuuint64_t dims[4] = {rdvc::GRU_C, static_cast<cuuint64_t>(horiz ? H : W), static_cast<cuuint64_t>(horiz ? W : H),
+                                static_cast<cuuint64_t>(B)};
+    const cuuint64_t strides[3] = {horiz ? row : px, horiz ? px : row, row * H};
+    const cuuint32_t box[4] = {64, rdvc::GRU_TA, rdvc::GRU_BOX_L, 1};
+    return make_tmap(m, dt, const_cast<void*>(base), 4, dims, strides, box);
+}
+
+int gru_weight_map(CUtensorMap* m, CUtensorMapDataType dt, const void* base, int n) {
+    const cuuint64_t dims[3] = {64, static_cast<cuuint64_t>(n), static_cast<cuuint64_t>(rdvc::GRU_KB * rdvc::GRU_TAPS)};
+    const cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(n) * 128};
+    const cuuint32_t box[3] = {64, static_cast<cuuint32_t>(n), 1};
+    return make_tmap(m, dt, const_cast<void*>(base), 3, dims, strides, box);
+}
+
+template <int MODE, typename ActT, typename OpT>
+int launch_convgru(const CUtensorMap& a0, const CUtensorMap& a1, const CUtensorMap& a2, const CUtensorMap& w,
+                   const rdvc::GruParams& p, cudaStream_t st) {
+    constexpr int SMEM = rdvc::GruCfg<MODE == 0 ? rdvc::GRU_ZR_N : rdvc::GRU_Q_N>::SMEM_LAUNCH;
+    auto kern = rdvc::convgru_kernel<MODE, ActT, OpT>;
+    static std::atomic<unsigned long long> attr_done{0};
+    if (int rc = ensure_dynamic_smem(kern, SMEM, attr_done, "cudaFuncSetAttribute(convgru, max dynamic smem)")) return rc;
+    const int grid = std::min(sm_count(), p.n_super);
+    kern<<<grid, rdvc::GRU_THREADS, SMEM, st>>>(a0, a1, a2, w, p);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, MODE == 0 ? "convgru_kernel (z|r) launch" : "convgru_kernel (q) launch");
+    return RDVC_OK;
+}
+
+uint16_t gru_round16(float v, int op_dtype) {
+    uint16_t bits;
+    if (op_dtype == RDVC_DT_F16) { const __half hv = __float2half_rn(v); memcpy(&bits, &hv, 2); }
+    else { const __nv_bfloat16 bv = __float2bfloat16_rn(v); memcpy(&bits, &bv, 2); }
+    return bits;
+}
+
+}  // namespace
+
+extern "C" {
+
+size_t rdvc_corr_convgru_packed_weight_bytes(void) {
+    return static_cast<size_t>(rdvc::GRU_W_ZR_ELEMS + rdvc::GRU_W_Q_ELEMS) * 2;
+}
+
+int rdvc_corr_convgru_pack_weights(const float* wz, const float* wr, const float* wq, int op_dtype, void* packed_host) {
+    if (!wz || !wr || !wq || !packed_host) return fail(RDVC_E_NULL, "null pointer argument");
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    constexpr int CIN = rdvc::GRU_KB * 64, T = rdvc::GRU_TAPS;
+    uint16_t* zr = static_cast<uint16_t*>(packed_host);
+    uint16_t* qq = zr + rdvc::GRU_W_ZR_ELEMS;
+    for (int kb = 0; kb < rdvc::GRU_KB; ++kb)
+        for (int t = 0; t < T; ++t)
+            for (int c = 0; c < 64; ++c) {
+                const size_t src = static_cast<size_t>(kb * 64 + c) * T + t;     // w[co][ci][t] of a (1, 5) or (5, 1) kernel
+                for (int n = 0; n < rdvc::GRU_ZR_N; ++n) {
+                    const float v = (n < rdvc::GRU_C ? wz[static_cast<size_t>(n) * CIN * T + src]
+                                                     : wr[static_cast<size_t>(n - rdvc::GRU_C) * CIN * T + src]);
+                    zr[(static_cast<size_t>(kb * T + t) * rdvc::GRU_ZR_N + n) * 64 + c] = gru_round16(v, op_dtype);
+                }
+                for (int n = 0; n < rdvc::GRU_Q_N; ++n)
+                    qq[(static_cast<size_t>(kb * T + t) * rdvc::GRU_Q_N + n) * 64 + c] =
+                        gru_round16(wq[static_cast<size_t>(n) * CIN * T + src], op_dtype);
+            }
+    return RDVC_OK;
+}
+
+size_t rdvc_corr_convgru_workspace_bytes(int B, int H, int W, int act_dtype) {
+    if (B <= 0 || H <= 0 || W <= 0) return 0;
+    if (act_dtype != RDVC_DT_F32 && act_dtype != RDVC_DT_F16 && act_dtype != RDVC_DT_BF16) return 0;
+    return (act_dtype == RDVC_DT_F32 ? 5 : 2) * gru_plane_bytes(B, H, W);
+}
+
+int rdvc_corr_convgru(const void* h, long long h_pixel_stride, const void* context, long long context_pixel_stride,
+                 const void* motion, long long motion_pixel_stride, int act_dtype, int op_dtype, int axis, int B, int H,
+                 int W, const void* packed_w, const float* bias_z, const float* bias_r, const float* bias_q,
+                 void* workspace, size_t workspace_bytes, void* out, void* stream) {
+    if (!h || !context || !motion || !packed_w || !bias_z || !bias_r || !bias_q || !workspace || !out)
+        return fail(RDVC_E_NULL, "null pointer argument");
+    if (B <= 0 || H <= 0 || W <= 0) return fail(RDVC_E_SHAPE, "non-positive dimension B=%d H=%d W=%d", B, H, W);
+    if (act_dtype != RDVC_DT_F32 && act_dtype != RDVC_DT_F16 && act_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "unsupported act_dtype=%d", act_dtype);
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    if (act_dtype != RDVC_DT_F32 && act_dtype != op_dtype)
+        return fail(RDVC_E_DTYPE, "16-bit activations are their own operands: act_dtype=%d needs op_dtype=%d", act_dtype,
+                    act_dtype);
+    if (axis != RDVC_GRU_HORIZONTAL && axis != RDVC_GRU_VERTICAL)
+        return fail(RDVC_E_UNSUPPORTED, "axis=%d is neither RDVC_GRU_HORIZONTAL nor RDVC_GRU_VERTICAL", axis);
+    const long long es = static_cast<long long>(elem_size(act_dtype));
+    const long long ps[3] = {h_pixel_stride, context_pixel_stride, motion_pixel_stride};
+    for (long long s : ps)
+        if (s < rdvc::GRU_C) return fail(RDVC_E_UNSUPPORTED, "pixel stride %lld < %d channels", s, rdvc::GRU_C);
+    const void* ptrs[5] = {h, context, motion, out, workspace};
+    for (const void* q : ptrs)
+        if (reinterpret_cast<uintptr_t>(q) & 15) return fail(RDVC_E_ALIGN, "activation buffers must be 16-byte aligned");
+    for (long long s : ps)
+        if ((s * es) % 16) return fail(RDVC_E_ALIGN, "pixel strides must be multiples of 16 bytes (got %lld elements)", s);
+    if ((reinterpret_cast<uintptr_t>(packed_w) & 15) || (reinterpret_cast<uintptr_t>(workspace) & 255))
+        return fail(RDVC_E_ALIGN, "packed weights must be 16-byte aligned, the workspace 256-byte aligned");
+    if (out == h || out == context || out == motion) return fail(RDVC_E_UNSUPPORTED, "the pass cannot run in place");
+    const long long n_pix = static_cast<long long>(B) * H * W;
+    if (n_pix >= (1LL << 31) || H >= (1 << 24) || W >= (1 << 24))
+        return fail(RDVC_E_UNSUPPORTED, "too many pixels for 32-bit TMA coordinates");
+    const size_t need = rdvc_corr_convgru_workspace_bytes(B, H, W, act_dtype);
+    if (workspace_bytes < need) return fail(RDVC_E_WORKSPACE, "workspace %zu < required %zu", workspace_bytes, need);
+
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const size_t plane = gru_plane_bytes(B, H, W);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    void* z = ws;
+    void* rh = ws + plane;
+    const void* a16[3] = {h, context, motion};          // the GEMMs' 16-bit operands
+    long long ps16[3] = {ps[0], ps[1], ps[2]};
+    if (act_dtype == RDVC_DT_F32) {
+        rdvc::GruCastParams cp;
+        memset(&cp, 0, sizeof(cp));
+        for (int i = 0; i < 3; ++i) {
+            cp.src[i] = static_cast<const float*>(a16[i]);
+            cp.ps[i] = ps[i];
+            cp.dst[i] = ws + (2 + i) * plane;
+            a16[i] = cp.dst[i];
+            ps16[i] = rdvc::GRU_C;
+        }
+        cp.n_pix = n_pix;
+        const dim3 grid(static_cast<unsigned>((n_pix * (rdvc::GRU_C / 8) + 255) / 256), 3);
+        if (op_dtype == RDVC_DT_F16) rdvc::convgru_cast_kernel<__half><<<grid, 256, 0, st>>>(cp);
+        else rdvc::convgru_cast_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(cp);
+        ++g_launches;
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return cuda_fail(e, "convgru_cast_kernel launch");
+    }
+    const int horiz = (axis == RDVC_GRU_HORIZONTAL) ? 1 : 0;
+    const CUtensorMapDataType dt = (op_dtype == RDVC_DT_F16) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    CUtensorMap t_h, t_rh, t_ctx, t_mot, t_wzr, t_wq;
+    if (int rc = gru_act_map(&t_h, dt, a16[0], ps16[0], B, H, W, horiz)) return rc;
+    if (int rc = gru_act_map(&t_ctx, dt, a16[1], ps16[1], B, H, W, horiz)) return rc;
+    if (int rc = gru_act_map(&t_mot, dt, a16[2], ps16[2], B, H, W, horiz)) return rc;
+    if (int rc = gru_act_map(&t_rh, dt, rh, rdvc::GRU_C, B, H, W, horiz)) return rc;
+    if (int rc = gru_weight_map(&t_wzr, dt, packed_w, rdvc::GRU_ZR_N)) return rc;
+    if (int rc = gru_weight_map(&t_wq, dt, static_cast<const uint16_t*>(packed_w) + rdvc::GRU_W_ZR_ELEMS, rdvc::GRU_Q_N))
+        return rc;
+
+    rdvc::GruParams p;
+    memset(&p, 0, sizeof(p));
+    p.B = B; p.H = H; p.W = W; p.horiz = horiz;
+    p.n_across = ((horiz ? H : W) + rdvc::GRU_TA - 1) / rdvc::GRU_TA;
+    p.n_along = ((horiz ? W : H) + rdvc::GRU_TL - 1) / rdvc::GRU_TL;
+    const long long n_tiles = static_cast<long long>(B) * p.n_across * p.n_along;
+    p.n_tiles = static_cast<int>(n_tiles);
+    p.n_super = static_cast<int>((n_tiles + rdvc::GRU_P - 1) / rdvc::GRU_P);
+    p.h = h; p.h_ps = ps[0];
+    p.z = z; p.rh = rh; p.out = out;
+    // the z|r pass reads bias0 = bz, bias1 = br; the q pass reads bias0 = bq (set between the launches)
+    p.bias0 = bias_z; p.bias1 = bias_r;
+    if (int rc = (act_dtype == RDVC_DT_F32 && op_dtype == RDVC_DT_F16)
+                     ? launch_convgru<0, float, __half>(t_h, t_ctx, t_mot, t_wzr, p, st)
+                 : (act_dtype == RDVC_DT_F32)   ? launch_convgru<0, float, __nv_bfloat16>(t_h, t_ctx, t_mot, t_wzr, p, st)
+                 : (op_dtype == RDVC_DT_F16)    ? launch_convgru<0, __half, __half>(t_h, t_ctx, t_mot, t_wzr, p, st)
+                                                : launch_convgru<0, __nv_bfloat16, __nv_bfloat16>(t_h, t_ctx, t_mot, t_wzr, p, st))
+        return rc;
+    p.bias0 = bias_q; p.bias1 = nullptr;
+    return (act_dtype == RDVC_DT_F32 && op_dtype == RDVC_DT_F16)
+               ? launch_convgru<1, float, __half>(t_rh, t_ctx, t_mot, t_wq, p, st)
+           : (act_dtype == RDVC_DT_F32) ? launch_convgru<1, float, __nv_bfloat16>(t_rh, t_ctx, t_mot, t_wq, p, st)
+           : (op_dtype == RDVC_DT_F16)  ? launch_convgru<1, __half, __half>(t_rh, t_ctx, t_mot, t_wq, p, st)
+                                        : launch_convgru<1, __nv_bfloat16, __nv_bfloat16>(t_rh, t_ctx, t_mot, t_wq, p, st);
 }
 
 }  // extern "C"

@@ -23,7 +23,9 @@ rows directly; the (2B, 256, h, w) fp32 feature maps (67 MB at 1080p) are never 
 :func:`raft_flow_sequence` is the same call for a RUN of n + 1 consecutive frames (the n pairs of an open-loop GOP):
 the feature encoder sees each frame once.
 
-All other convolutions stay stock PyTorch/cuDNN; only the correlation block (and those two 1x1s) is this library's.
+All other convolutions stay stock PyTorch/cuDNN; only the correlation block (and those two 1x1s) is this library's --
+unless the model's ``update_block.recurrent_block`` has been swapped for :class:`rc.RecurrentBlock`, which the fused
+path then hands ``context`` and the motion features as separate parts (no concatenation).
 
 :class:`GraphedRaftFlow` replays the whole call as ONE CUDA graph per input shape.  At the reference's
 default RAFT size (368x640, R:codec_processing.py:649-650) a P-frame's ~700 kernel launches cost more
@@ -39,6 +41,7 @@ import torch.nn.functional as F
 from torch import Tensor
 
 from .corr_block import TVCorrBlock, index_pyramid
+from .recurrent_block import RecurrentBlock
 
 
 def _coords_grid(batch: int, h: int, w: int, device) -> Tensor:
@@ -65,8 +68,11 @@ def _update_block_fused(model, blk: TVCorrBlock, hidden_state: Tensor, context: 
     f = me.convflow2(me.convflow1(flow))
     corr_flow = me.conv(torch.cat([corr, f], dim=1))
     motion_features = torch.cat([corr_flow, flow_orig], dim=1)
-    x = torch.cat([context, motion_features], dim=1)
-    hidden_state = ub.recurrent_block(hidden_state, x)
+    if isinstance(ub.recurrent_block, RecurrentBlock):       # reads context and motion features in place
+        hidden_state = ub.recurrent_block.forward_parts(hidden_state, context, motion_features)
+    else:
+        x = torch.cat([context, motion_features], dim=1)
+        hidden_state = ub.recurrent_block(hidden_state, x)
     return hidden_state, ub.flow_head(hidden_state)
 
 
