@@ -103,6 +103,14 @@ def run_sharded(args, own_process_group=True):
         rb = rc.RecurrentBlock(input_size=256, hidden_size=model.update_block.recurrent_block.hidden_size)
         rb.load_state_dict(model.update_block.recurrent_block.state_dict())
         model.update_block.recurrent_block = rb.to(dev)
+    if getattr(args, "b200_update_block", False):         # same weights, all three update-block submodules as this library's
+        ub = model.update_block
+        me, fh = rc.MotionEncoder(in_channels_corr=324), rc.FlowHead(in_channels=128, hidden_size=256)
+        me.load_state_dict(ub.motion_encoder.state_dict())
+        fh.load_state_dict(ub.flow_head.state_dict())
+        rb = rc.RecurrentBlock(input_size=256, hidden_size=ub.recurrent_block.hidden_size)
+        rb.load_state_dict(ub.recurrent_block.state_dict())
+        ub.motion_encoder, ub.recurrent_block, ub.flow_head = me.to(dev), rb.to(dev), fh.to(dev)
     h, w = args.height, args.width
     g = torch.Generator(device=dev).manual_seed(0)
     base = torch.rand(1, 3, h // 16 + 8, w // 16 + 8, device=dev, generator=g)
@@ -316,6 +324,8 @@ def run_sharded(args, own_process_group=True):
         }
         if getattr(args, "b200_recurrent_block", False):
             line["config"]["b200_recurrent_block"] = True
+        if getattr(args, "b200_update_block", False):
+            line["config"]["b200_update_block"] = True
         # flow end-point error of this configuration against STOCK torchvision RAFT (same weights, same autocast
         # setting) on one frame pair of the sequence -- outside the timed region
         a, b = frame_at(big, 3, h, w), frame_at(big, 4, h, w)
@@ -397,6 +407,9 @@ def main():
     ap.add_argument("--cpu-baseline", action="store_true", help="also time stock RAFT on the host cores for 1 P-frame")
     ap.add_argument("--b200-recurrent-block", action="store_true",
                     help="config 4: swap rc.RecurrentBlock (the SepConvGRU as fused tcgen05 convolutions) into the model")
+    ap.add_argument("--b200-update-block", action="store_true",
+                    help="swap rc.MotionEncoder, rc.RecurrentBlock and rc.FlowHead (the whole update block as this "
+                         "library's kernels) into the model")
     args = ap.parse_args()
     if args.cudnn_benchmark:
         torch.backends.cudnn.benchmark = True

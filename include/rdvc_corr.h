@@ -164,6 +164,16 @@ int rdvc_corr_lookup_conv1x1(const void* pyramid, int vol_dtype, int layout, con
                              int w, int num_levels, int radius, const void* packed_w, const float* bias, int cout,
                              int act, int feat_dtype, void* feat_ws, size_t feat_ws_bytes, void* out, int out_dtype,
                              void* stream);
+/* The _ex forms take out_pixel_stride: 0 = the (B, cout, h, w) output above; > 0 = NHWC, pixel m = b*h*w + y*w + x at
+ * out + m * out_pixel_stride, channel stride 1, out_dtype F16 | BF16, out 16-byte aligned, out_pixel_stride >= cout and
+ * a multiple of 8 (e.g. 256 for a channel slice of a 256-channel channels_last tensor).  Bit-identical values. */
+int rdvc_conv1x1_ex(const void* feat, int feat_dtype, const void* packed_w, const float* bias, int B, int h, int w,
+                    int num_levels, int radius, int cout, int act, void* out, int out_dtype, long long out_pixel_stride,
+                    void* stream);
+int rdvc_corr_lookup_conv1x1_ex(const void* pyramid, int vol_dtype, int layout, const float* coords, int B, int h,
+                                int w, int num_levels, int radius, const void* packed_w, const float* bias, int cout,
+                                int act, int feat_dtype, void* feat_ws, size_t feat_ws_bytes, void* out, int out_dtype,
+                                long long out_pixel_stride, void* stream);
 
 /* ---- next row f-2 (last sub-item): the feature encoder's final 1x1 convolution, fused into the operand repack ---- *
  * torchvision's FeatureEncoder ends in conv = Conv2d(128, 256, kernel_size=1) (TV:raft.py:139, called at :150); the
@@ -307,6 +317,52 @@ int rdvc_corr_convgru(const void* h, long long h_pixel_stride, const void* conte
                  const void* motion, long long motion_pixel_stride, int act_dtype, int op_dtype, int axis, int B, int H,
                  int W, const void* packed_w, const float* bias_z, const float* bias_r, const float* bias_q,
                  void* workspace, size_t workspace_bytes, void* out, void* stream);
+
+/* ---- RAFT's motion encoder and flow head: the rest of the update block ------------------------------------- *
+ * raft_large's MotionEncoder (TV:raft.py:171-211) after convcorr1 and its FlowHead (TV:raft.py:272-285) as convolutions
+ * over NHWC 16-bit activations (csrc/update_conv_sm100.cuh): the 3x3 layers are tcgen05 implicit GEMMs, convflow1 (7x7,
+ * 2 -> 128) a CUDA-core direct convolution.  16-bit operands (op_dtype), fp32 accumulation, bias (+ ReLU) in fp32.
+ *
+ * Layers (RDVC_UC_*), torchvision weight (cout, cin, k, k) contiguous fp32:
+ *   CONVCORR2  3x3 256 -> 192 + ReLU     TV:raft.py:186, 203     CONVFLOW1  7x7 2 -> 128 + ReLU   TV:raft.py:188, 205
+ *   CONVFLOW2  3x3 128 -> 64 + ReLU      TV:raft.py:189, 205     CONV       3x3 256 -> 126 + ReLU TV:raft.py:192, 208
+ *   FH_CONV1   3x3 128 -> 256 + ReLU     TV:raft.py:276, 285     FH_CONV2   3x3 256 -> 2          TV:raft.py:277, 285
+ * rdvc_corr_update_conv_pack_weights (HOST, no GPU needed) -> rdvc_corr_update_conv_packed_weight_bytes(layer) bytes of 16-bit
+ *   GEMM operand: 3x3 layers [cin / 64][dy * 3 + dx][N][64] (N = cout rounded up to 16: 192, 64, 128, 256, 16; padded
+ *   rows zero); CONVFLOW1 [128][128], column (ky * 7 + kx) * 2 + ci (K = 98, padded columns zero).  Copy to the device.
+ * rdvc_corr_update_conv: one layer.  in: DEVICE NHWC op_dtype, pixel stride in_pixel_stride elements (>= cin, a multiple of 8;
+ *   unused by CONVFLOW1).  flow (CONVFLOW1's input; CONV writes it into output channels 126-127): DEVICE fp32 at
+ *   flow[b * s[0] + c * s[1] + y * s[2] + x * s[3]], s = flow_strides (4 HOST long longs, elements).  bias: cout DEVICE
+ *   floats.  out: NHWC at out_pixel_stride elements (>= N, a multiple of 16 bytes), op_dtype -- except CONV (F32 or
+ *   op_dtype, the activation dtype) and FH_CONV2, which writes (B, 2, H, W) contiguous planes (F32 or op_dtype) and
+ *   ignores out_pixel_stride.  Channel slices of a channels_last tensor are read and written in place; nothing outside
+ *   [0, N) of each output pixel is written.
+ * rdvc_corr_motion_encoder: MotionEncoder.forward (TV:raft.py:200-211) from convcorr1's NHWC output c1 (op_dtype, 256
+ *   channels): 4 launches, out = the (B, H, W, 128) motion features [conv | flow] at out_pixel_stride, out_dtype F32 or
+ *   op_dtype.  packed_w / bias: 4 DEVICE pointers each, in the order CONVCORR2, CONVFLOW1, CONVFLOW2, CONV.  workspace:
+ *   DEVICE, rdvc_corr_motion_encoder_workspace_bytes(...), 256-byte aligned.
+ * rdvc_corr_flow_head: FlowHead.forward (TV:raft.py:284-285) on h (NHWC act_dtype, >= 128 channels at h_pixel_stride): out =
+ *   (B, 2, H, W) act_dtype.  16-bit act_dtype must be op_dtype; fp32 h is rounded into the workspace first (3 launches,
+ *   else 2).  packed_w / bias: FH_CONV1, FH_CONV2.  workspace: rdvc_corr_flow_head_workspace_bytes(...), 256-byte aligned. */
+#define RDVC_UC_CONVCORR2 0
+#define RDVC_UC_CONVFLOW1 1
+#define RDVC_UC_CONVFLOW2 2
+#define RDVC_UC_CONV 3
+#define RDVC_UC_FH_CONV1 4
+#define RDVC_UC_FH_CONV2 5
+size_t rdvc_corr_update_conv_packed_weight_bytes(int layer);
+int rdvc_corr_update_conv_pack_weights(int layer, const float* weight, int op_dtype, void* packed_host);
+int rdvc_corr_update_conv(int layer, const void* in, long long in_pixel_stride, const float* flow, const long long* flow_strides,
+                     int B, int H, int W, int op_dtype, const void* packed_w, const float* bias, void* out,
+                     long long out_pixel_stride, int out_dtype, void* stream);
+size_t rdvc_corr_motion_encoder_workspace_bytes(int B, int H, int W);
+int rdvc_corr_motion_encoder(const void* c1, long long c1_pixel_stride, const float* flow, const long long* flow_strides, int B,
+                        int H, int W, int op_dtype, const void* const* packed_w, const float* const* bias, void* workspace,
+                        size_t workspace_bytes, void* out, long long out_pixel_stride, int out_dtype, void* stream);
+size_t rdvc_corr_flow_head_workspace_bytes(int B, int H, int W, int act_dtype);
+int rdvc_corr_flow_head(const void* h, long long h_pixel_stride, int act_dtype, int B, int H, int W, int op_dtype,
+                   const void* const* packed_w, const float* const* bias, void* workspace, size_t workspace_bytes, void* out,
+                   void* stream);
 
 /* ---- next row f-4 (last piece): entropy-coder stand-in (HOST functions) ---- *
  * Stands in for the range coder behind EntropyBottleneck.compress / .decompress (R:codec_processing.py:433,447

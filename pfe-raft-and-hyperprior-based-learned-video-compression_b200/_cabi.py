@@ -15,6 +15,7 @@ RDVC_LAYOUT_ROWMAJOR, RDVC_LAYOUT_TILED = 0, 1
 RDVC_OUT_NCHW, RDVC_OUT_KMAJOR = 0, 1
 RDVC_ACT_NONE, RDVC_ACT_RELU = 0, 1
 RDVC_GRU_HORIZONTAL, RDVC_GRU_VERTICAL = 0, 1
+RDVC_UC_CONVCORR2, RDVC_UC_CONVFLOW1, RDVC_UC_CONVFLOW2, RDVC_UC_CONV, RDVC_UC_FH_CONV1, RDVC_UC_FH_CONV2 = range(6)
 
 RDVC_E = {
     -1: "RDVC_E_NULL", -2: "RDVC_E_SHAPE", -3: "RDVC_E_TOO_SMALL", -4: "RDVC_E_DTYPE",
@@ -85,6 +86,22 @@ SYMBOLS = {
     "rdvc_corr_convgru_workspace_bytes": (_c.c_size_t, [_c.c_int] * 4),
     "rdvc_corr_convgru": (_c.c_int, [_c.c_void_p, _c.c_longlong] * 3 + [_c.c_int] * 6 +
                      [_c.c_void_p] * 5 + [_c.c_size_t, _c.c_void_p, _c.c_void_p]),
+    "rdvc_conv1x1_ex": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_void_p, _c.c_void_p] + [_c.c_int] * 7 +
+                        [_c.c_void_p, _c.c_int, _c.c_longlong, _c.c_void_p]),
+    "rdvc_corr_lookup_conv1x1_ex": (_c.c_int, [_c.c_void_p, _c.c_int, _c.c_int, _c.c_void_p] + [_c.c_int] * 5 +
+                                    [_c.c_void_p, _c.c_void_p, _c.c_int, _c.c_int, _c.c_int, _c.c_void_p, _c.c_size_t,
+                                     _c.c_void_p, _c.c_int, _c.c_longlong, _c.c_void_p]),
+    "rdvc_corr_update_conv_packed_weight_bytes": (_c.c_size_t, [_c.c_int]),
+    "rdvc_corr_update_conv_pack_weights": (_c.c_int, [_c.c_int, _c.c_void_p, _c.c_int, _c.c_void_p]),
+    "rdvc_corr_update_conv": (_c.c_int, [_c.c_int, _c.c_void_p, _c.c_longlong, _c.c_void_p, _c.c_void_p] + [_c.c_int] * 4 +
+                         [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_longlong, _c.c_int, _c.c_void_p]),
+    "rdvc_corr_motion_encoder_workspace_bytes": (_c.c_size_t, [_c.c_int] * 3),
+    "rdvc_corr_motion_encoder": (_c.c_int, [_c.c_void_p, _c.c_longlong, _c.c_void_p, _c.c_void_p] + [_c.c_int] * 4 +
+                            [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_void_p, _c.c_longlong, _c.c_int,
+                             _c.c_void_p]),
+    "rdvc_corr_flow_head_workspace_bytes": (_c.c_size_t, [_c.c_int] * 4),
+    "rdvc_corr_flow_head": (_c.c_int, [_c.c_void_p, _c.c_longlong] + [_c.c_int] * 5 +
+                       [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_size_t, _c.c_void_p, _c.c_void_p]),
     "rdvc_corr_pair_host_submit": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p] +
                                    [_c.c_int] * 9),
     "rdvc_corr_pair_host_wait": (_c.c_int, [_c.c_int]),

@@ -416,7 +416,7 @@ class TVCorrBlock(nn.Module):
 
     def index_pyramid_convcorr1(self, centroids_coords: Tensor, weight: Tensor, bias: Optional[Tensor] = None,
                                 relu: bool = True, out_dtype: Optional[torch.dtype] = None,
-                                feat_dtype: Optional[torch.dtype] = None) -> Tensor:
+                                feat_dtype: Optional[torch.dtype] = None, nhwc: bool = False) -> Tensor:
         """``relu(conv1x1(index_pyramid(coords), weight, bias))`` -- the lookup fused with
         ``MotionEncoder.convcorr1`` (TV:raft.py:185,202) through ``rdvc_corr_lookup_conv1x1``: the (B, 324, h, w)
         fp32 lookup tensor is never written.  ``weight``: (cout, L*S*S[, 1, 1]) in torchvision's channel order.
@@ -424,7 +424,11 @@ class TVCorrBlock(nn.Module):
         convolution, and exactly what the stock path multiplies under the reference's default fp16 autocast; the
         conversion saturates at +-65504, three orders above any correlation value RAFT's features produce),
         ``feat_dtype=torch.bfloat16`` trades mantissa for range (within 1e-2).  The result is fp32, or the autocast
-        dtype when autocast is on."""
+        dtype when autocast is on.
+
+        ``nhwc=True``: the result is a channels_last (B, cout, h, w) tensor in ``feat_dtype``, written by the GEMM's
+        epilogue straight from the accumulator (``rdvc_corr_lookup_conv1x1_ex``), bit-identical to the default output
+        rounded to that dtype; it is what ``MotionEncoder.forward_fused`` reads in place."""
         if self._pyr is None:
             raise RuntimeError("index_pyramid_convcorr1 called before build_pyramid")
         pyr = self._pyr
@@ -442,8 +446,19 @@ class TVCorrBlock(nn.Module):
         shape = feat_shape(B, h, w, self.num_levels, self.radius)
         if self._feat is None or tuple(self._feat.shape) != shape or self._feat.dtype != feat_dtype or self._feat.device != dev:
             self._feat = torch.zeros(shape, dtype=feat_dtype, device=dev)
-        out = torch.empty((B, self._packed.cout, h, w), dtype=out_dtype, device=dev)
         lib = _cabi.load()
+        if nhwc:
+            out = torch.empty((B, h, w, self._packed.cout), dtype=feat_dtype, device=dev)
+            with torch.cuda.device(dev):
+                rc = lib.rdvc_corr_lookup_conv1x1_ex(
+                    pyr.buffer.data_ptr(), _VOL_DTYPES[pyr.volume_dtype], pyr.layout, c.data_ptr(), B, h, w,
+                    self.num_levels, self.radius, self._packed.weight.data_ptr(),
+                    0 if self._packed.bias is None else self._packed.bias.data_ptr(), self._packed.cout,
+                    _cabi.RDVC_ACT_RELU if relu else _cabi.RDVC_ACT_NONE, _FEAT_DTYPES[feat_dtype], self._feat.data_ptr(),
+                    self._feat.numel() * 2, out.data_ptr(), _FEAT_DTYPES[feat_dtype], self._packed.cout, _stream_ptr(dev))
+            _cabi.check(rc, "rdvc_corr_lookup_conv1x1_ex")
+            return out.permute(0, 3, 1, 2)
+        out = torch.empty((B, self._packed.cout, h, w), dtype=out_dtype, device=dev)
         with torch.cuda.device(dev):
             rc = lib.rdvc_corr_lookup_conv1x1(
                 pyr.buffer.data_ptr(), _VOL_DTYPES[pyr.volume_dtype], pyr.layout, c.data_ptr(), B, h, w, self.num_levels,

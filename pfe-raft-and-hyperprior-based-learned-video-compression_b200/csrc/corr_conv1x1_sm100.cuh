@@ -81,6 +81,7 @@ struct Conv1x1Params {
     int ab_format;          // tcgen05 kind::f16 operand format: 1 = bf16, 0 = fp16
     unsigned long long* dbg_timeline;   // RDVC_EXPERIMENTS builds only: 16 globaltimer stamps per CTA (nullptr = off)
     int dbg_flags;                      // RDVC_EXPERIMENTS builds only: 1 = no output stores, 2 = no TMEM reads (timing)
+    long long out_ps;                   // NHWC instantiations: `out` is (B*h*w) pixels of out_ps elements, channel stride 1
 };
 
 #ifdef RDVC_EXPERIMENTS
@@ -143,13 +144,28 @@ template <> __device__ __forceinline__ float c1_cvt<float>(float x) { return x; 
 template <> __device__ __forceinline__ __half c1_cvt<__half>(float x) { return __float2half_rn(x); }
 template <> __device__ __forceinline__ __nv_bfloat16 c1_cvt<__nv_bfloat16>(float x) { return __float2bfloat16_rn(x); }
 
+// 16 values -> one pixel's 16 consecutive 16-bit channels: two 16-byte stores
+template <typename OutT>
+__device__ __forceinline__ void c1_store16(OutT* dst, const float* v) {
+    static_assert(sizeof(OutT) == 2, "NHWC output is 16-bit");
+    uint32_t w[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+        const OutT lo = c1_cvt<OutT>(v[2 * j]), hi = c1_cvt<OutT>(v[2 * j + 1]);
+        w[j] = static_cast<uint32_t>(*reinterpret_cast<const uint16_t*>(&lo)) |
+               (static_cast<uint32_t>(*reinterpret_cast<const uint16_t*>(&hi)) << 16);
+    }
+    reinterpret_cast<uint4*>(dst)[0] = make_uint4(w[0], w[1], w[2], w[3]);
+    reinterpret_cast<uint4*>(dst)[1] = make_uint4(w[4], w[5], w[6], w[7]);
+}
+
 // grid: an even number of CTAs (clusters of 2); block: C1_THREADS; dynamic smem: C1_SMEM_LAUNCH.
 // tm_a: features as a {64 (8 rows x 8 elements), rows / 8, kp / 8} tensor, box {64, 16, 8}, no swizzle;
 // tm_w: packed weights {kpw, cout, 1}, box {64, cout / 2, 1}, 128-byte swizzle.
-template <typename OutT>
-__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(C1_THREADS, 1)
-corr_conv1x1_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_w,
-                    const Conv1x1Params p) {
+// NHWC: the result goes out as (pixel, channel) rows of p.out_ps 16-bit elements straight from the accumulator (thread =
+// pixel, 16-byte stores, no transpose): the layout the 3x3 convolutions that follow read (update_conv_sm100.cuh).
+template <typename OutT, bool NHWC>
+__device__ __forceinline__ void corr_conv1x1_body(const CUtensorMap& tm_a, const CUtensorMap& tm_w, const Conv1x1Params p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(
         (reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -327,6 +343,19 @@ corr_conv1x1_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_const
                     if (lane == 0) ptx::mbar_arrive_cluster_relaxed(t_empty_leader0 + 8u * acc);
                 }
                 const int nch = two ? 32 : 16;
+                if constexpr (NHWC) {
+                    if (ok && !C1_DBG(1)) {
+#pragma unroll
+                        for (int i = 0; i < 32; ++i) {
+                            v[i] += lds_ro_f32(s_bias + min(ch0 + c + i, p.cout - 1) * 4);
+                            if (p.relu) v[i] = fmaxf(v[i], 0.f);
+                        }
+                        OutT* d = static_cast<OutT*>(p.out) + pix * p.out_ps + ch0 + c;
+                        c1_store16(d, v);
+                        if (two) c1_store16(d + 16, v + 16);
+                    }
+                    continue;
+                }
                 if (p.vec4) {
                     // transpose through this warp's 4 KB buffer: [channel][pixel] fp32, a row is one conflict-free
                     // 128-byte st.shared; a quarter-warp then reads one row back as eight 16-byte pieces
@@ -371,6 +400,20 @@ corr_conv1x1_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_const
     ptx::cluster_sync_all();          // the leader's MMAs read the peer's shared memory until the very end
     if (warp == 0 && lane == 0) C1_STAMP(12);
     if (warp == 2) ptx::tmem_dealloc_2sm(tmem_base, 512);
+}
+
+template <typename OutT>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(C1_THREADS, 1)
+corr_conv1x1_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_w,
+                    const Conv1x1Params p) {
+    corr_conv1x1_body<OutT, false>(tm_a, tm_w, p);
+}
+
+template <typename OutT>
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(C1_THREADS, 1)
+corr_conv1x1_nhwc_kernel(const __grid_constant__ CUtensorMap tm_a, const __grid_constant__ CUtensorMap tm_w,
+                         const Conv1x1Params p) {
+    corr_conv1x1_body<OutT, true>(tm_a, tm_w, p);
 }
 
 }  // namespace rdvc

@@ -23,6 +23,7 @@
 #include "corr_lookup.cuh"
 #include "corr_pack.cuh"
 #include "convgru_sm100.cuh"
+#include "update_conv_sm100.cuh"
 #include "entropy_coder.h"
 #include "mcn_conv_sm100.cuh"
 #include "mcn_convx_sm100.cuh"
@@ -379,10 +380,13 @@ int dispatch_lookup_tiled(int out_mode, int dbg, int radius, const rdvc::LookupP
     }
 }
 
-template <typename OutT>
+template <typename OutT, bool NHWC = false>
 cudaError_t launch_conv1x1(const CUtensorMap& tm_a, const CUtensorMap& tm_w, const rdvc::Conv1x1Params& p, unsigned grid,
                            cudaStream_t st) {
-    auto kern = rdvc::corr_conv1x1_kernel<OutT>;
+    auto kern = [] {
+        if constexpr (NHWC) return rdvc::corr_conv1x1_nhwc_kernel<OutT>;
+        else return rdvc::corr_conv1x1_kernel<OutT>;
+    }();
     static std::atomic<unsigned long long> attr_done{0};
     if (ensure_dynamic_smem(kern, rdvc::C1_SMEM_LAUNCH, attr_done, "cudaFuncSetAttribute(conv1x1, max dynamic smem)"))
         return cudaErrorInvalidValue;
@@ -1115,6 +1119,13 @@ int rdvc_conv1x1_pack_weights(const float* weight, int cout, int num_levels, int
 
 int rdvc_conv1x1(const void* feat, int feat_dtype, const void* packed_w, const float* bias, int B, int h, int w,
                  int num_levels, int radius, int cout, int act, void* out, int out_dtype, void* stream) {
+    return rdvc_conv1x1_ex(feat, feat_dtype, packed_w, bias, B, h, w, num_levels, radius, cout, act, out, out_dtype, 0,
+                           stream);
+}
+
+int rdvc_conv1x1_ex(const void* feat, int feat_dtype, const void* packed_w, const float* bias, int B, int h, int w,
+                    int num_levels, int radius, int cout, int act, void* out, int out_dtype, long long out_pixel_stride,
+                    void* stream) {
     if (!feat || !packed_w || !out) return fail(RDVC_E_NULL, "null pointer argument");
     if (B <= 0 || h <= 0 || w <= 0) return fail(RDVC_E_SHAPE, "non-positive dimension B=%d h=%d w=%d", B, h, w);
     if (feat_dtype != RDVC_DT_BF16 && feat_dtype != RDVC_DT_F16)
@@ -1128,6 +1139,14 @@ int rdvc_conv1x1(const void* feat, int feat_dtype, const void* packed_w, const f
         return fail(RDVC_E_UNSUPPORTED, "cout=%d must be a multiple of 32 and <= %d", cout, rdvc::C1_MAX_COUT);
     if ((reinterpret_cast<uintptr_t>(feat) & 15) || (reinterpret_cast<uintptr_t>(packed_w) & 15))
         return fail(RDVC_E_ALIGN, "feature rows and packed weights must be 16-byte aligned");
+    if (out_pixel_stride < 0) return fail(RDVC_E_UNSUPPORTED, "negative out_pixel_stride %lld", out_pixel_stride);
+    if (out_pixel_stride > 0) {
+        if (out_dtype == RDVC_DT_F32) return fail(RDVC_E_DTYPE, "the NHWC output is 16-bit (F16 or BF16)");
+        if (out_pixel_stride < cout)
+            return fail(RDVC_E_UNSUPPORTED, "out_pixel_stride %lld < cout %d", out_pixel_stride, cout);
+        if ((out_pixel_stride % 8) || (reinterpret_cast<uintptr_t>(out) & 15))
+            return fail(RDVC_E_ALIGN, "NHWC output: 16-byte aligned with a pixel stride that is a multiple of 8 elements");
+    }
     const long long m_total = static_cast<long long>(B) * h * w;
     if (m_total >= (1LL << 31) - 256) return fail(RDVC_E_UNSUPPORTED, "too many pixels for 32-bit TMA coordinates");
     const size_t kpw = align_up(kp, 64);
@@ -1167,7 +1186,11 @@ int rdvc_conv1x1(const void* feat, int feat_dtype, const void* packed_w, const f
     grid = (grid + 1) & ~1LL;                                  // whole CTA pairs (a trailing CTA may own no rows)
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     cudaError_t e;
-    if (out_dtype == RDVC_DT_F32) e = launch_conv1x1<float>(tm_a, tm_w, p, static_cast<unsigned>(grid), st);
+    p.out_ps = out_pixel_stride;
+    if (out_pixel_stride > 0 && out_dtype == RDVC_DT_F16)
+        e = launch_conv1x1<__half, true>(tm_a, tm_w, p, static_cast<unsigned>(grid), st);
+    else if (out_pixel_stride > 0) e = launch_conv1x1<__nv_bfloat16, true>(tm_a, tm_w, p, static_cast<unsigned>(grid), st);
+    else if (out_dtype == RDVC_DT_F32) e = launch_conv1x1<float>(tm_a, tm_w, p, static_cast<unsigned>(grid), st);
     else if (out_dtype == RDVC_DT_F16) e = launch_conv1x1<__half>(tm_a, tm_w, p, static_cast<unsigned>(grid), st);
     else e = launch_conv1x1<__nv_bfloat16>(tm_a, tm_w, p, static_cast<unsigned>(grid), st);
     if (e != cudaSuccess) return cuda_fail(e, "corr_conv1x1_kernel launch");
@@ -1178,6 +1201,14 @@ int rdvc_corr_lookup_conv1x1(const void* pyramid, int vol_dtype, int layout, con
                              int w, int num_levels, int radius, const void* packed_w, const float* bias, int cout,
                              int act, int feat_dtype, void* feat_ws, size_t feat_ws_bytes, void* out, int out_dtype,
                              void* stream) {
+    return rdvc_corr_lookup_conv1x1_ex(pyramid, vol_dtype, layout, coords, B, h, w, num_levels, radius, packed_w, bias, cout,
+                                       act, feat_dtype, feat_ws, feat_ws_bytes, out, out_dtype, 0, stream);
+}
+
+int rdvc_corr_lookup_conv1x1_ex(const void* pyramid, int vol_dtype, int layout, const float* coords, int B, int h,
+                                int w, int num_levels, int radius, const void* packed_w, const float* bias, int cout,
+                                int act, int feat_dtype, void* feat_ws, size_t feat_ws_bytes, void* out, int out_dtype,
+                                long long out_pixel_stride, void* stream) {
     if (!feat_ws) return fail(RDVC_E_NULL, "null pointer argument");
     const size_t kp = rdvc_corr_feat_pitch(num_levels, radius);
     if (kp == 0) return fail(RDVC_E_UNSUPPORTED, "num_levels=%d / radius=%d not supported", num_levels, radius);
@@ -1187,7 +1218,8 @@ int rdvc_corr_lookup_conv1x1(const void* pyramid, int vol_dtype, int layout, con
     int rc = rdvc_corr_lookup_ex(pyramid, vol_dtype, layout, coords, B, h, w, num_levels, radius, feat_ws, feat_dtype,
                                  RDVC_OUT_KMAJOR, stream);
     if (rc) return rc;
-    return rdvc_conv1x1(feat_ws, feat_dtype, packed_w, bias, B, h, w, num_levels, radius, cout, act, out, out_dtype, stream);
+    return rdvc_conv1x1_ex(feat_ws, feat_dtype, packed_w, bias, B, h, w, num_levels, radius, cout, act, out, out_dtype,
+                           out_pixel_stride, stream);
 }
 
 int rdvc_motion_warp(const float* prev, const float* flow, int B, int C, int H, int W, int h_in, int w_in,
@@ -1775,6 +1807,281 @@ int rdvc_corr_convgru(const void* h, long long h_pixel_stride, const void* conte
            : (act_dtype == RDVC_DT_F32) ? launch_convgru<1, float, __nv_bfloat16>(t_rh, t_ctx, t_mot, t_wq, p, st)
            : (op_dtype == RDVC_DT_F16)  ? launch_convgru<1, __half, __half>(t_rh, t_ctx, t_mot, t_wq, p, st)
                                         : launch_convgru<1, __nv_bfloat16, __nv_bfloat16>(t_rh, t_ctx, t_mot, t_wq, p, st);
+}
+
+}  // extern "C"
+
+// ---- RAFT's motion encoder and flow head: 3x3 (and convflow1's 7x7) convolutions over NHWC 16-bit activations ---------
+namespace {
+
+struct UcLayer {
+    int cin, cout, k, n;        // input / output channels, kernel size, GEMM width (cout padded to a multiple of 16)
+};
+// indexed by RDVC_UC_*: raft_large's MotionEncoder (TV:raft.py:184-196) and FlowHead (TV:raft.py:276-277)
+constexpr UcLayer UC_LAYERS[6] = {
+    {256, 192, 3, 192},     // RDVC_UC_CONVCORR2
+    {2, 128, 7, 128},       // RDVC_UC_CONVFLOW1 (K = 98 padded to 128)
+    {128, 64, 3, 64},       // RDVC_UC_CONVFLOW2
+    {256, 126, 3, 128},     // RDVC_UC_CONV
+    {128, 256, 3, 256},     // RDVC_UC_FH_CONV1
+    {256, 2, 3, 16},        // RDVC_UC_FH_CONV2
+};
+
+size_t uc_packed_elems(int layer) {
+    const UcLayer& L = UC_LAYERS[layer];
+    if (layer == RDVC_UC_CONVFLOW1) return static_cast<size_t>(L.n) * rdvc::CF1_KP;
+    return static_cast<size_t>(L.cin / 64) * 9 * L.n * 64;
+}
+
+size_t uc_plane_bytes(int B, int H, int W, int channels) {
+    return align_up(static_cast<size_t>(B) * H * W * channels * 2, 256);
+}
+
+template <int N, int EPI, typename OutT, typename OpT>
+int launch_update_conv(const CUtensorMap& a, const CUtensorMap& w, const rdvc::UcParams& p, cudaStream_t st) {
+    constexpr int SMEM = rdvc::UcCfg<N>::SMEM_LAUNCH;
+    auto kern = rdvc::update_conv_kernel<N, EPI, OutT, OpT>;
+    static std::atomic<unsigned long long> attr_done{0};
+    if (int rc = ensure_dynamic_smem(kern, SMEM, attr_done, "cudaFuncSetAttribute(update_conv, max dynamic smem)")) return rc;
+    const int grid = std::min(sm_count(), p.n_super);
+    kern<<<grid, rdvc::UC_THREADS, SMEM, st>>>(a, w, p);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "update_conv_kernel launch");
+    return RDVC_OK;
+}
+
+template <typename OpT>
+int launch_convflow1(const rdvc::Cf1Params& p, cudaStream_t st) {
+    auto kern = rdvc::convflow1_kernel<OpT>;
+    static std::atomic<unsigned long long> attr_done{0};
+    if (int rc = ensure_dynamic_smem(kern, rdvc::CF1_SMEM, attr_done, "cudaFuncSetAttribute(convflow1, max dynamic smem)"))
+        return rc;
+    const long long groups = (p.n_pix + 31) / 32;
+    const long long grid = std::min<long long>(4LL * sm_count(), (groups + 1) / 2);
+    kern<<<static_cast<unsigned>(grid), rdvc::CF1_THREADS, rdvc::CF1_SMEM, st>>>(p);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "convflow1_kernel launch");
+    return RDVC_OK;
+}
+
+// the 3x3 layers' dispatch: one instantiation per (layer, output dtype, operand dtype)
+template <typename OpT>
+int dispatch_update_conv(int layer, int out_dtype, const CUtensorMap& a, const CUtensorMap& w, const rdvc::UcParams& p,
+                         cudaStream_t st) {
+    const bool f32 = (out_dtype == RDVC_DT_F32);
+    switch (layer) {
+        case RDVC_UC_CONVCORR2: return launch_update_conv<192, rdvc::UC_EPI_RELU, OpT, OpT>(a, w, p, st);
+        case RDVC_UC_CONVFLOW2: return launch_update_conv<64, rdvc::UC_EPI_RELU, OpT, OpT>(a, w, p, st);
+        case RDVC_UC_FH_CONV1: return launch_update_conv<256, rdvc::UC_EPI_RELU, OpT, OpT>(a, w, p, st);
+        case RDVC_UC_CONV:
+            return f32 ? launch_update_conv<128, rdvc::UC_EPI_RELU_FLOW, float, OpT>(a, w, p, st)
+                       : launch_update_conv<128, rdvc::UC_EPI_RELU_FLOW, OpT, OpT>(a, w, p, st);
+        default:
+            return f32 ? launch_update_conv<16, rdvc::UC_EPI_FLOW2, float, OpT>(a, w, p, st)
+                       : launch_update_conv<16, rdvc::UC_EPI_FLOW2, OpT, OpT>(a, w, p, st);
+    }
+}
+
+}  // namespace
+
+extern "C" {
+
+size_t rdvc_corr_update_conv_packed_weight_bytes(int layer) {
+    if (layer < 0 || layer > RDVC_UC_FH_CONV2) return 0;
+    return uc_packed_elems(layer) * 2;
+}
+
+int rdvc_corr_update_conv_pack_weights(int layer, const float* weight, int op_dtype, void* packed_host) {
+    if (!weight || !packed_host) return fail(RDVC_E_NULL, "null pointer argument");
+    if (layer < 0 || layer > RDVC_UC_FH_CONV2) return fail(RDVC_E_UNSUPPORTED, "unknown layer %d", layer);
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    const UcLayer& L = UC_LAYERS[layer];
+    uint16_t* out = static_cast<uint16_t*>(packed_host);
+    memset(out, 0, uc_packed_elems(layer) * 2);                 // padded rows (N > cout) and columns (K > 98) are zero
+    const int kk = L.k * L.k;
+    if (layer == RDVC_UC_CONVFLOW1) {                           // [n][(ky * 7 + kx) * 2 + ci]
+        for (int n = 0; n < L.cout; ++n)
+            for (int ci = 0; ci < L.cin; ++ci)
+                for (int t = 0; t < kk; ++t)
+                    out[static_cast<size_t>(n) * rdvc::CF1_KP + t * 2 + ci] =
+                        gru_round16(weight[(static_cast<size_t>(n) * L.cin + ci) * kk + t], op_dtype);
+        return RDVC_OK;
+    }
+    for (int kb = 0; kb < L.cin / 64; ++kb)                     // [k-block][dy * 3 + dx][n][64]
+        for (int t = 0; t < 9; ++t)
+            for (int n = 0; n < L.cout; ++n)
+                for (int c = 0; c < 64; ++c)
+                    out[((static_cast<size_t>(kb) * 9 + t) * L.n + n) * 64 + c] =
+                        gru_round16(weight[(static_cast<size_t>(n) * L.cin + kb * 64 + c) * 9 + t], op_dtype);
+    return RDVC_OK;
+}
+
+int rdvc_corr_update_conv(int layer, const void* in, long long in_pixel_stride, const float* flow, const long long* flow_strides,
+                     int B, int H, int W, int op_dtype, const void* packed_w, const float* bias, void* out,
+                     long long out_pixel_stride, int out_dtype, void* stream) {
+    if (layer < 0 || layer > RDVC_UC_FH_CONV2) return fail(RDVC_E_UNSUPPORTED, "unknown layer %d", layer);
+    const UcLayer& L = UC_LAYERS[layer];
+    const bool uses_flow = (layer == RDVC_UC_CONVFLOW1 || layer == RDVC_UC_CONV);
+    if (!packed_w || !bias || !out || (layer != RDVC_UC_CONVFLOW1 && !in) || (uses_flow && (!flow || !flow_strides)))
+        return fail(RDVC_E_NULL, "null pointer argument");
+    if (B <= 0 || H <= 0 || W <= 0) return fail(RDVC_E_SHAPE, "non-positive dimension B=%d H=%d W=%d", B, H, W);
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    const bool act_out = (layer == RDVC_UC_CONV || layer == RDVC_UC_FH_CONV2);    // written in the activation dtype
+    if (act_out ? (out_dtype != RDVC_DT_F32 && out_dtype != op_dtype) : (out_dtype != op_dtype))
+        return fail(RDVC_E_DTYPE, "layer %d cannot write out_dtype=%d with op_dtype=%d", layer, out_dtype, op_dtype);
+    const long long n_pix = static_cast<long long>(B) * H * W;
+    if (n_pix >= (1LL << 31) || H >= (1 << 24) || W >= (1 << 24))
+        return fail(RDVC_E_UNSUPPORTED, "too many pixels for 32-bit TMA coordinates");
+    if ((reinterpret_cast<uintptr_t>(packed_w) & 15) || (reinterpret_cast<uintptr_t>(out) & 15) ||
+        (in && (reinterpret_cast<uintptr_t>(in) & 15)))
+        return fail(RDVC_E_ALIGN, "input, output and packed weights must be 16-byte aligned");
+    if (layer != RDVC_UC_CONVFLOW1) {
+        if (in_pixel_stride < L.cin) return fail(RDVC_E_UNSUPPORTED, "in_pixel_stride %lld < %d", in_pixel_stride, L.cin);
+        if (in_pixel_stride % 8) return fail(RDVC_E_ALIGN, "in_pixel_stride must be a multiple of 8 elements");
+    }
+    if (layer != RDVC_UC_FH_CONV2) {
+        const long long es = (out_dtype == RDVC_DT_F32) ? 4 : 2;
+        if (out_pixel_stride < L.n) return fail(RDVC_E_UNSUPPORTED, "out_pixel_stride %lld < %d", out_pixel_stride, L.n);
+        if ((out_pixel_stride * es) % 16) return fail(RDVC_E_ALIGN, "out_pixel_stride must be a multiple of 16 bytes");
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (layer == RDVC_UC_CONVFLOW1) {
+        rdvc::Cf1Params p;
+        memset(&p, 0, sizeof(p));
+        p.flow = flow;
+        p.fs_b = flow_strides[0]; p.fs_c = flow_strides[1]; p.fs_y = flow_strides[2]; p.fs_x = flow_strides[3];
+        p.w = packed_w; p.bias = bias; p.out = out; p.out_ps = out_pixel_stride;
+        p.B = B; p.H = H; p.W = W; p.n_pix = n_pix;
+        return op_dtype == RDVC_DT_F16 ? launch_convflow1<__half>(p, st) : launch_convflow1<__nv_bfloat16>(p, st);
+    }
+    const CUtensorMapDataType dt = (op_dtype == RDVC_DT_F16) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    CUtensorMap tm_a, tm_w;
+    {
+        const cuuint64_t px = static_cast<cuuint64_t>(in_pixel_stride) * 2, row = px * W;
+        const cuuint64_t dims[4] = {static_cast<cuuint64_t>(L.cin), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H),
+                                    static_cast<cuuint64_t>(B)};
+        const cuuint64_t strides[3] = {px, row, row * H};
+        const cuuint32_t box[4] = {64, rdvc::UC_TX, rdvc::UC_BOX_Y, 1};
+        if (int rc = make_tmap(&tm_a, dt, const_cast<void*>(in), 4, dims, strides, box)) return rc;
+    }
+    {
+        const cuuint64_t dims[3] = {64, static_cast<cuuint64_t>(L.n), static_cast<cuuint64_t>(L.cin / 64 * 9)};
+        const cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(L.n) * 128};
+        const cuuint32_t box[3] = {64, static_cast<cuuint32_t>(L.n), 1};
+        if (int rc = make_tmap(&tm_w, dt, const_cast<void*>(packed_w), 3, dims, strides, box)) return rc;
+    }
+    rdvc::UcParams p;
+    memset(&p, 0, sizeof(p));
+    p.B = B; p.H = H; p.W = W;
+    p.n_kb = L.cin / 64;
+    p.n_tx = (W + rdvc::UC_TX - 1) / rdvc::UC_TX;
+    p.n_ty = (H + rdvc::UC_TY - 1) / rdvc::UC_TY;
+    const long long n_tiles = static_cast<long long>(B) * p.n_tx * p.n_ty;
+    p.n_tiles = static_cast<int>(n_tiles);
+    p.n_super = static_cast<int>((n_tiles + rdvc::UC_P - 1) / rdvc::UC_P);
+    p.bias = bias; p.cout = L.cout;
+    p.out = out; p.out_ps = out_pixel_stride;
+    if (uses_flow) {
+        p.flow = flow;
+        p.fs_b = flow_strides[0]; p.fs_c = flow_strides[1]; p.fs_y = flow_strides[2]; p.fs_x = flow_strides[3];
+    }
+    return op_dtype == RDVC_DT_F16 ? dispatch_update_conv<__half>(layer, out_dtype, tm_a, tm_w, p, st)
+                                   : dispatch_update_conv<__nv_bfloat16>(layer, out_dtype, tm_a, tm_w, p, st);
+}
+
+size_t rdvc_corr_motion_encoder_workspace_bytes(int B, int H, int W) {
+    if (B <= 0 || H <= 0 || W <= 0) return 0;
+    return uc_plane_bytes(B, H, W, 128) + uc_plane_bytes(B, H, W, 256);
+}
+
+int rdvc_corr_motion_encoder(const void* c1, long long c1_pixel_stride, const float* flow, const long long* flow_strides, int B,
+                        int H, int W, int op_dtype, const void* const* packed_w, const float* const* bias, void* workspace,
+                        size_t workspace_bytes, void* out, long long out_pixel_stride, int out_dtype, void* stream) {
+    if (!c1 || !flow || !flow_strides || !packed_w || !bias || !workspace || !out)
+        return fail(RDVC_E_NULL, "null pointer argument");
+    for (int i = 0; i < 4; ++i)
+        if (!packed_w[i] || !bias[i]) return fail(RDVC_E_NULL, "null packed weight or bias pointer");
+    if (B <= 0 || H <= 0 || W <= 0) return fail(RDVC_E_SHAPE, "non-positive dimension B=%d H=%d W=%d", B, H, W);
+    const size_t need = rdvc_corr_motion_encoder_workspace_bytes(B, H, W);
+    if (workspace_bytes < need) return fail(RDVC_E_WORKSPACE, "workspace %zu < required %zu", workspace_bytes, need);
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(RDVC_E_ALIGN, "the workspace must be 256-byte aligned");
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    uint8_t* f1 = ws;                                            // convflow1 output (B, H, W, 128)
+    uint8_t* cf = ws + uc_plane_bytes(B, H, W, 128);             // [convcorr2 | convflow2] (B, H, W, 256)
+    // TV:raft.py:203-205: flo = convflow2(convflow1(flow)); cor = convcorr2(cor); the cat is two channel slices of cf
+    if (int rc = rdvc_corr_update_conv(RDVC_UC_CONVFLOW1, nullptr, 0, flow, flow_strides, B, H, W, op_dtype, packed_w[1], bias[1],
+                                  f1, 128, op_dtype, stream))
+        return rc;
+    if (int rc = rdvc_corr_update_conv(RDVC_UC_CONVFLOW2, f1, 128, nullptr, nullptr, B, H, W, op_dtype, packed_w[2], bias[2],
+                                  cf + 192 * 2, 256, op_dtype, stream))
+        return rc;
+    if (int rc = rdvc_corr_update_conv(RDVC_UC_CONVCORR2, c1, c1_pixel_stride, nullptr, nullptr, B, H, W, op_dtype, packed_w[0],
+                                  bias[0], cf, 256, op_dtype, stream))
+        return rc;
+    // TV:raft.py:207-210: conv(cat(cor, flo)), then cat with the flow: channels 126-127 written by the same epilogue
+    return rdvc_corr_update_conv(RDVC_UC_CONV, cf, 256, flow, flow_strides, B, H, W, op_dtype, packed_w[3], bias[3], out,
+                            out_pixel_stride, out_dtype, stream);
+}
+
+size_t rdvc_corr_flow_head_workspace_bytes(int B, int H, int W, int act_dtype) {
+    if (B <= 0 || H <= 0 || W <= 0) return 0;
+    if (act_dtype != RDVC_DT_F32 && act_dtype != RDVC_DT_F16 && act_dtype != RDVC_DT_BF16) return 0;
+    return uc_plane_bytes(B, H, W, 256) + (act_dtype == RDVC_DT_F32 ? uc_plane_bytes(B, H, W, 128) : 0);
+}
+
+int rdvc_corr_flow_head(const void* h, long long h_pixel_stride, int act_dtype, int B, int H, int W, int op_dtype,
+                   const void* const* packed_w, const float* const* bias, void* workspace, size_t workspace_bytes, void* out,
+                   void* stream) {
+    if (!h || !packed_w || !bias || !workspace || !out) return fail(RDVC_E_NULL, "null pointer argument");
+    for (int i = 0; i < 2; ++i)
+        if (!packed_w[i] || !bias[i]) return fail(RDVC_E_NULL, "null packed weight or bias pointer");
+    if (B <= 0 || H <= 0 || W <= 0) return fail(RDVC_E_SHAPE, "non-positive dimension B=%d H=%d W=%d", B, H, W);
+    if (act_dtype != RDVC_DT_F32 && act_dtype != RDVC_DT_F16 && act_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "unsupported act_dtype=%d", act_dtype);
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    if (act_dtype != RDVC_DT_F32 && act_dtype != op_dtype)
+        return fail(RDVC_E_DTYPE, "16-bit activations are their own operands: act_dtype=%d needs op_dtype=%d", act_dtype,
+                    act_dtype);
+    if (h_pixel_stride < 128) return fail(RDVC_E_UNSUPPORTED, "h_pixel_stride %lld < 128 channels", h_pixel_stride);
+    if ((reinterpret_cast<uintptr_t>(h) & 15) || ((h_pixel_stride * elem_size(act_dtype)) % 16))
+        return fail(RDVC_E_ALIGN, "h must be 16-byte aligned with a pixel stride of a multiple of 16 bytes");
+    const size_t need = rdvc_corr_flow_head_workspace_bytes(B, H, W, act_dtype);
+    if (workspace_bytes < need) return fail(RDVC_E_WORKSPACE, "workspace %zu < required %zu", workspace_bytes, need);
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(RDVC_E_ALIGN, "the workspace must be 256-byte aligned");
+    const long long n_pix = static_cast<long long>(B) * H * W;
+    if (n_pix >= (1LL << 31)) return fail(RDVC_E_UNSUPPORTED, "too many pixels for 32-bit TMA coordinates");
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    uint8_t* fh = ws;                                            // conv1 output (B, H, W, 256)
+    const void* h16 = h;
+    long long h16_ps = h_pixel_stride;
+    if (act_dtype == RDVC_DT_F32) {                              // the 16-bit operand copy of h
+        rdvc::GruCastParams cp;
+        memset(&cp, 0, sizeof(cp));
+        cp.src[0] = static_cast<const float*>(h);
+        cp.ps[0] = h_pixel_stride;
+        cp.dst[0] = ws + uc_plane_bytes(B, H, W, 256);
+        cp.n_pix = n_pix;
+        const dim3 grid(static_cast<unsigned>((n_pix * (rdvc::GRU_C / 8) + 255) / 256), 1);
+        if (op_dtype == RDVC_DT_F16) rdvc::convgru_cast_kernel<__half><<<grid, 256, 0, st>>>(cp);
+        else rdvc::convgru_cast_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(cp);
+        ++g_launches;
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return cuda_fail(e, "convgru_cast_kernel launch");
+        h16 = cp.dst[0];
+        h16_ps = 128;
+    }
+    // TV:raft.py:284-285: conv2(relu(conv1(x)))
+    if (int rc = rdvc_corr_update_conv(RDVC_UC_FH_CONV1, h16, h16_ps, nullptr, nullptr, B, H, W, op_dtype, packed_w[0], bias[0],
+                                  fh, 256, op_dtype, stream))
+        return rc;
+    return rdvc_corr_update_conv(RDVC_UC_FH_CONV2, fh, 256, nullptr, nullptr, B, H, W, op_dtype, packed_w[1], bias[1], out, 0,
+                            act_dtype, stream);
 }
 
 }  // extern "C"

@@ -25,7 +25,9 @@ the feature encoder sees each frame once.
 
 All other convolutions stay stock PyTorch/cuDNN; only the correlation block (and those two 1x1s) is this library's --
 unless the model's ``update_block.recurrent_block`` has been swapped for :class:`rc.RecurrentBlock`, which the fused
-path then hands ``context`` and the motion features as separate parts (no concatenation).
+path then hands ``context`` and the motion features as separate parts (no concatenation).  With
+:class:`rc.MotionEncoder` swapped in, the fused path has the 1x1 GEMM write convcorr1's output NHWC and the module
+reads it in place; :class:`rc.FlowHead` reads the hidden state in place.
 
 :class:`GraphedRaftFlow` replays the whole call as ONE CUDA graph per input shape.  At the reference's
 default RAFT size (368x640, R:codec_processing.py:649-650) a P-frame's ~700 kernel launches cost more
@@ -41,6 +43,7 @@ import torch.nn.functional as F
 from torch import Tensor
 
 from .corr_block import TVCorrBlock, index_pyramid
+from .motion_encoder import MotionEncoder
 from .recurrent_block import RecurrentBlock
 
 
@@ -59,15 +62,19 @@ def _update_block_fused(model, blk: TVCorrBlock, hidden_state: Tensor, context: 
     ub = model.update_block
     me = ub.motion_encoder
     conv = me.convcorr1[0]                              # Conv2dNormActivation(324, 256, norm_layer=None, kernel_size=1): [Conv2d, ReLU]
-    corr = blk.index_pyramid_convcorr1(coords1, conv.weight, conv.bias, relu=True)
-    if channels_last:
-        corr = corr.contiguous(memory_format=torch.channels_last)
-        flow = flow.contiguous(memory_format=torch.channels_last)
-    corr = me.convcorr2(corr)
-    flow_orig = flow
-    f = me.convflow2(me.convflow1(flow))
-    corr_flow = me.conv(torch.cat([corr, f], dim=1))
-    motion_features = torch.cat([corr_flow, flow_orig], dim=1)
+    if isinstance(me, MotionEncoder):       # convcorr1 writes NHWC 16-bit, the rest of the encoder reads it in place
+        motion_features = me.forward_fused(flow, blk.index_pyramid_convcorr1(coords1, conv.weight, conv.bias, relu=True,
+                                                                             nhwc=True))
+    else:
+        corr = blk.index_pyramid_convcorr1(coords1, conv.weight, conv.bias, relu=True)
+        if channels_last:
+            corr = corr.contiguous(memory_format=torch.channels_last)
+            flow = flow.contiguous(memory_format=torch.channels_last)
+        corr = me.convcorr2(corr)
+        flow_orig = flow
+        f = me.convflow2(me.convflow1(flow))
+        corr_flow = me.conv(torch.cat([corr, f], dim=1))
+        motion_features = torch.cat([corr_flow, flow_orig], dim=1)
     if isinstance(ub.recurrent_block, RecurrentBlock):       # reads context and motion features in place
         hidden_state = ub.recurrent_block.forward_parts(hidden_state, context, motion_features)
     else:
