@@ -111,6 +111,10 @@ def run_sharded(args, own_process_group=True):
         rb = rc.RecurrentBlock(input_size=256, hidden_size=ub.recurrent_block.hidden_size)
         rb.load_state_dict(ub.recurrent_block.state_dict())
         ub.motion_encoder, ub.recurrent_block, ub.flow_head = me.to(dev), rb.to(dev), fh.to(dev)
+    if getattr(args, "b200_mask_predictor", False):       # same weights, mask + convex upsampling as one fused GEMM
+        mp = rc.MaskPredictor(in_channels=128, hidden_size=256, multiplier=model.mask_predictor.multiplier)
+        mp.load_state_dict(model.mask_predictor.state_dict())
+        model.mask_predictor = mp.to(dev)
     h, w = args.height, args.width
     g = torch.Generator(device=dev).manual_seed(0)
     base = torch.rand(1, 3, h // 16 + 8, w // 16 + 8, device=dev, generator=g)
@@ -326,6 +330,8 @@ def run_sharded(args, own_process_group=True):
             line["config"]["b200_recurrent_block"] = True
         if getattr(args, "b200_update_block", False):
             line["config"]["b200_update_block"] = True
+        if getattr(args, "b200_mask_predictor", False):
+            line["config"]["b200_mask_predictor"] = True
         # flow end-point error of this configuration against STOCK torchvision RAFT (same weights, same autocast
         # setting) on one frame pair of the sequence -- outside the timed region
         a, b = frame_at(big, 3, h, w), frame_at(big, 4, h, w)
@@ -410,6 +416,9 @@ def main():
     ap.add_argument("--b200-update-block", action="store_true",
                     help="swap rc.MotionEncoder, rc.RecurrentBlock and rc.FlowHead (the whole update block as this "
                          "library's kernels) into the model")
+    ap.add_argument("--b200-mask-predictor", action="store_true",
+                    help="swap rc.MaskPredictor into the model: the mask, its softmax and the convex 8x upsampling as "
+                         "one fused GEMM")
     args = ap.parse_args()
     if args.cudnn_benchmark:
         torch.backends.cudnn.benchmark = True

@@ -364,6 +364,39 @@ int rdvc_corr_flow_head(const void* h, long long h_pixel_stride, int act_dtype, 
                    const void* const* packed_w, const float* const* bias, void* workspace, size_t workspace_bytes, void* out,
                    void* stream);
 
+/* ---- RAFT's mask predictor and the convex 8x upsampling ----------------------------------------------------- *
+ * raft_large's MaskPredictor (TV:raft.py:311-334: convrelu = 3x3 128 -> 256 + ReLU, conv = 1x1 256 -> 576, x multiplier)
+ * followed by torchvision's upsample_flow with a mask (TV:_utils.py:29-48): per output pixel (8y + i, 8x + j) a softmax
+ * over the 9 mask channels k * 64 + i * 8 + j (k = ky * 3 + kx), then the convex combination of 8 * flow at
+ * (y + ky - 1, x + kx - 1), neighbours outside the image zero (F.unfold, padding 1).  convrelu runs as FH_CONV1's
+ * kernel; the 1x1 is a tcgen05 GEMM (csrc/mask_upsample_sm100.cuh) whose epilogue does the softmax, the combination and
+ * the pixel shuffle, so the 576-channel mask never reaches memory.  16-bit operands, fp32 accumulation and epilogue.
+ *
+ * rdvc_corr_mask_conv_pack_weights (HOST, no GPU needed): conv's weight (576, 256) and bias (576), contiguous fp32 ->
+ *   rdvc_corr_mask_conv_packed_weight_bytes() bytes of 16-bit GEMM operand, packed [c][k-block][144][64], and bias_host
+ *   (576 floats), both in GEMM row order: row n = c * 144 + k * 16 + s holds stock channel k * 64 + 16 c + s (c = 0..3,
+ *   k = 0..8, s = 0..15).  Copy both to the device.  convrelu is packed with
+ *   rdvc_corr_update_conv_pack_weights(RDVC_UC_FH_CONV1, ...).
+ * rdvc_corr_mask_predictor: h: DEVICE NHWC act_dtype (F32 | F16 | BF16; 16-bit must be op_dtype), >= 128 channels at
+ *   h_pixel_stride elements (a multiple of 16 bytes), 16-byte aligned.  packed_w / bias: 2 DEVICE pointers each,
+ *   convrelu's (FH_CONV1 packing, 256 floats) then conv's (the permuted operand and bias above).  out_form:
+ *   RDVC_MASK_OUT_UPSAMPLED: flow DEVICE fp32 (B, 2, H, W) at flow[b * s[0] + c * s[1] + y * s[2] + x * s[3]],
+ *     s = flow_strides (4 HOST long longs, elements); out = the upsampled flow (B, 2, 8H, 8W) contiguous fp32.
+ *   RDVC_MASK_OUT_MASK: flow ignored; out = multiplier * conv(...) (B, 576, H, W) contiguous act_dtype, stock
+ *     channel order (MaskPredictor.forward's contract).
+ *   out 16-byte aligned.  workspace: DEVICE, rdvc_corr_mask_predictor_workspace_bytes(...), 256-byte aligned.  2 launches
+ *   (3 for F32 h).  Deterministic: no atomics, every output element is written by one thread.                       */
+#define RDVC_MASK_OUT_UPSAMPLED 0
+#define RDVC_MASK_OUT_MASK 1
+size_t rdvc_corr_mask_conv_packed_weight_bytes(void);
+int rdvc_corr_mask_conv_pack_weights(const float* weight, const float* bias, int op_dtype, void* packed_host,
+                                     float* bias_host);
+size_t rdvc_corr_mask_predictor_workspace_bytes(int B, int H, int W, int act_dtype);
+int rdvc_corr_mask_predictor(const void* h, long long h_pixel_stride, int act_dtype, int B, int H, int W, int op_dtype,
+                             const void* const* packed_w, const float* const* bias, float multiplier, const float* flow,
+                             const long long* flow_strides, int out_form, void* workspace, size_t workspace_bytes, void* out,
+                             void* stream);
+
 /* ---- next row f-4 (last piece): entropy-coder stand-in (HOST functions) ---- *
  * Stands in for the range coder behind EntropyBottleneck.compress / .decompress (R:codec_processing.py:433,447
  * construction, :488-497 compress, :509-536 decompress; compressai's RansEncoder.encode_with_indexes /

@@ -24,6 +24,7 @@
 #include "corr_pack.cuh"
 #include "convgru_sm100.cuh"
 #include "update_conv_sm100.cuh"
+#include "mask_upsample_sm100.cuh"
 #include "entropy_coder.h"
 #include "mcn_conv_sm100.cuh"
 #include "mcn_convx_sm100.cuh"
@@ -1884,6 +1885,28 @@ int dispatch_update_conv(int layer, int out_dtype, const CUtensorMap& a, const C
     }
 }
 
+// the 16-bit operand form of a 128-channel hidden state h (NHWC, pixel stride *ps): 16-bit h is used in place, fp32 h
+// is rounded to op_dtype into dst (B * H * W x 128, pixel stride 128) and *h, *ps are pointed at it
+int hidden_operand(const void** h, long long* ps, int act_dtype, int op_dtype, long long n_pix, void* dst, void* stream) {
+    if (act_dtype != RDVC_DT_F32) return RDVC_OK;
+    rdvc::GruCastParams cp;
+    memset(&cp, 0, sizeof(cp));
+    cp.src[0] = static_cast<const float*>(*h);
+    cp.ps[0] = *ps;
+    cp.dst[0] = dst;
+    cp.n_pix = n_pix;
+    const dim3 grid(static_cast<unsigned>((n_pix * (rdvc::GRU_C / 8) + 255) / 256), 1);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    if (op_dtype == RDVC_DT_F16) rdvc::convgru_cast_kernel<__half><<<grid, 256, 0, st>>>(cp);
+    else rdvc::convgru_cast_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(cp);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "convgru_cast_kernel launch");
+    *h = dst;
+    *ps = 128;
+    return RDVC_OK;
+}
+
 }  // namespace
 
 extern "C" {
@@ -2055,33 +2078,151 @@ int rdvc_corr_flow_head(const void* h, long long h_pixel_stride, int act_dtype, 
     if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(RDVC_E_ALIGN, "the workspace must be 256-byte aligned");
     const long long n_pix = static_cast<long long>(B) * H * W;
     if (n_pix >= (1LL << 31)) return fail(RDVC_E_UNSUPPORTED, "too many pixels for 32-bit TMA coordinates");
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
     uint8_t* ws = static_cast<uint8_t*>(workspace);
     uint8_t* fh = ws;                                            // conv1 output (B, H, W, 256)
     const void* h16 = h;
     long long h16_ps = h_pixel_stride;
-    if (act_dtype == RDVC_DT_F32) {                              // the 16-bit operand copy of h
-        rdvc::GruCastParams cp;
-        memset(&cp, 0, sizeof(cp));
-        cp.src[0] = static_cast<const float*>(h);
-        cp.ps[0] = h_pixel_stride;
-        cp.dst[0] = ws + uc_plane_bytes(B, H, W, 256);
-        cp.n_pix = n_pix;
-        const dim3 grid(static_cast<unsigned>((n_pix * (rdvc::GRU_C / 8) + 255) / 256), 1);
-        if (op_dtype == RDVC_DT_F16) rdvc::convgru_cast_kernel<__half><<<grid, 256, 0, st>>>(cp);
-        else rdvc::convgru_cast_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(cp);
-        ++g_launches;
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return cuda_fail(e, "convgru_cast_kernel launch");
-        h16 = cp.dst[0];
-        h16_ps = 128;
-    }
+    if (int rc = hidden_operand(&h16, &h16_ps, act_dtype, op_dtype, n_pix, ws + uc_plane_bytes(B, H, W, 256), stream))
+        return rc;
     // TV:raft.py:284-285: conv2(relu(conv1(x)))
     if (int rc = rdvc_corr_update_conv(RDVC_UC_FH_CONV1, h16, h16_ps, nullptr, nullptr, B, H, W, op_dtype, packed_w[0], bias[0],
                                   fh, 256, op_dtype, stream))
         return rc;
     return rdvc_corr_update_conv(RDVC_UC_FH_CONV2, fh, 256, nullptr, nullptr, B, H, W, op_dtype, packed_w[1], bias[1], out, 0,
                             act_dtype, stream);
+}
+
+}  // extern "C"
+
+// ---- RAFT's mask predictor with the convex 8x upsampling fused into its 1x1 GEMM -------------------------------------
+namespace {
+
+template <int EPI, typename OutT, typename OpT>
+int launch_mask_upsample(const CUtensorMap& a, const CUtensorMap& w, const rdvc::MuParams& p, cudaStream_t st) {
+    auto kern = rdvc::mask_upsample_kernel<EPI, OutT, OpT>;
+    static std::atomic<unsigned long long> attr_done{0};
+    if (int rc = ensure_dynamic_smem(kern, rdvc::MU_SMEM_LAUNCH, attr_done,
+                                     "cudaFuncSetAttribute(mask_upsample, max dynamic smem)"))
+        return rc;
+    const int grid = std::min(sm_count(), p.n_tiles);
+    kern<<<grid, rdvc::MU_THREADS, rdvc::MU_SMEM_LAUNCH, st>>>(a, w, p);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "mask_upsample_kernel launch");
+    return RDVC_OK;
+}
+
+template <typename OpT>
+int dispatch_mask_upsample(int out_form, int act_dtype, const CUtensorMap& a, const CUtensorMap& w, const rdvc::MuParams& p,
+                           cudaStream_t st) {
+    if (out_form == RDVC_MASK_OUT_UPSAMPLED) return launch_mask_upsample<rdvc::MU_EPI_UPSAMPLED, float, OpT>(a, w, p, st);
+    return act_dtype == RDVC_DT_F32 ? launch_mask_upsample<rdvc::MU_EPI_MASK, float, OpT>(a, w, p, st)
+                                    : launch_mask_upsample<rdvc::MU_EPI_MASK, OpT, OpT>(a, w, p, st);
+}
+
+}  // namespace
+
+extern "C" {
+
+size_t rdvc_corr_mask_conv_packed_weight_bytes(void) { return static_cast<size_t>(rdvc::MU_COUT) * rdvc::MU_CIN * 2; }
+
+int rdvc_corr_mask_conv_pack_weights(const float* weight, const float* bias, int op_dtype, void* packed_host,
+                                     float* bias_host) {
+    if (!weight || !bias || !packed_host || !bias_host) return fail(RDVC_E_NULL, "null pointer argument");
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    uint16_t* out = static_cast<uint16_t*>(packed_host);
+    // GEMM row n = c * 144 + k * 16 + s  <-  stock channel k * 64 + 16 c + s;  packed [c][k-block][144][64]
+    for (int c = 0; c < rdvc::MU_CHUNKS; ++c)
+        for (int k = 0; k < 9; ++k)
+            for (int s = 0; s < 16; ++s) {
+                const int row = k * 16 + s, src = k * 64 + 16 * c + s;
+                bias_host[c * rdvc::MU_NC + row] = bias[src];
+                for (int kb = 0; kb < rdvc::MU_KB; ++kb)
+                    for (int ch = 0; ch < 64; ++ch)
+                        out[((static_cast<size_t>(c) * rdvc::MU_KB + kb) * rdvc::MU_NC + row) * 64 + ch] =
+                            gru_round16(weight[static_cast<size_t>(src) * rdvc::MU_CIN + kb * 64 + ch], op_dtype);
+            }
+    return RDVC_OK;
+}
+
+size_t rdvc_corr_mask_predictor_workspace_bytes(int B, int H, int W, int act_dtype) {
+    return rdvc_corr_flow_head_workspace_bytes(B, H, W, act_dtype);      // the same two buffers: convrelu's output, h16
+}
+
+int rdvc_corr_mask_predictor(const void* h, long long h_pixel_stride, int act_dtype, int B, int H, int W, int op_dtype,
+                             const void* const* packed_w, const float* const* bias, float multiplier, const float* flow,
+                             const long long* flow_strides, int out_form, void* workspace, size_t workspace_bytes, void* out,
+                             void* stream) {
+    if (!h || !packed_w || !bias || !workspace || !out) return fail(RDVC_E_NULL, "null pointer argument");
+    for (int i = 0; i < 2; ++i)
+        if (!packed_w[i] || !bias[i]) return fail(RDVC_E_NULL, "null packed weight or bias pointer");
+    if (out_form != RDVC_MASK_OUT_UPSAMPLED && out_form != RDVC_MASK_OUT_MASK)
+        return fail(RDVC_E_UNSUPPORTED, "unknown out_form %d", out_form);
+    if (out_form == RDVC_MASK_OUT_UPSAMPLED && (!flow || !flow_strides))
+        return fail(RDVC_E_NULL, "RDVC_MASK_OUT_UPSAMPLED needs the flow and its strides");
+    if (B <= 0 || H <= 0 || W <= 0) return fail(RDVC_E_SHAPE, "non-positive dimension B=%d H=%d W=%d", B, H, W);
+    if (act_dtype != RDVC_DT_F32 && act_dtype != RDVC_DT_F16 && act_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "unsupported act_dtype=%d", act_dtype);
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    if (act_dtype != RDVC_DT_F32 && act_dtype != op_dtype)
+        return fail(RDVC_E_DTYPE, "16-bit activations are their own operands: act_dtype=%d needs op_dtype=%d", act_dtype,
+                    act_dtype);
+    if (h_pixel_stride < 128) return fail(RDVC_E_UNSUPPORTED, "h_pixel_stride %lld < 128 channels", h_pixel_stride);
+    if ((reinterpret_cast<uintptr_t>(h) & 15) || ((h_pixel_stride * elem_size(act_dtype)) % 16))
+        return fail(RDVC_E_ALIGN, "h must be 16-byte aligned with a pixel stride of a multiple of 16 bytes");
+    if ((reinterpret_cast<uintptr_t>(out) & 15) || (reinterpret_cast<uintptr_t>(packed_w[1]) & 15))
+        return fail(RDVC_E_ALIGN, "out and the packed 1x1 weights must be 16-byte aligned");
+    const size_t need = rdvc_corr_mask_predictor_workspace_bytes(B, H, W, act_dtype);
+    if (workspace_bytes < need) return fail(RDVC_E_WORKSPACE, "workspace %zu < required %zu", workspace_bytes, need);
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(RDVC_E_ALIGN, "the workspace must be 256-byte aligned");
+    const long long n_pix = static_cast<long long>(B) * H * W;
+    if (n_pix >= (1LL << 31) || H >= (1 << 24) || W >= (1 << 24))
+        return fail(RDVC_E_UNSUPPORTED, "too many pixels for 32-bit TMA coordinates");
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    uint8_t* hid = ws;                                           // convrelu output (B, H, W, 256), op_dtype
+    const void* h16 = h;
+    long long h16_ps = h_pixel_stride;
+    if (int rc = hidden_operand(&h16, &h16_ps, act_dtype, op_dtype, n_pix, ws + uc_plane_bytes(B, H, W, 256), stream))
+        return rc;
+    // TV:raft.py:331: convrelu -- the 3x3 128 -> 256 + ReLU of flow_head.conv1's shape, same kernel
+    if (int rc = rdvc_corr_update_conv(RDVC_UC_FH_CONV1, h16, h16_ps, nullptr, nullptr, B, H, W, op_dtype, packed_w[0], bias[0],
+                                       hid, 256, op_dtype, stream))
+        return rc;
+    // TV:raft.py:332-333 (conv, x multiplier) and, UPSAMPLED, TV:_utils.py:39-48 in the epilogue
+    const CUtensorMapDataType dt = (op_dtype == RDVC_DT_F16) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    CUtensorMap tm_a, tm_w;
+    {
+        const cuuint64_t px = static_cast<cuuint64_t>(rdvc::MU_CIN) * 2, row = px * W;
+        const cuuint64_t dims[4] = {static_cast<cuuint64_t>(rdvc::MU_CIN), static_cast<cuuint64_t>(W),
+                                    static_cast<cuuint64_t>(H), static_cast<cuuint64_t>(B)};
+        const cuuint64_t strides[3] = {px, row, row * H};
+        const cuuint32_t box[4] = {64, rdvc::MU_TX, rdvc::MU_TY, 1};
+        if (int rc = make_tmap(&tm_a, dt, hid, 4, dims, strides, box)) return rc;
+    }
+    {
+        const cuuint64_t dims[3] = {64, static_cast<cuuint64_t>(rdvc::MU_NC), rdvc::MU_CHUNKS * rdvc::MU_KB};
+        const cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(rdvc::MU_NC) * 128};
+        const cuuint32_t box[3] = {64, static_cast<cuuint32_t>(rdvc::MU_NC), 1};
+        if (int rc = make_tmap(&tm_w, dt, const_cast<void*>(packed_w[1]), 3, dims, strides, box)) return rc;
+    }
+    rdvc::MuParams p;
+    memset(&p, 0, sizeof(p));
+    p.B = B; p.H = H; p.W = W;
+    p.n_tx = (W + rdvc::MU_TX - 1) / rdvc::MU_TX;
+    p.n_ty = (H + rdvc::MU_TY - 1) / rdvc::MU_TY;
+    p.n_tiles = static_cast<int>(static_cast<long long>(B) * p.n_tx * p.n_ty);
+    p.bias = bias[1];
+    p.multiplier = multiplier;
+    p.out = out;
+    if (out_form == RDVC_MASK_OUT_UPSAMPLED) {
+        p.flow = flow;
+        p.fs_b = flow_strides[0]; p.fs_c = flow_strides[1]; p.fs_y = flow_strides[2]; p.fs_x = flow_strides[3];
+    }
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    return op_dtype == RDVC_DT_F16 ? dispatch_mask_upsample<__half>(out_form, act_dtype, tm_a, tm_w, p, st)
+                                   : dispatch_mask_upsample<__nv_bfloat16>(out_form, act_dtype, tm_a, tm_w, p, st);
 }
 
 }  // extern "C"

@@ -27,7 +27,9 @@ All other convolutions stay stock PyTorch/cuDNN; only the correlation block (and
 unless the model's ``update_block.recurrent_block`` has been swapped for :class:`rc.RecurrentBlock`, which the fused
 path then hands ``context`` and the motion features as separate parts (no concatenation).  With
 :class:`rc.MotionEncoder` swapped in, the fused path has the 1x1 GEMM write convcorr1's output NHWC and the module
-reads it in place; :class:`rc.FlowHead` reads the hidden state in place.
+reads it in place; :class:`rc.FlowHead` reads the hidden state in place.  With :class:`rc.MaskPredictor` as
+``model.mask_predictor`` the mask, its softmax and the convex 8x upsampling run as one GEMM epilogue
+(``MaskPredictor.upsample_flow``), in the fused and the unfused path alike.
 
 :class:`GraphedRaftFlow` replays the whole call as ONE CUDA graph per input shape.  At the reference's
 default RAFT size (368x640, R:codec_processing.py:649-650) a P-frame's ~700 kernel launches cost more
@@ -43,6 +45,7 @@ import torch.nn.functional as F
 from torch import Tensor
 
 from .corr_block import TVCorrBlock, index_pyramid
+from .mask_predictor import MaskPredictor
 from .motion_encoder import MotionEncoder
 from .recurrent_block import RecurrentBlock
 
@@ -216,8 +219,11 @@ def _raft_flow_impl(model, enc_in: Tensor, split, image1: Tensor, num_flow_updat
             hidden_state, delta_flow = model.update_block(hidden_state, context, corr_features, flow)
         coords1 = coords1 + delta_flow
         if all_predictions or it == num_flow_updates - 1:
-            up_mask = None if model.mask_predictor is None else model.mask_predictor(hidden_state).contiguous()   # upsample_flow views it
-            preds.append(upsample_flow(flow=(coords1 - coords0).contiguous(), up_mask=up_mask))
+            if isinstance(model.mask_predictor, MaskPredictor):     # mask, softmax and convex sum in one GEMM epilogue
+                preds.append(model.mask_predictor.upsample_flow(coords1 - coords0, hidden_state))
+            else:
+                up_mask = None if model.mask_predictor is None else model.mask_predictor(hidden_state).contiguous()   # upsample_flow views it
+                preds.append(upsample_flow(flow=(coords1 - coords0).contiguous(), up_mask=up_mask))
     return preds if all_predictions else preds[-1]
 
 
