@@ -115,6 +115,10 @@ def run_sharded(args, own_process_group=True):
         mp = rc.MaskPredictor(in_channels=128, hidden_size=256, multiplier=model.mask_predictor.multiplier)
         mp.load_state_dict(model.mask_predictor.state_dict())
         model.mask_predictor = mp.to(dev)
+    if getattr(args, "b200_context_encoder", False):      # same weights and BatchNorm statistics, folded into tcgen05 convolutions
+        ce = rc.ContextEncoder()
+        ce.load_state_dict(model.context_encoder.state_dict())
+        model.context_encoder = ce.to(dev).eval()
     h, w = args.height, args.width
     g = torch.Generator(device=dev).manual_seed(0)
     base = torch.rand(1, 3, h // 16 + 8, w // 16 + 8, device=dev, generator=g)
@@ -332,6 +336,8 @@ def run_sharded(args, own_process_group=True):
             line["config"]["b200_update_block"] = True
         if getattr(args, "b200_mask_predictor", False):
             line["config"]["b200_mask_predictor"] = True
+        if getattr(args, "b200_context_encoder", False):
+            line["config"]["b200_context_encoder"] = True
         # flow end-point error of this configuration against STOCK torchvision RAFT (same weights, same autocast
         # setting) on one frame pair of the sequence -- outside the timed region
         a, b = frame_at(big, 3, h, w), frame_at(big, 4, h, w)
@@ -419,6 +425,9 @@ def main():
     ap.add_argument("--b200-mask-predictor", action="store_true",
                     help="swap rc.MaskPredictor into the model: the mask, its softmax and the convex 8x upsampling as "
                          "one fused GEMM")
+    ap.add_argument("--b200-context-encoder", action="store_true",
+                    help="swap rc.ContextEncoder into the model: the context encoder with BatchNorm folded into tcgen05 "
+                         "convolutions, RAFT's tanh / relu in its last epilogue")
     args = ap.parse_args()
     if args.cudnn_benchmark:
         torch.backends.cudnn.benchmark = True

@@ -397,6 +397,49 @@ int rdvc_corr_mask_predictor(const void* h, long long h_pixel_stride, int act_dt
                              const long long* flow_strides, int out_form, void* workspace, size_t workspace_bytes, void* out,
                              void* stream);
 
+/* ---- RAFT's context encoder (torchvision FeatureEncoder, BatchNorm2d in eval mode, raft_large's configuration) ---- *
+ * The 16 convolutions, in parameter-tree order (layer index i of the pack arrays):
+ *   0 convnormrelu (7x7 s2, 3 -> 64); 1-4 layer1.{0,1}.convnormrelu{1,2} (3x3, 64 -> 64);
+ *   5 layer2.0.convnormrelu1 (3x3 s2, 64 -> 96), 6 layer2.0.downsample (1x1 s2, 64 -> 96), 7 layer2.0.convnormrelu2,
+ *   8-9 layer2.1.convnormrelu{1,2} (3x3, 96 -> 96); 10 layer3.0.convnormrelu1 (3x3 s2, 96 -> 128), 11 layer3.0.downsample,
+ *   12 layer3.0.convnormrelu2, 13-14 layer3.1.convnormrelu{1,2} (3x3, 128 -> 128); 15 conv (1x1, 128 -> 256, no BN).
+ * BatchNorm folds into the convolution in fp64: s = gamma / sqrt(var + eps), w' = w s, b' = beta + (b - mean) s, each
+ * rounded once (w' to op_dtype, b' to fp32).  Every activation between layers is NHWC op_dtype; layer2's 96 channels
+ * are stored at a 128-channel stride with channels 96-127 zero.  tcgen05 implicit GEMMs
+ * (csrc/context_encoder_sm100.cuh), 16-bit operands, fp32 accumulation and epilogues; the residual blocks' epilogue is
+ * relu(res + relu(acc + b)) (TV:raft.py:64-71); each stride-2 block's downsample runs in its first convolution.
+ *
+ * rdvc_corr_context_encoder_pack_weights (HOST, no GPU needed): per layer i, conv_w[i] (cout, cin, k, k) and conv_b[i]
+ *   (cout) contiguous fp32; for i < 15 bn_w / bn_b / bn_mean / bn_var [i] (cout) fp32 and eps[i] (entries 15 ignored).
+ *   Writes rdvc_corr_context_encoder_packed_weight_bytes() bytes of 16-bit GEMM operand to packed_host and
+ *   rdvc_corr_context_encoder_packed_bias_bytes() bytes of fp32 biases to bias_host.  Copy both to the device.
+ * rdvc_corr_context_encoder: image DEVICE (B, 3, H, W) in_dtype (F32 | F16 | BF16) at image[b * s[0] + c * s[1] + y * s[2]
+ *   + x * s[3]], s = image_strides (4 HOST long longs, elements, >= 0), aligned to its element size; any H, W >= 1.
+ *   out: DEVICE NHWC (B, ceil(H / 8), ceil(W / 8), 256) out_dtype (F32 or op_dtype) at out_pixel_stride elements (>= 256,
+ *   a multiple of 16 bytes), 16-byte aligned, overlapping neither the image nor the workspace.  out_form:
+ *   RDVC_CE_OUT_RAW: conv's output (FeatureEncoder.forward); RDVC_CE_OUT_SPLIT: tanh on channels 0-127 and ReLU on
+ *   128-255 (RAFT's hidden state and context).  workspace: DEVICE, rdvc_corr_context_encoder_workspace_bytes(...),
+ *   256-byte aligned; after the call it holds every intermediate, each in its own buffer of
+ *   align256(B * h * w * c * 2) bytes, in this order: at (H1, W1) = ceil((H, W) / 2), c = 64: the stem operand (per
+ *   pixel 4 horizontal taps x 2 row phases x 2 column phases x 3 channels, zero-padded 48 -> 64), then the outputs
+ *   of convnormrelu, layer1.0.convnormrelu1, layer1.0, layer1.1.convnormrelu1, layer1; at (H2, W2) = ceil((H1, W1) / 2),
+ *   c = 128: layer2.0.convnormrelu1, layer2.0.downsample, layer2.0, layer2.1.convnormrelu1, layer2; at (H3, W3) =
+ *   ceil((H2, W2) / 2), c = 128: the same for layer3.  15 launches.  Deterministic: no atomics; tiles never span images, so a sample's result does not
+ *   depend on the batch it is in.                                                                                   */
+#define RDVC_CE_OUT_RAW 0
+#define RDVC_CE_OUT_SPLIT 1
+#define RDVC_CE_LAYERS 16
+size_t rdvc_corr_context_encoder_packed_weight_bytes(void);
+size_t rdvc_corr_context_encoder_packed_bias_bytes(void);
+int rdvc_corr_context_encoder_pack_weights(const float* const* conv_w, const float* const* conv_b,
+                                           const float* const* bn_w, const float* const* bn_b,
+                                           const float* const* bn_mean, const float* const* bn_var, const double* eps,
+                                           int op_dtype, void* packed_host, float* bias_host);
+size_t rdvc_corr_context_encoder_workspace_bytes(int B, int H, int W, int act_dtype);
+int rdvc_corr_context_encoder(const void* image, const long long* image_strides, int in_dtype, int B, int H, int W,
+                              int op_dtype, const void* packed_w, const float* biases, int out_form, void* workspace,
+                              size_t workspace_bytes, void* out, long long out_pixel_stride, int out_dtype, void* stream);
+
 /* ---- next row f-4 (last piece): entropy-coder stand-in (HOST functions) ---- *
  * Stands in for the range coder behind EntropyBottleneck.compress / .decompress (R:codec_processing.py:433,447
  * construction, :488-497 compress, :509-536 decompress; compressai's RansEncoder.encode_with_indexes /

@@ -25,6 +25,7 @@
 #include "convgru_sm100.cuh"
 #include "update_conv_sm100.cuh"
 #include "mask_upsample_sm100.cuh"
+#include "context_encoder_sm100.cuh"
 #include "entropy_coder.h"
 #include "mcn_conv_sm100.cuh"
 #include "mcn_convx_sm100.cuh"
@@ -164,10 +165,11 @@ EncodeTiledFn encode_tiled_fn() {
 // Tiled TMA descriptor, 128-byte swizzle, zero OOB fill (loads) / clipped (stores).
 int make_tmap(CUtensorMap* m, CUtensorMapDataType dt, void* base, int rank, const cuuint64_t* dims,
               const cuuint64_t* strides_bytes, const cuuint32_t* box,
-              CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B) {
+              CUtensorMapSwizzle swizzle = CU_TENSOR_MAP_SWIZZLE_128B, const cuuint32_t* elem_strides = nullptr) {
     EncodeTiledFn fn = encode_tiled_fn();
     if (!fn) return fail(RDVC_E_DRIVER, "cuTensorMapEncodeTiled not available from the driver");
-    cuuint32_t estr[5] = {1, 1, 1, 1, 1};
+    const cuuint32_t ones[5] = {1, 1, 1, 1, 1};
+    const cuuint32_t* estr = elem_strides ? elem_strides : ones;
     CUresult r = fn(m, dt, rank, base, dims, strides_bytes, box, estr,
                     CU_TENSOR_MAP_INTERLEAVE_NONE, swizzle,
                     CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
@@ -2223,6 +2225,365 @@ int rdvc_corr_mask_predictor(const void* h, long long h_pixel_stride, int act_dt
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     return op_dtype == RDVC_DT_F16 ? dispatch_mask_upsample<__half>(out_form, act_dtype, tm_a, tm_w, p, st)
                                    : dispatch_mask_upsample<__nv_bfloat16>(out_form, act_dtype, tm_a, tm_w, p, st);
+}
+
+}  // extern "C"
+
+// ---- RAFT's context encoder: FeatureEncoder with frozen BatchNorm folded into tcgen05 convolutions ----------------
+namespace {
+
+struct CeLayer {
+    int cin, cout, k;
+};
+// indexed like the pack arrays (parameter-tree order, see include/rdvc_corr.h)
+constexpr CeLayer CE_LAYERS[RDVC_CE_LAYERS] = {
+    {3, 64, 7},   {64, 64, 3},  {64, 64, 3},  {64, 64, 3},   {64, 64, 3},   {64, 96, 3},   {64, 96, 1},   {96, 96, 3},
+    {96, 96, 3},  {96, 96, 3},  {96, 128, 3}, {96, 128, 1},  {128, 128, 3}, {128, 128, 3}, {128, 128, 3}, {128, 256, 1},
+};
+
+struct CeUnit {
+    int geom, n, n_kb, epi;
+    int conv, ds;               // layer index of the convolution and of the fused downsample (-1: none)
+};
+// one kernel launch each, in execution order
+constexpr int CE_N_UNITS = 14;
+constexpr CeUnit CE_UNITS[CE_N_UNITS] = {
+    {rdvc::CE_G_STEM, 64, 1, rdvc::CE_EPI_RELU, 0, -1},
+    {rdvc::CE_G_S1, 64, 1, rdvc::CE_EPI_RELU, 1, -1},   {rdvc::CE_G_S1, 64, 1, rdvc::CE_EPI_RES, 2, -1},
+    {rdvc::CE_G_S1, 64, 1, rdvc::CE_EPI_RELU, 3, -1},   {rdvc::CE_G_S1, 64, 1, rdvc::CE_EPI_RES, 4, -1},
+    {rdvc::CE_G_S2, 128, 1, rdvc::CE_EPI_DS, 5, 6},     {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RES, 7, -1},
+    {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RELU, 8, -1},  {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RES, 9, -1},
+    {rdvc::CE_G_S2, 128, 2, rdvc::CE_EPI_DS, 10, 11},   {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RES, 12, -1},
+    {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RELU, 13, -1}, {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RES, 14, -1},
+    {rdvc::CE_G_1X1, 256, 2, rdvc::CE_EPI_RAW, 15, -1},
+};
+
+int ce_slabs(int geom) {
+    switch (geom) {
+        case rdvc::CE_G_S1: return rdvc::CeGeom<rdvc::CE_G_S1>::SLABS;
+        case rdvc::CE_G_S2: return rdvc::CeGeom<rdvc::CE_G_S2>::SLABS;
+        case rdvc::CE_G_STEM: return rdvc::CeGeom<rdvc::CE_G_STEM>::SLABS;
+        default: return rdvc::CeGeom<rdvc::CE_G_1X1>::SLABS;
+    }
+}
+size_t ce_unit_w_elems(const CeUnit& u) { return static_cast<size_t>(u.n_kb) * ce_slabs(u.geom) * u.n * 64; }
+size_t ce_unit_b_floats(const CeUnit& u) { return static_cast<size_t>(u.n) * (u.ds >= 0 ? 2 : 1); }
+
+size_t ce_w_elems_total() {
+    size_t s = 0;
+    for (const CeUnit& u : CE_UNITS) s += ce_unit_w_elems(u);
+    return s;
+}
+size_t ce_b_floats_total() {
+    size_t s = 0;
+    for (const CeUnit& u : CE_UNITS) s += ce_unit_b_floats(u);
+    return s;
+}
+
+uint16_t ce_round16(double v, int op_dtype) {         // one rounding, fp64 -> 16 bits
+    uint16_t bits;
+    if (op_dtype == RDVC_DT_F16) { const __half hv = __double2half(v); memcpy(&bits, &hv, 2); }
+    else { const __nv_bfloat16 bv = __double2bfloat16(v); memcpy(&bits, &bv, 2); }
+    return bits;
+}
+
+// w' = w s, b' = beta + (b - mean) s with s = gamma / sqrt(var + eps), in fp64 (layer 15 has no BatchNorm)
+void ce_fold(int i, const float* const* conv_w, const float* const* conv_b, const float* const* bn_w,
+             const float* const* bn_b, const float* const* bn_mean, const float* const* bn_var, const double* eps,
+             std::vector<double>& w, std::vector<double>& b) {
+    const CeLayer& L = CE_LAYERS[i];
+    const size_t per = static_cast<size_t>(L.cin) * L.k * L.k;
+    w.assign(conv_w[i], conv_w[i] + L.cout * per);
+    b.assign(conv_b[i], conv_b[i] + L.cout);
+    if (i == RDVC_CE_LAYERS - 1) return;
+    for (int n = 0; n < L.cout; ++n) {
+        const double s = static_cast<double>(bn_w[i][n]) / std::sqrt(static_cast<double>(bn_var[i][n]) + eps[i]);
+        for (size_t e = 0; e < per; ++e) w[n * per + e] *= s;
+        b[n] = static_cast<double>(bn_b[i][n]) + (b[n] - static_cast<double>(bn_mean[i][n])) * s;
+    }
+}
+
+template <int G, int N, int EPI, typename OutT, typename OpT>
+int launch_context_conv(const CUtensorMap& a, const CUtensorMap& w, const rdvc::CeParams& p, cudaStream_t st) {
+    constexpr int SMEM = rdvc::CeCfg<G, N, EPI == rdvc::CE_EPI_DS>::SMEM_LAUNCH;
+    auto kern = rdvc::context_conv_kernel<G, N, EPI, OutT, OpT>;
+    static std::atomic<unsigned long long> attr_done{0};
+    if (int rc = ensure_dynamic_smem(kern, SMEM, attr_done, "cudaFuncSetAttribute(context_conv, max dynamic smem)"))
+        return rc;
+    const int grid = std::min(sm_count(), p.n_super);
+    kern<<<grid, rdvc::UC_THREADS, SMEM, st>>>(a, w, p);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "context_conv_kernel launch");
+    return RDVC_OK;
+}
+
+// one instantiation per (geometry, N, epilogue, output dtype, operand dtype) the unit table uses
+template <typename OpT>
+int dispatch_context_conv(const CeUnit& u, int epi, bool f32_out, const CUtensorMap& a, const CUtensorMap& w,
+                          const rdvc::CeParams& p, cudaStream_t st) {
+    using namespace rdvc;
+    switch (u.geom) {
+        case CE_G_STEM: return launch_context_conv<CE_G_STEM, 64, CE_EPI_RELU, OpT, OpT>(a, w, p, st);
+        case CE_G_S2: return launch_context_conv<CE_G_S2, 128, CE_EPI_DS, OpT, OpT>(a, w, p, st);
+        case CE_G_S1:
+            if (u.n == 64)
+                return epi == CE_EPI_RES ? launch_context_conv<CE_G_S1, 64, CE_EPI_RES, OpT, OpT>(a, w, p, st)
+                                         : launch_context_conv<CE_G_S1, 64, CE_EPI_RELU, OpT, OpT>(a, w, p, st);
+            return epi == CE_EPI_RES ? launch_context_conv<CE_G_S1, 128, CE_EPI_RES, OpT, OpT>(a, w, p, st)
+                                     : launch_context_conv<CE_G_S1, 128, CE_EPI_RELU, OpT, OpT>(a, w, p, st);
+        default:
+            if (epi == CE_EPI_SPLIT)
+                return f32_out ? launch_context_conv<CE_G_1X1, 256, CE_EPI_SPLIT, float, OpT>(a, w, p, st)
+                               : launch_context_conv<CE_G_1X1, 256, CE_EPI_SPLIT, OpT, OpT>(a, w, p, st);
+            return f32_out ? launch_context_conv<CE_G_1X1, 256, CE_EPI_RAW, float, OpT>(a, w, p, st)
+                           : launch_context_conv<CE_G_1X1, 256, CE_EPI_RAW, OpT, OpT>(a, w, p, st);
+    }
+}
+
+// one unit: input NHWC op_dtype (B, Hin, Win, n_kb * 64 of in_ps channels) -> output grid (Hout, Wout)
+int run_context_unit(const CeUnit& u, int epi, const void* in, long long in_ps, int B, int Hin, int Win, int Hout,
+                     int Wout, int op_dtype, const void* w, const float* bias, void* out, long long out_ps,
+                     int out_dtype, void* out2, const void* res, long long res_ps, cudaStream_t st) {
+    const CUtensorMapDataType dt = (op_dtype == RDVC_DT_F16) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    CUtensorMap tm_a, tm_w;
+    {
+        const cuuint64_t px = static_cast<cuuint64_t>(in_ps) * 2, row = px * Win;
+        const cuuint64_t dims[4] = {static_cast<cuuint64_t>(u.n_kb) * 64, static_cast<cuuint64_t>(Win),
+                                    static_cast<cuuint64_t>(Hin), static_cast<cuuint64_t>(B)};
+        const cuuint64_t strides[3] = {px, row, row * Hin};
+        int box_y = rdvc::CeGeom<rdvc::CE_G_1X1>::BOX_Y;
+        if (u.geom == rdvc::CE_G_S1) box_y = rdvc::CeGeom<rdvc::CE_G_S1>::BOX_Y;
+        if (u.geom == rdvc::CE_G_STEM) box_y = rdvc::CeGeom<rdvc::CE_G_STEM>::BOX_Y;
+        const bool s2 = (u.geom == rdvc::CE_G_S2);
+        // stride 2: TMA traverses every second pixel and row, a box of {32, 18} lands 16 x 9 of them
+        const cuuint32_t box[4] = {64, static_cast<cuuint32_t>(s2 ? 2 * rdvc::UC_TX : rdvc::UC_TX),
+                                   static_cast<cuuint32_t>(s2 ? 2 * rdvc::CeGeom<rdvc::CE_G_S2>::BOX_Y : box_y), 1};
+        const cuuint32_t estr[4] = {1, 2, 2, 1};
+        if (int rc = make_tmap(&tm_a, dt, const_cast<void*>(in), 4, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                               s2 ? estr : nullptr))
+            return rc;
+    }
+    {
+        const cuuint64_t dims[3] = {64, static_cast<cuuint64_t>(u.n), static_cast<cuuint64_t>(u.n_kb) * ce_slabs(u.geom)};
+        const cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(u.n) * 128};
+        const cuuint32_t box[3] = {64, static_cast<cuuint32_t>(u.n), 1};
+        if (int rc = make_tmap(&tm_w, dt, const_cast<void*>(w), 3, dims, strides, box)) return rc;
+    }
+    rdvc::CeParams p;
+    memset(&p, 0, sizeof(p));
+    p.B = B; p.H = Hout; p.W = Wout;
+    p.n_kb = u.n_kb;
+    p.n_tx = (Wout + rdvc::UC_TX - 1) / rdvc::UC_TX;
+    p.n_ty = (Hout + rdvc::UC_TY - 1) / rdvc::UC_TY;
+    const long long n_tiles = static_cast<long long>(B) * p.n_tx * p.n_ty;
+    p.n_tiles = static_cast<int>(n_tiles);
+    p.n_super = static_cast<int>((n_tiles + rdvc::UC_P - 1) / rdvc::UC_P);
+    p.bias = bias;
+    p.out = out; p.out_ps = out_ps;
+    p.out2 = out2;
+    p.res = res; p.res_ps = res_ps;
+    const bool f32 = (out_dtype == RDVC_DT_F32);
+    return op_dtype == RDVC_DT_F16 ? dispatch_context_conv<__half>(u, epi, f32, tm_a, tm_w, p, st)
+                                   : dispatch_context_conv<__nv_bfloat16>(u, epi, f32, tm_a, tm_w, p, st);
+}
+
+template <typename InT, typename OpT>
+int launch_ce_stem_pack(const rdvc::CeStemParams& p, cudaStream_t st) {
+    const long long threads = p.n_pix * 8;
+    rdvc::ce_stem_pack_kernel<InT, OpT><<<static_cast<unsigned>((threads + 255) / 256), 256, 0, st>>>(p);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "ce_stem_pack_kernel launch");
+    return RDVC_OK;
+}
+
+template <typename OpT>
+int dispatch_ce_stem_pack(int in_dtype, const rdvc::CeStemParams& p, cudaStream_t st) {
+    if (in_dtype == RDVC_DT_F32) return launch_ce_stem_pack<float, OpT>(p, st);
+    if (in_dtype == RDVC_DT_F16) return launch_ce_stem_pack<__half, OpT>(p, st);
+    return launch_ce_stem_pack<__nv_bfloat16, OpT>(p, st);
+}
+
+struct CeSizes {
+    int H1, W1, H2, W2, H3, W3;
+    size_t p1, p2, p3;          // bytes of one activation buffer per level
+};
+
+CeSizes ce_sizes(int B, int H, int W) {
+    CeSizes s;
+    s.H1 = (H + 1) / 2; s.W1 = (W + 1) / 2;
+    s.H2 = (s.H1 + 1) / 2; s.W2 = (s.W1 + 1) / 2;
+    s.H3 = (s.H2 + 1) / 2; s.W3 = (s.W2 + 1) / 2;
+    s.p1 = uc_plane_bytes(B, s.H1, s.W1, 64);
+    s.p2 = uc_plane_bytes(B, s.H2, s.W2, 128);
+    s.p3 = uc_plane_bytes(B, s.H3, s.W3, 128);
+    return s;
+}
+
+bool ranges_overlap(const void* a, size_t a_bytes, const void* b, size_t b_bytes) {
+    const uintptr_t x = reinterpret_cast<uintptr_t>(a), y = reinterpret_cast<uintptr_t>(b);
+    return x < y + b_bytes && y < x + a_bytes;
+}
+
+}  // namespace
+
+extern "C" {
+
+size_t rdvc_corr_context_encoder_packed_weight_bytes(void) { return ce_w_elems_total() * 2; }
+
+size_t rdvc_corr_context_encoder_packed_bias_bytes(void) { return ce_b_floats_total() * 4; }
+
+int rdvc_corr_context_encoder_pack_weights(const float* const* conv_w, const float* const* conv_b,
+                                           const float* const* bn_w, const float* const* bn_b,
+                                           const float* const* bn_mean, const float* const* bn_var, const double* eps,
+                                           int op_dtype, void* packed_host, float* bias_host) {
+    if (!conv_w || !conv_b || !bn_w || !bn_b || !bn_mean || !bn_var || !eps || !packed_host || !bias_host)
+        return fail(RDVC_E_NULL, "null pointer argument");
+    for (int i = 0; i < RDVC_CE_LAYERS; ++i) {
+        if (!conv_w[i] || !conv_b[i]) return fail(RDVC_E_NULL, "null weight or bias of layer %d", i);
+        if (i < RDVC_CE_LAYERS - 1 && (!bn_w[i] || !bn_b[i] || !bn_mean[i] || !bn_var[i]))
+            return fail(RDVC_E_NULL, "null BatchNorm vector of layer %d", i);
+        if (i < RDVC_CE_LAYERS - 1 && !(eps[i] >= 0.0)) return fail(RDVC_E_UNSUPPORTED, "eps[%d] = %g", i, eps[i]);
+    }
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    uint16_t* out = static_cast<uint16_t*>(packed_host);
+    memset(out, 0, ce_w_elems_total() * 2);                  // padded rows, columns and stem taps are zero
+    memset(bias_host, 0, ce_b_floats_total() * 4);
+    std::vector<double> w, b;
+    size_t wo = 0, bo = 0;
+    for (const CeUnit& u : CE_UNITS) {
+        const int S = ce_slabs(u.geom);
+        for (int part = 0; part < (u.ds >= 0 ? 2 : 1); ++part) {
+            const int li = part ? u.ds : u.conv;
+            const CeLayer& L = CE_LAYERS[li];
+            ce_fold(li, conv_w, conv_b, bn_w, bn_b, bn_mean, bn_var, eps, w, b);
+            for (int n = 0; n < L.cout; ++n) bias_host[bo + part * u.n + n] = static_cast<float>(b[n]);
+            if (u.geom == rdvc::CE_G_STEM) {                 // [ty][n][k], k = tx * 12 + py * 6 + px * 3 + c
+                for (int ty = 0; ty < 4; ++ty)
+                    for (int n = 0; n < L.cout; ++n)
+                        for (int k = 0; k < 48; ++k) {
+                            const int tx = k / 12, py = k % 12 / 6, px = k % 6 / 3, c = k % 3;
+                            const int ky = 2 * ty + py - 1, kx = 2 * tx + px - 1;
+                            if (ky < 0 || kx < 0 || ky >= 7 || kx >= 7) continue;
+                            out[wo + (static_cast<size_t>(ty) * u.n + n) * 64 + k] =
+                                ce_round16(w[((static_cast<size_t>(n) * 3 + c) * 7 + ky) * 7 + kx], op_dtype);
+                        }
+                continue;
+            }
+            const int kk = L.k * L.k;
+            for (int kb = 0; kb < u.n_kb; ++kb)               // [k-block][slab][n][64]
+                for (int t = 0; t < kk; ++t) {
+                    const int slab = part ? S - 1 : t;       // the downsample is the stride-2 unit's last slab
+                    for (int n = 0; n < L.cout; ++n)
+                        for (int c = 0; c < 64 && kb * 64 + c < L.cin; ++c)
+                            out[wo + ((static_cast<size_t>(kb) * S + slab) * u.n + n) * 64 + c] =
+                                ce_round16(w[(static_cast<size_t>(n) * L.cin + kb * 64 + c) * kk + t], op_dtype);
+                }
+        }
+        wo += ce_unit_w_elems(u);
+        bo += ce_unit_b_floats(u);
+    }
+    return RDVC_OK;
+}
+
+size_t rdvc_corr_context_encoder_workspace_bytes(int B, int H, int W, int act_dtype) {
+    if (B <= 0 || H <= 0 || W <= 0) return 0;
+    if (act_dtype != RDVC_DT_F32 && act_dtype != RDVC_DT_F16 && act_dtype != RDVC_DT_BF16) return 0;
+    const CeSizes s = ce_sizes(B, H, W);
+    return 6 * s.p1 + 5 * s.p2 + 5 * s.p3;
+}
+
+int rdvc_corr_context_encoder(const void* image, const long long* image_strides, int in_dtype, int B, int H, int W,
+                              int op_dtype, const void* packed_w, const float* biases, int out_form, void* workspace,
+                              size_t workspace_bytes, void* out, long long out_pixel_stride, int out_dtype, void* stream) {
+    if (!image || !image_strides || !packed_w || !biases || !workspace || !out) return fail(RDVC_E_NULL, "null pointer argument");
+    if (out_form != RDVC_CE_OUT_RAW && out_form != RDVC_CE_OUT_SPLIT) return fail(RDVC_E_UNSUPPORTED, "unknown out_form %d", out_form);
+    if (B <= 0 || H <= 0 || W <= 0) return fail(RDVC_E_SHAPE, "non-positive dimension B=%d H=%d W=%d", B, H, W);
+    if (in_dtype != RDVC_DT_F32 && in_dtype != RDVC_DT_F16 && in_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "unsupported in_dtype=%d", in_dtype);
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    if (out_dtype != RDVC_DT_F32 && out_dtype != op_dtype)
+        return fail(RDVC_E_DTYPE, "out_dtype=%d must be F32 or op_dtype=%d", out_dtype, op_dtype);
+    for (int i = 0; i < 4; ++i)
+        if (image_strides[i] < 0) return fail(RDVC_E_UNSUPPORTED, "negative image stride %lld", image_strides[i]);
+    if (H >= (1 << 24) || W >= (1 << 24) || static_cast<long long>(B) * ((H + 1) / 2) * ((W + 1) / 2) >= (1LL << 31))
+        return fail(RDVC_E_UNSUPPORTED, "too many pixels for 32-bit TMA coordinates");
+    const size_t in_es = elem_size(in_dtype), out_es = elem_size(out_dtype);
+    if (reinterpret_cast<uintptr_t>(image) % in_es) return fail(RDVC_E_ALIGN, "the image must be aligned to its element size");
+    if ((reinterpret_cast<uintptr_t>(packed_w) & 15) || (reinterpret_cast<uintptr_t>(biases) & 15) ||
+        (reinterpret_cast<uintptr_t>(out) & 15))
+        return fail(RDVC_E_ALIGN, "out, the packed weights and the biases must be 16-byte aligned");
+    if (out_pixel_stride < 256) return fail(RDVC_E_UNSUPPORTED, "out_pixel_stride %lld < 256", out_pixel_stride);
+    if ((out_pixel_stride * static_cast<long long>(out_es)) % 16)
+        return fail(RDVC_E_ALIGN, "out_pixel_stride must be a multiple of 16 bytes");
+    const size_t need = rdvc_corr_context_encoder_workspace_bytes(B, H, W, RDVC_DT_F32);
+    if (workspace_bytes < need) return fail(RDVC_E_WORKSPACE, "workspace %zu < required %zu", workspace_bytes, need);
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(RDVC_E_ALIGN, "the workspace must be 256-byte aligned");
+    const CeSizes s = ce_sizes(B, H, W);
+    const long long dims[4] = {B, 3, H, W};
+    size_t img_elems = 1;
+    for (int i = 0; i < 4; ++i) img_elems += static_cast<size_t>(dims[i] - 1) * static_cast<size_t>(image_strides[i]);
+    const size_t out_bytes = (static_cast<size_t>(B) * s.H3 * s.W3 - 1) * out_pixel_stride * out_es + 256 * out_es;
+    if (ranges_overlap(out, out_bytes, image, img_elems * in_es) || ranges_overlap(out, out_bytes, workspace, need))
+        return fail(RDVC_E_UNSUPPORTED, "out overlaps the image or the workspace");
+
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    // every intermediate keeps its own buffer (the layout of include/rdvc_corr.h): level 1 (H1 x W1, 64 channels)
+    // S X0 T0 X1 T1 X2, level 2 (H2 x W2, 128-channel stride) T R Y T' Z, level 3 the same
+    void* l1[6];
+    void* l2[5];
+    void* l3[5];
+    uint8_t* wsp = static_cast<uint8_t*>(workspace);
+    for (void*& q : l1) { q = wsp; wsp += s.p1; }
+    for (void*& q : l2) { q = wsp; wsp += s.p2; }
+    for (void*& q : l3) { q = wsp; wsp += s.p3; }
+
+    rdvc::CeStemParams sp;
+    memset(&sp, 0, sizeof(sp));
+    sp.img = image;
+    sp.sb = image_strides[0]; sp.sc = image_strides[1]; sp.sy = image_strides[2]; sp.sx = image_strides[3];
+    sp.H = H; sp.W = W; sp.H1 = s.H1; sp.W1 = s.W1;
+    sp.out = l1[0];
+    sp.n_pix = static_cast<long long>(B) * s.H1 * s.W1;
+    if (int rc = op_dtype == RDVC_DT_F16 ? dispatch_ce_stem_pack<__half>(in_dtype, sp, st)
+                                         : dispatch_ce_stem_pack<__nv_bfloat16>(in_dtype, sp, st))
+        return rc;
+
+    const uint8_t* wp = static_cast<const uint8_t*>(packed_w);
+    const float* bp = biases;
+    auto unit = [&](int i, const void* in, long long in_ps, int Hin, int Win, int Hout, int Wout, void* o, long long o_ps,
+                    void* o2, const void* res, long long res_ps) {
+        const CeUnit& u = CE_UNITS[i];
+        const int epi = (i == CE_N_UNITS - 1 && out_form == RDVC_CE_OUT_SPLIT) ? rdvc::CE_EPI_SPLIT : u.epi;
+        const int od = (i == CE_N_UNITS - 1) ? out_dtype : op_dtype;
+        const int rc = run_context_unit(u, epi, in, in_ps, B, Hin, Win, Hout, Wout, op_dtype, wp, bp, o, o_ps, od, o2, res,
+                                        res_ps, st);
+        wp += ce_unit_w_elems(u) * 2;
+        bp += ce_unit_b_floats(u);
+        return rc;
+    };
+    const int H1 = s.H1, W1 = s.W1, H2 = s.H2, W2 = s.W2, H3 = s.H3, W3 = s.W3;
+    int rc = 0;
+    // TV:raft.py:145: convnormrelu; 146: layer1 = two residual blocks relu(x + relu(bn2(conv2(relu(bn1(conv1(x)))))))
+    if ((rc = unit(0, l1[0], 64, H1, W1, H1, W1, l1[1], 64, nullptr, nullptr, 0))) return rc;
+    if ((rc = unit(1, l1[1], 64, H1, W1, H1, W1, l1[2], 64, nullptr, nullptr, 0))) return rc;
+    if ((rc = unit(2, l1[2], 64, H1, W1, H1, W1, l1[3], 64, nullptr, l1[1], 64))) return rc;
+    if ((rc = unit(3, l1[3], 64, H1, W1, H1, W1, l1[4], 64, nullptr, nullptr, 0))) return rc;
+    if ((rc = unit(4, l1[4], 64, H1, W1, H1, W1, l1[5], 64, nullptr, l1[3], 64))) return rc;
+    // 147: layer2; its first block's downsample is the second accumulator of its stride-2 convolution
+    if ((rc = unit(5, l1[5], 64, H1, W1, H2, W2, l2[0], 128, l2[1], nullptr, 0))) return rc;
+    if ((rc = unit(6, l2[0], 128, H2, W2, H2, W2, l2[2], 128, nullptr, l2[1], 128))) return rc;
+    if ((rc = unit(7, l2[2], 128, H2, W2, H2, W2, l2[3], 128, nullptr, nullptr, 0))) return rc;
+    if ((rc = unit(8, l2[3], 128, H2, W2, H2, W2, l2[4], 128, nullptr, l2[2], 128))) return rc;
+    // 148: layer3
+    if ((rc = unit(9, l2[4], 128, H2, W2, H3, W3, l3[0], 128, l3[1], nullptr, 0))) return rc;
+    if ((rc = unit(10, l3[0], 128, H3, W3, H3, W3, l3[2], 128, nullptr, l3[1], 128))) return rc;
+    if ((rc = unit(11, l3[2], 128, H3, W3, H3, W3, l3[3], 128, nullptr, nullptr, 0))) return rc;
+    if ((rc = unit(12, l3[3], 128, H3, W3, H3, W3, l3[4], 128, nullptr, l3[2], 128))) return rc;
+    return unit(13, l3[4], 128, H3, W3, H3, W3, out, out_pixel_stride, nullptr, nullptr, 0);
 }
 
 }  // extern "C"

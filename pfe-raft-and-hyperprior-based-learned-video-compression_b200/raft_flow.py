@@ -29,7 +29,9 @@ path then hands ``context`` and the motion features as separate parts (no concat
 :class:`rc.MotionEncoder` swapped in, the fused path has the 1x1 GEMM write convcorr1's output NHWC and the module
 reads it in place; :class:`rc.FlowHead` reads the hidden state in place.  With :class:`rc.MaskPredictor` as
 ``model.mask_predictor`` the mask, its softmax and the convex 8x upsampling run as one GEMM epilogue
-(``MaskPredictor.upsample_flow``), in the fused and the unfused path alike.
+(``MaskPredictor.upsample_flow``), in the fused and the unfused path alike.  With :class:`rc.ContextEncoder` as
+``model.context_encoder`` the hidden state and context come from ``ContextEncoder.forward_split``: RAFT's tanh and
+ReLU run in its last layer's epilogue, and both are channel slices of one NHWC buffer.
 
 :class:`GraphedRaftFlow` replays the whole call as ONE CUDA graph per input shape.  At the reference's
 default RAFT size (368x640, R:codec_processing.py:649-650) a P-frame's ~700 kernel launches cost more
@@ -44,6 +46,7 @@ import torch
 import torch.nn.functional as F
 from torch import Tensor
 
+from .context_encoder import ContextEncoder
 from .corr_block import TVCorrBlock, index_pyramid
 from .mask_predictor import MaskPredictor
 from .motion_encoder import MotionEncoder
@@ -190,20 +193,26 @@ def _raft_flow_impl(model, enc_in: Tensor, split, image1: Tensor, num_flow_updat
     # context encoder 2.6 -> 1.8 ms per P-frame at 1080p, tools/exp_update_block_layout.py, exp_encoder_layout.py).
     # The feature encoder stays NCHW: its InstanceNorm is slower in NHWC (3.1 -> 4.3 ms).
     cl = bool(update_block_channels_last) and fuse
+    own_ce = isinstance(model.context_encoder, ContextEncoder)
     if cl:
-        _to_channels_last(model.context_encoder)
+        if not own_ce:
+            _to_channels_last(model.context_encoder)
         _to_channels_last(model.update_block)
         if model.mask_predictor is not None:
             _to_channels_last(model.mask_predictor)
-        image1 = image1.contiguous(memory_format=torch.channels_last)
-    context_out = model.context_encoder(image1)
+        if not own_ce:
+            image1 = image1.contiguous(memory_format=torch.channels_last)
     hidden_size = model.update_block.hidden_state_size
-    hidden_state, context = torch.split(context_out, [hidden_size, context_out.shape[1] - hidden_size], dim=1)
-    hidden_state = torch.tanh(hidden_state)
-    context = F.relu(context)
-    if cl:      # no-ops when the context encoder already produced NHWC
-        hidden_state = hidden_state.contiguous(memory_format=torch.channels_last)
-        context = context.contiguous(memory_format=torch.channels_last)
+    if own_ce:      # tanh / relu in the last layer's epilogue; both are channel slices of one NHWC buffer
+        hidden_state, context = model.context_encoder.forward_split(image1, hidden_size)
+    else:
+        context_out = model.context_encoder(image1)
+        hidden_state, context = torch.split(context_out, [hidden_size, context_out.shape[1] - hidden_size], dim=1)
+        hidden_state = torch.tanh(hidden_state)
+        context = F.relu(context)
+        if cl:      # no-ops when the context encoder already produced NHWC
+            hidden_state = hidden_state.contiguous(memory_format=torch.channels_last)
+            context = context.contiguous(memory_format=torch.channels_last)
 
     coords0 = _coords_grid(batch, h // 8, w // 8, fmap1.device)
     coords1 = coords0.clone()
