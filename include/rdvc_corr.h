@@ -294,7 +294,7 @@ int rdvc_mcn_forward(const float* warped, const float* flow, const float* ref, i
  * rdvc_corr_convgru replaces ONE ConvGRU.forward (TV:raft.py:223-229) of torchvision's RecurrentBlock (TV:raft.py:238-270;
  * raft_large: hidden size 128, input 256 = [context | motion features], kernels (1, 5) then (5, 1)):
  *   z = sigmoid(convz([h | x])), r = sigmoid(convr([h | x])), q = tanh(convq([r * h | x])), out = (1 - z) h + z q
- * as two tcgen05 implicit GEMMs (csrc/convgru_sm100.cuh): 16-bit operands (op_dtype), fp32 accumulation, fp32
+ * as two tcgen05 implicit GEMMs (csrc/tap_conv_sm100.cuh): 16-bit operands (op_dtype), fp32 accumulation, fp32
  * epilogue; z and r * h pass through the workspace in op_dtype; the blend uses h as given (act_dtype).
  *
  * rdvc_corr_convgru_pack_weights (HOST, no GPU needed): convz / convr / convq weights, each (128, 384, 1, 5) or
@@ -320,7 +320,7 @@ int rdvc_corr_convgru(const void* h, long long h_pixel_stride, const void* conte
 
 /* ---- RAFT's motion encoder and flow head: the rest of the update block ------------------------------------- *
  * raft_large's MotionEncoder (TV:raft.py:171-211) after convcorr1 and its FlowHead (TV:raft.py:272-285) as convolutions
- * over NHWC 16-bit activations (csrc/update_conv_sm100.cuh): the 3x3 layers are tcgen05 implicit GEMMs, convflow1 (7x7,
+ * over NHWC 16-bit activations (csrc/tap_conv_sm100.cuh): the 3x3 layers are tcgen05 implicit GEMMs, convflow1 (7x7,
  * 2 -> 128) a CUDA-core direct convolution.  16-bit operands (op_dtype), fp32 accumulation, bias (+ ReLU) in fp32.
  *
  * Layers (RDVC_UC_*), torchvision weight (cout, cin, k, k) contiguous fp32:
@@ -406,7 +406,7 @@ int rdvc_corr_mask_predictor(const void* h, long long h_pixel_stride, int act_dt
  * BatchNorm folds into the convolution in fp64: s = gamma / sqrt(var + eps), w' = w s, b' = beta + (b - mean) s, each
  * rounded once (w' to op_dtype, b' to fp32).  Every activation between layers is NHWC op_dtype; layer2's 96 channels
  * are stored at a 128-channel stride with channels 96-127 zero.  tcgen05 implicit GEMMs
- * (csrc/context_encoder_sm100.cuh), 16-bit operands, fp32 accumulation and epilogues; the residual blocks' epilogue is
+ * (csrc/tap_conv_sm100.cuh), 16-bit operands, fp32 accumulation and epilogues; the residual blocks' epilogue is
  * relu(res + relu(acc + b)) (TV:raft.py:64-71); each stride-2 block's downsample runs in its first convolution.
  *
  * rdvc_corr_context_encoder_pack_weights (HOST, no GPU needed): per layer i, conv_w[i] (cout, cin, k, k) and conv_b[i]

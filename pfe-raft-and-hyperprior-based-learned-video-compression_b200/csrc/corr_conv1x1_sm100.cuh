@@ -163,7 +163,7 @@ __device__ __forceinline__ void c1_store16(OutT* dst, const float* v) {
 // tm_a: features as a {64 (8 rows x 8 elements), rows / 8, kp / 8} tensor, box {64, 16, 8}, no swizzle;
 // tm_w: packed weights {kpw, cout, 1}, box {64, cout / 2, 1}, 128-byte swizzle.
 // NHWC: the result goes out as (pixel, channel) rows of p.out_ps 16-bit elements straight from the accumulator (thread =
-// pixel, 16-byte stores, no transpose): the layout the 3x3 convolutions that follow read (update_conv_sm100.cuh).
+// pixel, 16-byte stores, no transpose): the layout the 3x3 convolutions that follow read (tap_conv_sm100.cuh).
 template <typename OutT, bool NHWC>
 __device__ __forceinline__ void corr_conv1x1_body(const CUtensorMap& tm_a, const CUtensorMap& tm_w, const Conv1x1Params p) {
     extern __shared__ uint8_t smem_raw[];

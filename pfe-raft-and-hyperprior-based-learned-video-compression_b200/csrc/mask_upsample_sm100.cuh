@@ -1,5 +1,5 @@
 // mask_upsample_sm100.cuh -- the 1x1 convolution of RAFT's mask predictor (torchvision MaskPredictor.conv, 256 -> 576,
-// TV:raft.py:311-334) as a persistent tcgen05 GEMM over the NHWC 16-bit output of convrelu (update_conv_kernel's
+// TV:raft.py:311-334) as a persistent tcgen05 GEMM over the NHWC 16-bit output of convrelu (tap_conv_kernel's
 // flow_head.conv1 instantiation), with torchvision's convex 8x upsampling (TV:_utils.py:29-48) fused into its epilogue.
 //
 // Channel mapping (torchvision): mask channel k * 64 + i * 8 + j (tap k = ky * 3 + kx) weighs neighbour
@@ -15,7 +15,7 @@
 // Weights stream from L2 in (chunk, k-block) slabs of 144 x 64 (packed [c][k-block][144][64], 18 KB) through a
 // 4-stage ring; every tile reads all 16 slabs (288 KB).
 //
-// Persistent, one CTA per SM, warp-specialised as update_conv_sm100.cuh:
+// Persistent, one CTA per SM, warp-specialised as tap_conv_sm100.cuh:
 //   warp 0     TMA producer: per tile the 4 A boxes, then the 16 weight slabs
 //   warp 1     tcgen05.mma issuer (converged warp, tcgen05 under elect_one): M128 x N144 x K16, fp32 accumulators
 //   warp 2     TMEM allocator

@@ -22,10 +22,8 @@
 #include "corr_encoder_tail_sm100.cuh"
 #include "corr_lookup.cuh"
 #include "corr_pack.cuh"
-#include "convgru_sm100.cuh"
-#include "update_conv_sm100.cuh"
 #include "mask_upsample_sm100.cuh"
-#include "context_encoder_sm100.cuh"
+#include "tap_conv_sm100.cuh"
 #include "entropy_coder.h"
 #include "mcn_conv_sm100.cuh"
 #include "mcn_convx_sm100.cuh"
@@ -1632,6 +1630,98 @@ int rdvc_mcn_forward(const float* warped, const float* flow, const float* ref, i
 
 }  // extern "C"
 
+// ---- the tap-convolution engine (tap_conv_sm100.cuh): tensor maps, tile grid, launches ----------------------------
+namespace {
+
+// {C, W, H, B} over NHWC 16-bit activations with pixel stride `ps` elements, box {64, box_x, box_y, 1}; `yx` lists y
+// before x (the GRU's 1x5 pass convolves along the map's third dimension), `s2` reads every second pixel and row
+int act_map(CUtensorMap* m, CUtensorMapDataType dt, const void* base, long long ps, int C, int B, int H, int W, int box_x,
+            int box_y, bool yx = false, bool s2 = false) {
+    const cuuint64_t px = static_cast<cuuint64_t>(ps) * 2, row = px * W;
+    const cuuint64_t dims[4] = {static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(yx ? H : W),
+                                static_cast<cuuint64_t>(yx ? W : H), static_cast<cuuint64_t>(B)};
+    const cuuint64_t strides[3] = {yx ? row : px, yx ? px : row, row * H};
+    const cuuint32_t box[4] = {64, static_cast<cuuint32_t>(box_x), static_cast<cuuint32_t>(box_y), 1};
+    const cuuint32_t estr[4] = {1, 2, 2, 1};
+    return make_tmap(m, dt, const_cast<void*>(base), 4, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
+                     s2 ? estr : nullptr);
+}
+
+// `slabs` weight slabs of n x 64 16-bit values, one slab per box
+int slab_map(CUtensorMap* m, CUtensorMapDataType dt, const void* base, int n, int slabs) {
+    const cuuint64_t dims[3] = {64, static_cast<cuuint64_t>(n), static_cast<cuuint64_t>(slabs)};
+    const cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(n) * 128};
+    const cuuint32_t box[3] = {64, static_cast<cuuint32_t>(n), 1};
+    return make_tmap(m, dt, const_cast<void*>(base), 3, dims, strides, box);
+}
+
+CUtensorMapDataType op_map_dtype(int op_dtype) {
+    return op_dtype == RDVC_DT_F16 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+}
+
+// parameters of one launch over the output grid B x H x W, with its tile grid; everything else zero
+rdvc::TapParams tap_params(int B, int H, int W, int n_kb, int horiz = 0) {
+    rdvc::TapParams p;
+    memset(&p, 0, sizeof(p));
+    p.B = B; p.H = H; p.W = W;
+    p.n_kb = n_kb;
+    p.horiz = horiz;
+    p.n_tx = ((horiz ? H : W) + rdvc::TAP_TX - 1) / rdvc::TAP_TX;
+    p.n_ty = ((horiz ? W : H) + rdvc::TAP_TY - 1) / rdvc::TAP_TY;
+    const long long n_tiles = static_cast<long long>(B) * p.n_tx * p.n_ty;
+    p.n_tiles = static_cast<int>(n_tiles);
+    p.n_super = static_cast<int>((n_tiles + rdvc::TAP_P - 1) / rdvc::TAP_P);
+    return p;
+}
+
+template <int G, int N, int EPI, typename OutT, typename OpT>
+int launch_tap_conv(const rdvc::TapMaps<rdvc::TapGeom<G>::MAPS>& maps, const rdvc::TapParams& p, cudaStream_t st) {
+    constexpr int SMEM = rdvc::TapCfg<G, N, EPI>::SMEM_LAUNCH;
+    auto kern = rdvc::tap_conv_kernel<G, N, EPI, OutT, OpT>;
+    static std::atomic<unsigned long long> attr_done{0};
+    if (int rc = ensure_dynamic_smem(kern, SMEM, attr_done, "cudaFuncSetAttribute(tap_conv, max dynamic smem)")) return rc;
+    const int grid = std::min(sm_count(), p.n_super);
+    kern<<<grid, rdvc::TAP_THREADS, SMEM, st>>>(maps, p);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "tap_conv_kernel launch");
+    return RDVC_OK;
+}
+
+// Shared memory and TMEM columns of every (geometry, N, epilogue) the dispatch tables instantiate: the tile and ring
+// sizes these kernels are measured with.  A change that moves one of them is a performance change.
+template <int G, int N, int EPI>
+constexpr bool tap_cfg_is(int smem, int tmem) {
+    return rdvc::TapCfg<G, N, EPI>::SMEM_LAUNCH == smem && rdvc::TapCfg<G, N, EPI>::TMEM_COLS == tmem;
+}
+static_assert(tap_cfg_is<rdvc::TAP_G_GRU5, 256, rdvc::TAP_EPI_GRU_ZR>(197888, 512), "GRU z|r");
+static_assert(tap_cfg_is<rdvc::TAP_G_GRU5, 128, rdvc::TAP_EPI_GRU_Q>(165120, 256), "GRU q");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 192, rdvc::TAP_EPI_RELU>(181504, 512), "convcorr2");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 64, rdvc::TAP_EPI_RELU>(115968, 128), "convflow2, layer1");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 256, rdvc::TAP_EPI_RELU>(214272, 512), "flow_head.conv1");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 128, rdvc::TAP_EPI_RELU_FLOW>(148736, 256), "conv");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 16, rdvc::TAP_EPI_FLOW2>(91392, 32), "flow_head.conv2");
+static_assert(tap_cfg_is<rdvc::TAP_G_STEM, 64, rdvc::TAP_EPI_RELU>(124160, 128), "stem");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 64, rdvc::TAP_EPI_RES>(115968, 128), "layer1 residual");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 128, rdvc::TAP_EPI_RELU>(148736, 256), "layer2/3");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 128, rdvc::TAP_EPI_RES>(148736, 256), "layer2/3 residual");
+static_assert(tap_cfg_is<rdvc::TAP_G_S2, 128, rdvc::TAP_EPI_DS>(140544, 512), "stride 2 + downsample");
+static_assert(tap_cfg_is<rdvc::TAP_G_1X1, 256, rdvc::TAP_EPI_RAW>(197888, 512), "1x1");
+static_assert(tap_cfg_is<rdvc::TAP_G_1X1, 256, rdvc::TAP_EPI_SPLIT>(197888, 512), "1x1 split");
+
+// fp32 activations -> 16-bit NHWC operand copies (128 channels of each of the first n_src sources of cp)
+int launch_gru_cast(const rdvc::GruCastParams& cp, int n_src, int op_dtype, cudaStream_t st) {
+    const dim3 grid(static_cast<unsigned>((cp.n_pix * (rdvc::GRU_C / 8) + 255) / 256), n_src);
+    if (op_dtype == RDVC_DT_F16) rdvc::convgru_cast_kernel<__half><<<grid, 256, 0, st>>>(cp);
+    else rdvc::convgru_cast_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(cp);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "convgru_cast_kernel launch");
+    return RDVC_OK;
+}
+
+}  // namespace
+
 // ---- RAFT's recurrent block: one ConvGRU pass as two tcgen05 implicit GEMMs ------------------------------------
 namespace {
 
@@ -1639,37 +1729,12 @@ size_t gru_plane_bytes(int B, int H, int W) {
     return align_up(static_cast<size_t>(B) * H * W * rdvc::GRU_C * 2, 256);
 }
 
-// {128 channels, across, along, B} over an NHWC tensor with pixel stride `ps` (16-bit elements); `horiz` lists y
-// before x so that the tap axis (x) is the map's third dimension (convgru_sm100.cuh, "Tile geometry")
-int gru_act_map(CUtensorMap* m, CUtensorMapDataType dt, const void* base, long long ps, int B, int H, int W, int horiz) {
-    const cuuint64_t px = static_cast<cuuint64_t>(ps) * 2, row = px * W;
-    const cuuint64_t dims[4] = {rdvc::GRU_C, static_cast<cuuint64_t>(horiz ? H : W), static_cast<cuuint64_t>(horiz ? W : H),
-                                static_cast<cuuint64_t>(B)};
-    const cuuint64_t strides[3] = {horiz ? row : px, horiz ? px : row, row * H};
-    const cuuint32_t box[4] = {64, rdvc::GRU_TA, rdvc::GRU_BOX_L, 1};
-    return make_tmap(m, dt, const_cast<void*>(base), 4, dims, strides, box);
-}
-
-int gru_weight_map(CUtensorMap* m, CUtensorMapDataType dt, const void* base, int n) {
-    const cuuint64_t dims[3] = {64, static_cast<cuuint64_t>(n), static_cast<cuuint64_t>(rdvc::GRU_KB * rdvc::GRU_TAPS)};
-    const cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(n) * 128};
-    const cuuint32_t box[3] = {64, static_cast<cuuint32_t>(n), 1};
-    return make_tmap(m, dt, const_cast<void*>(base), 3, dims, strides, box);
-}
-
-template <int MODE, typename ActT, typename OpT>
-int launch_convgru(const CUtensorMap& a0, const CUtensorMap& a1, const CUtensorMap& a2, const CUtensorMap& w,
-                   const rdvc::GruParams& p, cudaStream_t st) {
-    constexpr int SMEM = rdvc::GruCfg<MODE == 0 ? rdvc::GRU_ZR_N : rdvc::GRU_Q_N>::SMEM_LAUNCH;
-    auto kern = rdvc::convgru_kernel<MODE, ActT, OpT>;
-    static std::atomic<unsigned long long> attr_done{0};
-    if (int rc = ensure_dynamic_smem(kern, SMEM, attr_done, "cudaFuncSetAttribute(convgru, max dynamic smem)")) return rc;
-    const int grid = std::min(sm_count(), p.n_super);
-    kern<<<grid, rdvc::GRU_THREADS, SMEM, st>>>(a0, a1, a2, w, p);
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, MODE == 0 ? "convgru_kernel (z|r) launch" : "convgru_kernel (q) launch");
-    return RDVC_OK;
+template <typename ActT, typename OpT>
+int launch_convgru(const rdvc::TapMaps<3>& m_zr, const rdvc::TapMaps<3>& m_q, const rdvc::TapParams& p_zr,
+                   const rdvc::TapParams& p_q, cudaStream_t st) {
+    if (int rc = launch_tap_conv<rdvc::TAP_G_GRU5, rdvc::GRU_ZR_N, rdvc::TAP_EPI_GRU_ZR, ActT, OpT>(m_zr, p_zr, st))
+        return rc;
+    return launch_tap_conv<rdvc::TAP_G_GRU5, rdvc::GRU_Q_N, rdvc::TAP_EPI_GRU_Q, ActT, OpT>(m_q, p_q, st);
 }
 
 uint16_t gru_round16(float v, int op_dtype) {
@@ -1768,48 +1833,36 @@ int rdvc_corr_convgru(const void* h, long long h_pixel_stride, const void* conte
             ps16[i] = rdvc::GRU_C;
         }
         cp.n_pix = n_pix;
-        const dim3 grid(static_cast<unsigned>((n_pix * (rdvc::GRU_C / 8) + 255) / 256), 3);
-        if (op_dtype == RDVC_DT_F16) rdvc::convgru_cast_kernel<__half><<<grid, 256, 0, st>>>(cp);
-        else rdvc::convgru_cast_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(cp);
-        ++g_launches;
-        cudaError_t e = cudaGetLastError();
-        if (e != cudaSuccess) return cuda_fail(e, "convgru_cast_kernel launch");
+        if (int rc = launch_gru_cast(cp, 3, op_dtype, st)) return rc;
     }
     const int horiz = (axis == RDVC_GRU_HORIZONTAL) ? 1 : 0;
-    const CUtensorMapDataType dt = (op_dtype == RDVC_DT_F16) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-    CUtensorMap t_h, t_rh, t_ctx, t_mot, t_wzr, t_wq;
-    if (int rc = gru_act_map(&t_h, dt, a16[0], ps16[0], B, H, W, horiz)) return rc;
-    if (int rc = gru_act_map(&t_ctx, dt, a16[1], ps16[1], B, H, W, horiz)) return rc;
-    if (int rc = gru_act_map(&t_mot, dt, a16[2], ps16[2], B, H, W, horiz)) return rc;
-    if (int rc = gru_act_map(&t_rh, dt, rh, rdvc::GRU_C, B, H, W, horiz)) return rc;
-    if (int rc = gru_weight_map(&t_wzr, dt, packed_w, rdvc::GRU_ZR_N)) return rc;
-    if (int rc = gru_weight_map(&t_wq, dt, static_cast<const uint16_t*>(packed_w) + rdvc::GRU_W_ZR_ELEMS, rdvc::GRU_Q_N))
+    const CUtensorMapDataType dt = op_map_dtype(op_dtype);
+    rdvc::TapMaps<3> zr, q;                             // a: [h or r*h, context, motion]
+    for (int i = 0; i < 3; ++i)
+        if (int rc = act_map(&zr.a[i], dt, a16[i], ps16[i], rdvc::GRU_C, B, H, W, rdvc::TAP_TX,
+                             rdvc::TapGeom<rdvc::TAP_G_GRU5>::BOX_Y, horiz))
+            return rc;
+    q.a[1] = zr.a[1];
+    q.a[2] = zr.a[2];
+    if (int rc = act_map(&q.a[0], dt, rh, rdvc::GRU_C, rdvc::GRU_C, B, H, W, rdvc::TAP_TX,
+                         rdvc::TapGeom<rdvc::TAP_G_GRU5>::BOX_Y, horiz))
+        return rc;
+    constexpr int SLABS = rdvc::GRU_KB * rdvc::GRU_TAPS;
+    if (int rc = slab_map(&zr.w, dt, packed_w, rdvc::GRU_ZR_N, SLABS)) return rc;
+    if (int rc = slab_map(&q.w, dt, static_cast<const uint16_t*>(packed_w) + rdvc::GRU_W_ZR_ELEMS, rdvc::GRU_Q_N, SLABS))
         return rc;
 
-    rdvc::GruParams p;
-    memset(&p, 0, sizeof(p));
-    p.B = B; p.H = H; p.W = W; p.horiz = horiz;
-    p.n_across = ((horiz ? H : W) + rdvc::GRU_TA - 1) / rdvc::GRU_TA;
-    p.n_along = ((horiz ? W : H) + rdvc::GRU_TL - 1) / rdvc::GRU_TL;
-    const long long n_tiles = static_cast<long long>(B) * p.n_across * p.n_along;
-    p.n_tiles = static_cast<int>(n_tiles);
-    p.n_super = static_cast<int>((n_tiles + rdvc::GRU_P - 1) / rdvc::GRU_P);
-    p.h = h; p.h_ps = ps[0];
-    p.z = z; p.rh = rh; p.out = out;
-    // the z|r pass reads bias0 = bz, bias1 = br; the q pass reads bias0 = bq (set between the launches)
-    p.bias0 = bias_z; p.bias1 = bias_r;
-    if (int rc = (act_dtype == RDVC_DT_F32 && op_dtype == RDVC_DT_F16)
-                     ? launch_convgru<0, float, __half>(t_h, t_ctx, t_mot, t_wzr, p, st)
-                 : (act_dtype == RDVC_DT_F32)   ? launch_convgru<0, float, __nv_bfloat16>(t_h, t_ctx, t_mot, t_wzr, p, st)
-                 : (op_dtype == RDVC_DT_F16)    ? launch_convgru<0, __half, __half>(t_h, t_ctx, t_mot, t_wzr, p, st)
-                                                : launch_convgru<0, __nv_bfloat16, __nv_bfloat16>(t_h, t_ctx, t_mot, t_wzr, p, st))
-        return rc;
-    p.bias0 = bias_q; p.bias1 = nullptr;
-    return (act_dtype == RDVC_DT_F32 && op_dtype == RDVC_DT_F16)
-               ? launch_convgru<1, float, __half>(t_rh, t_ctx, t_mot, t_wq, p, st)
-           : (act_dtype == RDVC_DT_F32) ? launch_convgru<1, float, __nv_bfloat16>(t_rh, t_ctx, t_mot, t_wq, p, st)
-           : (op_dtype == RDVC_DT_F16)  ? launch_convgru<1, __half, __half>(t_rh, t_ctx, t_mot, t_wq, p, st)
-                                        : launch_convgru<1, __nv_bfloat16, __nv_bfloat16>(t_rh, t_ctx, t_mot, t_wq, p, st);
+    rdvc::TapParams p_zr = tap_params(B, H, W, rdvc::GRU_KB, horiz);
+    p_zr.res = h; p_zr.res_ps = ps[0];
+    rdvc::TapParams p_q = p_zr;
+    p_zr.bias = bias_z; p_zr.bias_r = bias_r;
+    p_zr.out = z; p_zr.out2 = rh;
+    p_q.bias = bias_q;
+    p_q.z = z; p_q.out = out;
+    return (act_dtype == RDVC_DT_F32 && op_dtype == RDVC_DT_F16) ? launch_convgru<float, __half>(zr, q, p_zr, p_q, st)
+           : (act_dtype == RDVC_DT_F32) ? launch_convgru<float, __nv_bfloat16>(zr, q, p_zr, p_q, st)
+           : (op_dtype == RDVC_DT_F16)  ? launch_convgru<__half, __half>(zr, q, p_zr, p_q, st)
+                                        : launch_convgru<__nv_bfloat16, __nv_bfloat16>(zr, q, p_zr, p_q, st);
 }
 
 }  // extern "C"
@@ -1840,20 +1893,6 @@ size_t uc_plane_bytes(int B, int H, int W, int channels) {
     return align_up(static_cast<size_t>(B) * H * W * channels * 2, 256);
 }
 
-template <int N, int EPI, typename OutT, typename OpT>
-int launch_update_conv(const CUtensorMap& a, const CUtensorMap& w, const rdvc::UcParams& p, cudaStream_t st) {
-    constexpr int SMEM = rdvc::UcCfg<N>::SMEM_LAUNCH;
-    auto kern = rdvc::update_conv_kernel<N, EPI, OutT, OpT>;
-    static std::atomic<unsigned long long> attr_done{0};
-    if (int rc = ensure_dynamic_smem(kern, SMEM, attr_done, "cudaFuncSetAttribute(update_conv, max dynamic smem)")) return rc;
-    const int grid = std::min(sm_count(), p.n_super);
-    kern<<<grid, rdvc::UC_THREADS, SMEM, st>>>(a, w, p);
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "update_conv_kernel launch");
-    return RDVC_OK;
-}
-
 template <typename OpT>
 int launch_convflow1(const rdvc::Cf1Params& p, cudaStream_t st) {
     auto kern = rdvc::convflow1_kernel<OpT>;
@@ -1871,19 +1910,19 @@ int launch_convflow1(const rdvc::Cf1Params& p, cudaStream_t st) {
 
 // the 3x3 layers' dispatch: one instantiation per (layer, output dtype, operand dtype)
 template <typename OpT>
-int dispatch_update_conv(int layer, int out_dtype, const CUtensorMap& a, const CUtensorMap& w, const rdvc::UcParams& p,
-                         cudaStream_t st) {
+int dispatch_update_conv(int layer, int out_dtype, const rdvc::TapMaps<1>& m, const rdvc::TapParams& p, cudaStream_t st) {
+    using namespace rdvc;
     const bool f32 = (out_dtype == RDVC_DT_F32);
     switch (layer) {
-        case RDVC_UC_CONVCORR2: return launch_update_conv<192, rdvc::UC_EPI_RELU, OpT, OpT>(a, w, p, st);
-        case RDVC_UC_CONVFLOW2: return launch_update_conv<64, rdvc::UC_EPI_RELU, OpT, OpT>(a, w, p, st);
-        case RDVC_UC_FH_CONV1: return launch_update_conv<256, rdvc::UC_EPI_RELU, OpT, OpT>(a, w, p, st);
+        case RDVC_UC_CONVCORR2: return launch_tap_conv<TAP_G_S1, 192, TAP_EPI_RELU, OpT, OpT>(m, p, st);
+        case RDVC_UC_CONVFLOW2: return launch_tap_conv<TAP_G_S1, 64, TAP_EPI_RELU, OpT, OpT>(m, p, st);
+        case RDVC_UC_FH_CONV1: return launch_tap_conv<TAP_G_S1, 256, TAP_EPI_RELU, OpT, OpT>(m, p, st);
         case RDVC_UC_CONV:
-            return f32 ? launch_update_conv<128, rdvc::UC_EPI_RELU_FLOW, float, OpT>(a, w, p, st)
-                       : launch_update_conv<128, rdvc::UC_EPI_RELU_FLOW, OpT, OpT>(a, w, p, st);
+            return f32 ? launch_tap_conv<TAP_G_S1, 128, TAP_EPI_RELU_FLOW, float, OpT>(m, p, st)
+                       : launch_tap_conv<TAP_G_S1, 128, TAP_EPI_RELU_FLOW, OpT, OpT>(m, p, st);
         default:
-            return f32 ? launch_update_conv<16, rdvc::UC_EPI_FLOW2, float, OpT>(a, w, p, st)
-                       : launch_update_conv<16, rdvc::UC_EPI_FLOW2, OpT, OpT>(a, w, p, st);
+            return f32 ? launch_tap_conv<TAP_G_S1, 16, TAP_EPI_FLOW2, float, OpT>(m, p, st)
+                       : launch_tap_conv<TAP_G_S1, 16, TAP_EPI_FLOW2, OpT, OpT>(m, p, st);
     }
 }
 
@@ -1897,13 +1936,7 @@ int hidden_operand(const void** h, long long* ps, int act_dtype, int op_dtype, l
     cp.ps[0] = *ps;
     cp.dst[0] = dst;
     cp.n_pix = n_pix;
-    const dim3 grid(static_cast<unsigned>((n_pix * (rdvc::GRU_C / 8) + 255) / 256), 1);
-    cudaStream_t st = static_cast<cudaStream_t>(stream);
-    if (op_dtype == RDVC_DT_F16) rdvc::convgru_cast_kernel<__half><<<grid, 256, 0, st>>>(cp);
-    else rdvc::convgru_cast_kernel<__nv_bfloat16><<<grid, 256, 0, st>>>(cp);
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "convgru_cast_kernel launch");
+    if (int rc = launch_gru_cast(cp, 1, op_dtype, static_cast<cudaStream_t>(stream))) return rc;
     *h = dst;
     *ps = 128;
     return RDVC_OK;
@@ -1983,39 +2016,21 @@ int rdvc_corr_update_conv(int layer, const void* in, long long in_pixel_stride, 
         p.B = B; p.H = H; p.W = W; p.n_pix = n_pix;
         return op_dtype == RDVC_DT_F16 ? launch_convflow1<__half>(p, st) : launch_convflow1<__nv_bfloat16>(p, st);
     }
-    const CUtensorMapDataType dt = (op_dtype == RDVC_DT_F16) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-    CUtensorMap tm_a, tm_w;
-    {
-        const cuuint64_t px = static_cast<cuuint64_t>(in_pixel_stride) * 2, row = px * W;
-        const cuuint64_t dims[4] = {static_cast<cuuint64_t>(L.cin), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H),
-                                    static_cast<cuuint64_t>(B)};
-        const cuuint64_t strides[3] = {px, row, row * H};
-        const cuuint32_t box[4] = {64, rdvc::UC_TX, rdvc::UC_BOX_Y, 1};
-        if (int rc = make_tmap(&tm_a, dt, const_cast<void*>(in), 4, dims, strides, box)) return rc;
-    }
-    {
-        const cuuint64_t dims[3] = {64, static_cast<cuuint64_t>(L.n), static_cast<cuuint64_t>(L.cin / 64 * 9)};
-        const cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(L.n) * 128};
-        const cuuint32_t box[3] = {64, static_cast<cuuint32_t>(L.n), 1};
-        if (int rc = make_tmap(&tm_w, dt, const_cast<void*>(packed_w), 3, dims, strides, box)) return rc;
-    }
-    rdvc::UcParams p;
-    memset(&p, 0, sizeof(p));
-    p.B = B; p.H = H; p.W = W;
-    p.n_kb = L.cin / 64;
-    p.n_tx = (W + rdvc::UC_TX - 1) / rdvc::UC_TX;
-    p.n_ty = (H + rdvc::UC_TY - 1) / rdvc::UC_TY;
-    const long long n_tiles = static_cast<long long>(B) * p.n_tx * p.n_ty;
-    p.n_tiles = static_cast<int>(n_tiles);
-    p.n_super = static_cast<int>((n_tiles + rdvc::UC_P - 1) / rdvc::UC_P);
+    const CUtensorMapDataType dt = op_map_dtype(op_dtype);
+    rdvc::TapMaps<1> m;
+    if (int rc = act_map(&m.a[0], dt, in, in_pixel_stride, L.cin, B, H, W, rdvc::TAP_TX,
+                         rdvc::TapGeom<rdvc::TAP_G_S1>::BOX_Y))
+        return rc;
+    if (int rc = slab_map(&m.w, dt, packed_w, L.n, L.cin / 64 * 9)) return rc;
+    rdvc::TapParams p = tap_params(B, H, W, L.cin / 64);
     p.bias = bias; p.cout = L.cout;
     p.out = out; p.out_ps = out_pixel_stride;
     if (uses_flow) {
         p.flow = flow;
         p.fs_b = flow_strides[0]; p.fs_c = flow_strides[1]; p.fs_y = flow_strides[2]; p.fs_x = flow_strides[3];
     }
-    return op_dtype == RDVC_DT_F16 ? dispatch_update_conv<__half>(layer, out_dtype, tm_a, tm_w, p, st)
-                                   : dispatch_update_conv<__nv_bfloat16>(layer, out_dtype, tm_a, tm_w, p, st);
+    return op_dtype == RDVC_DT_F16 ? dispatch_update_conv<__half>(layer, out_dtype, m, p, st)
+                                   : dispatch_update_conv<__nv_bfloat16>(layer, out_dtype, m, p, st);
 }
 
 size_t rdvc_corr_motion_encoder_workspace_bytes(int B, int H, int W) {
@@ -2193,22 +2208,10 @@ int rdvc_corr_mask_predictor(const void* h, long long h_pixel_stride, int act_dt
                                        hid, 256, op_dtype, stream))
         return rc;
     // TV:raft.py:332-333 (conv, x multiplier) and, UPSAMPLED, TV:_utils.py:39-48 in the epilogue
-    const CUtensorMapDataType dt = (op_dtype == RDVC_DT_F16) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
+    const CUtensorMapDataType dt = op_map_dtype(op_dtype);
     CUtensorMap tm_a, tm_w;
-    {
-        const cuuint64_t px = static_cast<cuuint64_t>(rdvc::MU_CIN) * 2, row = px * W;
-        const cuuint64_t dims[4] = {static_cast<cuuint64_t>(rdvc::MU_CIN), static_cast<cuuint64_t>(W),
-                                    static_cast<cuuint64_t>(H), static_cast<cuuint64_t>(B)};
-        const cuuint64_t strides[3] = {px, row, row * H};
-        const cuuint32_t box[4] = {64, rdvc::MU_TX, rdvc::MU_TY, 1};
-        if (int rc = make_tmap(&tm_a, dt, hid, 4, dims, strides, box)) return rc;
-    }
-    {
-        const cuuint64_t dims[3] = {64, static_cast<cuuint64_t>(rdvc::MU_NC), rdvc::MU_CHUNKS * rdvc::MU_KB};
-        const cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(rdvc::MU_NC) * 128};
-        const cuuint32_t box[3] = {64, static_cast<cuuint32_t>(rdvc::MU_NC), 1};
-        if (int rc = make_tmap(&tm_w, dt, const_cast<void*>(packed_w[1]), 3, dims, strides, box)) return rc;
-    }
+    if (int rc = act_map(&tm_a, dt, hid, rdvc::MU_CIN, rdvc::MU_CIN, B, H, W, rdvc::MU_TX, rdvc::MU_TY)) return rc;
+    if (int rc = slab_map(&tm_w, dt, packed_w[1], rdvc::MU_NC, rdvc::MU_CHUNKS * rdvc::MU_KB)) return rc;
     rdvc::MuParams p;
     memset(&p, 0, sizeof(p));
     p.B = B; p.H = H; p.W = W;
@@ -2248,25 +2251,30 @@ struct CeUnit {
 // one kernel launch each, in execution order
 constexpr int CE_N_UNITS = 14;
 constexpr CeUnit CE_UNITS[CE_N_UNITS] = {
-    {rdvc::CE_G_STEM, 64, 1, rdvc::CE_EPI_RELU, 0, -1},
-    {rdvc::CE_G_S1, 64, 1, rdvc::CE_EPI_RELU, 1, -1},   {rdvc::CE_G_S1, 64, 1, rdvc::CE_EPI_RES, 2, -1},
-    {rdvc::CE_G_S1, 64, 1, rdvc::CE_EPI_RELU, 3, -1},   {rdvc::CE_G_S1, 64, 1, rdvc::CE_EPI_RES, 4, -1},
-    {rdvc::CE_G_S2, 128, 1, rdvc::CE_EPI_DS, 5, 6},     {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RES, 7, -1},
-    {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RELU, 8, -1},  {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RES, 9, -1},
-    {rdvc::CE_G_S2, 128, 2, rdvc::CE_EPI_DS, 10, 11},   {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RES, 12, -1},
-    {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RELU, 13, -1}, {rdvc::CE_G_S1, 128, 2, rdvc::CE_EPI_RES, 14, -1},
-    {rdvc::CE_G_1X1, 256, 2, rdvc::CE_EPI_RAW, 15, -1},
+    {rdvc::TAP_G_STEM, 64, 1, rdvc::TAP_EPI_RELU, 0, -1},
+    {rdvc::TAP_G_S1, 64, 1, rdvc::TAP_EPI_RELU, 1, -1},   {rdvc::TAP_G_S1, 64, 1, rdvc::TAP_EPI_RES, 2, -1},
+    {rdvc::TAP_G_S1, 64, 1, rdvc::TAP_EPI_RELU, 3, -1},   {rdvc::TAP_G_S1, 64, 1, rdvc::TAP_EPI_RES, 4, -1},
+    {rdvc::TAP_G_S2, 128, 1, rdvc::TAP_EPI_DS, 5, 6},     {rdvc::TAP_G_S1, 128, 2, rdvc::TAP_EPI_RES, 7, -1},
+    {rdvc::TAP_G_S1, 128, 2, rdvc::TAP_EPI_RELU, 8, -1},  {rdvc::TAP_G_S1, 128, 2, rdvc::TAP_EPI_RES, 9, -1},
+    {rdvc::TAP_G_S2, 128, 2, rdvc::TAP_EPI_DS, 10, 11},   {rdvc::TAP_G_S1, 128, 2, rdvc::TAP_EPI_RES, 12, -1},
+    {rdvc::TAP_G_S1, 128, 2, rdvc::TAP_EPI_RELU, 13, -1}, {rdvc::TAP_G_S1, 128, 2, rdvc::TAP_EPI_RES, 14, -1},
+    {rdvc::TAP_G_1X1, 256, 2, rdvc::TAP_EPI_RAW, 15, -1},
 };
 
-int ce_slabs(int geom) {
+// slabs per k-block and box height of a geometry
+struct CeGeomSizes {
+    int slabs, box_y;
+};
+CeGeomSizes ce_geom(int geom) {
+    using namespace rdvc;
     switch (geom) {
-        case rdvc::CE_G_S1: return rdvc::CeGeom<rdvc::CE_G_S1>::SLABS;
-        case rdvc::CE_G_S2: return rdvc::CeGeom<rdvc::CE_G_S2>::SLABS;
-        case rdvc::CE_G_STEM: return rdvc::CeGeom<rdvc::CE_G_STEM>::SLABS;
-        default: return rdvc::CeGeom<rdvc::CE_G_1X1>::SLABS;
+        case TAP_G_S1: return {TapGeom<TAP_G_S1>::SLABS, TapGeom<TAP_G_S1>::BOX_Y};
+        case TAP_G_S2: return {TapGeom<TAP_G_S2>::SLABS, TapGeom<TAP_G_S2>::BOX_Y};
+        case TAP_G_STEM: return {TapGeom<TAP_G_STEM>::SLABS, TapGeom<TAP_G_STEM>::BOX_Y};
+        default: return {TapGeom<TAP_G_1X1>::SLABS, TapGeom<TAP_G_1X1>::BOX_Y};
     }
 }
-size_t ce_unit_w_elems(const CeUnit& u) { return static_cast<size_t>(u.n_kb) * ce_slabs(u.geom) * u.n * 64; }
+size_t ce_unit_w_elems(const CeUnit& u) { return static_cast<size_t>(u.n_kb) * ce_geom(u.geom).slabs * u.n * 64; }
 size_t ce_unit_b_floats(const CeUnit& u) { return static_cast<size_t>(u.n) * (u.ds >= 0 ? 2 : 1); }
 
 size_t ce_w_elems_total() {
@@ -2303,41 +2311,26 @@ void ce_fold(int i, const float* const* conv_w, const float* const* conv_b, cons
     }
 }
 
-template <int G, int N, int EPI, typename OutT, typename OpT>
-int launch_context_conv(const CUtensorMap& a, const CUtensorMap& w, const rdvc::CeParams& p, cudaStream_t st) {
-    constexpr int SMEM = rdvc::CeCfg<G, N, EPI == rdvc::CE_EPI_DS>::SMEM_LAUNCH;
-    auto kern = rdvc::context_conv_kernel<G, N, EPI, OutT, OpT>;
-    static std::atomic<unsigned long long> attr_done{0};
-    if (int rc = ensure_dynamic_smem(kern, SMEM, attr_done, "cudaFuncSetAttribute(context_conv, max dynamic smem)"))
-        return rc;
-    const int grid = std::min(sm_count(), p.n_super);
-    kern<<<grid, rdvc::UC_THREADS, SMEM, st>>>(a, w, p);
-    ++g_launches;
-    cudaError_t e = cudaGetLastError();
-    if (e != cudaSuccess) return cuda_fail(e, "context_conv_kernel launch");
-    return RDVC_OK;
-}
-
 // one instantiation per (geometry, N, epilogue, output dtype, operand dtype) the unit table uses
 template <typename OpT>
-int dispatch_context_conv(const CeUnit& u, int epi, bool f32_out, const CUtensorMap& a, const CUtensorMap& w,
-                          const rdvc::CeParams& p, cudaStream_t st) {
+int dispatch_context_conv(const CeUnit& u, int epi, bool f32_out, const rdvc::TapMaps<1>& m, const rdvc::TapParams& p,
+                          cudaStream_t st) {
     using namespace rdvc;
     switch (u.geom) {
-        case CE_G_STEM: return launch_context_conv<CE_G_STEM, 64, CE_EPI_RELU, OpT, OpT>(a, w, p, st);
-        case CE_G_S2: return launch_context_conv<CE_G_S2, 128, CE_EPI_DS, OpT, OpT>(a, w, p, st);
-        case CE_G_S1:
+        case TAP_G_STEM: return launch_tap_conv<TAP_G_STEM, 64, TAP_EPI_RELU, OpT, OpT>(m, p, st);
+        case TAP_G_S2: return launch_tap_conv<TAP_G_S2, 128, TAP_EPI_DS, OpT, OpT>(m, p, st);
+        case TAP_G_S1:
             if (u.n == 64)
-                return epi == CE_EPI_RES ? launch_context_conv<CE_G_S1, 64, CE_EPI_RES, OpT, OpT>(a, w, p, st)
-                                         : launch_context_conv<CE_G_S1, 64, CE_EPI_RELU, OpT, OpT>(a, w, p, st);
-            return epi == CE_EPI_RES ? launch_context_conv<CE_G_S1, 128, CE_EPI_RES, OpT, OpT>(a, w, p, st)
-                                     : launch_context_conv<CE_G_S1, 128, CE_EPI_RELU, OpT, OpT>(a, w, p, st);
+                return epi == TAP_EPI_RES ? launch_tap_conv<TAP_G_S1, 64, TAP_EPI_RES, OpT, OpT>(m, p, st)
+                                          : launch_tap_conv<TAP_G_S1, 64, TAP_EPI_RELU, OpT, OpT>(m, p, st);
+            return epi == TAP_EPI_RES ? launch_tap_conv<TAP_G_S1, 128, TAP_EPI_RES, OpT, OpT>(m, p, st)
+                                      : launch_tap_conv<TAP_G_S1, 128, TAP_EPI_RELU, OpT, OpT>(m, p, st);
         default:
-            if (epi == CE_EPI_SPLIT)
-                return f32_out ? launch_context_conv<CE_G_1X1, 256, CE_EPI_SPLIT, float, OpT>(a, w, p, st)
-                               : launch_context_conv<CE_G_1X1, 256, CE_EPI_SPLIT, OpT, OpT>(a, w, p, st);
-            return f32_out ? launch_context_conv<CE_G_1X1, 256, CE_EPI_RAW, float, OpT>(a, w, p, st)
-                           : launch_context_conv<CE_G_1X1, 256, CE_EPI_RAW, OpT, OpT>(a, w, p, st);
+            if (epi == TAP_EPI_SPLIT)
+                return f32_out ? launch_tap_conv<TAP_G_1X1, 256, TAP_EPI_SPLIT, float, OpT>(m, p, st)
+                               : launch_tap_conv<TAP_G_1X1, 256, TAP_EPI_SPLIT, OpT, OpT>(m, p, st);
+            return f32_out ? launch_tap_conv<TAP_G_1X1, 256, TAP_EPI_RAW, float, OpT>(m, p, st)
+                           : launch_tap_conv<TAP_G_1X1, 256, TAP_EPI_RAW, OpT, OpT>(m, p, st);
     }
 }
 
@@ -2345,47 +2338,21 @@ int dispatch_context_conv(const CeUnit& u, int epi, bool f32_out, const CUtensor
 int run_context_unit(const CeUnit& u, int epi, const void* in, long long in_ps, int B, int Hin, int Win, int Hout,
                      int Wout, int op_dtype, const void* w, const float* bias, void* out, long long out_ps,
                      int out_dtype, void* out2, const void* res, long long res_ps, cudaStream_t st) {
-    const CUtensorMapDataType dt = (op_dtype == RDVC_DT_F16) ? CU_TENSOR_MAP_DATA_TYPE_FLOAT16 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16;
-    CUtensorMap tm_a, tm_w;
-    {
-        const cuuint64_t px = static_cast<cuuint64_t>(in_ps) * 2, row = px * Win;
-        const cuuint64_t dims[4] = {static_cast<cuuint64_t>(u.n_kb) * 64, static_cast<cuuint64_t>(Win),
-                                    static_cast<cuuint64_t>(Hin), static_cast<cuuint64_t>(B)};
-        const cuuint64_t strides[3] = {px, row, row * Hin};
-        int box_y = rdvc::CeGeom<rdvc::CE_G_1X1>::BOX_Y;
-        if (u.geom == rdvc::CE_G_S1) box_y = rdvc::CeGeom<rdvc::CE_G_S1>::BOX_Y;
-        if (u.geom == rdvc::CE_G_STEM) box_y = rdvc::CeGeom<rdvc::CE_G_STEM>::BOX_Y;
-        const bool s2 = (u.geom == rdvc::CE_G_S2);
-        // stride 2: TMA traverses every second pixel and row, a box of {32, 18} lands 16 x 9 of them
-        const cuuint32_t box[4] = {64, static_cast<cuuint32_t>(s2 ? 2 * rdvc::UC_TX : rdvc::UC_TX),
-                                   static_cast<cuuint32_t>(s2 ? 2 * rdvc::CeGeom<rdvc::CE_G_S2>::BOX_Y : box_y), 1};
-        const cuuint32_t estr[4] = {1, 2, 2, 1};
-        if (int rc = make_tmap(&tm_a, dt, const_cast<void*>(in), 4, dims, strides, box, CU_TENSOR_MAP_SWIZZLE_128B,
-                               s2 ? estr : nullptr))
-            return rc;
-    }
-    {
-        const cuuint64_t dims[3] = {64, static_cast<cuuint64_t>(u.n), static_cast<cuuint64_t>(u.n_kb) * ce_slabs(u.geom)};
-        const cuuint64_t strides[2] = {128, static_cast<cuuint64_t>(u.n) * 128};
-        const cuuint32_t box[3] = {64, static_cast<cuuint32_t>(u.n), 1};
-        if (int rc = make_tmap(&tm_w, dt, const_cast<void*>(w), 3, dims, strides, box)) return rc;
-    }
-    rdvc::CeParams p;
-    memset(&p, 0, sizeof(p));
-    p.B = B; p.H = Hout; p.W = Wout;
-    p.n_kb = u.n_kb;
-    p.n_tx = (Wout + rdvc::UC_TX - 1) / rdvc::UC_TX;
-    p.n_ty = (Hout + rdvc::UC_TY - 1) / rdvc::UC_TY;
-    const long long n_tiles = static_cast<long long>(B) * p.n_tx * p.n_ty;
-    p.n_tiles = static_cast<int>(n_tiles);
-    p.n_super = static_cast<int>((n_tiles + rdvc::UC_P - 1) / rdvc::UC_P);
+    const CUtensorMapDataType dt = op_map_dtype(op_dtype);
+    const CeGeomSizes g = ce_geom(u.geom);
+    const int k = (u.geom == rdvc::TAP_G_S2) ? 2 : 1;      // stride 2: a box of {32, 18} lands 16 x 9 pixels
+    rdvc::TapMaps<1> m;
+    if (int rc = act_map(&m.a[0], dt, in, in_ps, u.n_kb * 64, B, Hin, Win, k * rdvc::TAP_TX, k * g.box_y, false, k == 2))
+        return rc;
+    if (int rc = slab_map(&m.w, dt, w, u.n, u.n_kb * g.slabs)) return rc;
+    rdvc::TapParams p = tap_params(B, Hout, Wout, u.n_kb);
     p.bias = bias;
     p.out = out; p.out_ps = out_ps;
     p.out2 = out2;
     p.res = res; p.res_ps = res_ps;
     const bool f32 = (out_dtype == RDVC_DT_F32);
-    return op_dtype == RDVC_DT_F16 ? dispatch_context_conv<__half>(u, epi, f32, tm_a, tm_w, p, st)
-                                   : dispatch_context_conv<__nv_bfloat16>(u, epi, f32, tm_a, tm_w, p, st);
+    return op_dtype == RDVC_DT_F16 ? dispatch_context_conv<__half>(u, epi, f32, m, p, st)
+                                   : dispatch_context_conv<__nv_bfloat16>(u, epi, f32, m, p, st);
 }
 
 template <typename InT, typename OpT>
@@ -2454,13 +2421,13 @@ int rdvc_corr_context_encoder_pack_weights(const float* const* conv_w, const flo
     std::vector<double> w, b;
     size_t wo = 0, bo = 0;
     for (const CeUnit& u : CE_UNITS) {
-        const int S = ce_slabs(u.geom);
+        const int S = ce_geom(u.geom).slabs;
         for (int part = 0; part < (u.ds >= 0 ? 2 : 1); ++part) {
             const int li = part ? u.ds : u.conv;
             const CeLayer& L = CE_LAYERS[li];
             ce_fold(li, conv_w, conv_b, bn_w, bn_b, bn_mean, bn_var, eps, w, b);
             for (int n = 0; n < L.cout; ++n) bias_host[bo + part * u.n + n] = static_cast<float>(b[n]);
-            if (u.geom == rdvc::CE_G_STEM) {                 // [ty][n][k], k = tx * 12 + py * 6 + px * 3 + c
+            if (u.geom == rdvc::TAP_G_STEM) {                // [ty][n][k], k = tx * 12 + py * 6 + px * 3 + c
                 for (int ty = 0; ty < 4; ++ty)
                     for (int n = 0; n < L.cout; ++n)
                         for (int k = 0; k < 48; ++k) {
@@ -2557,7 +2524,7 @@ int rdvc_corr_context_encoder(const void* image, const long long* image_strides,
     auto unit = [&](int i, const void* in, long long in_ps, int Hin, int Win, int Hout, int Wout, void* o, long long o_ps,
                     void* o2, const void* res, long long res_ps) {
         const CeUnit& u = CE_UNITS[i];
-        const int epi = (i == CE_N_UNITS - 1 && out_form == RDVC_CE_OUT_SPLIT) ? rdvc::CE_EPI_SPLIT : u.epi;
+        const int epi = (i == CE_N_UNITS - 1 && out_form == RDVC_CE_OUT_SPLIT) ? rdvc::TAP_EPI_SPLIT : u.epi;
         const int od = (i == CE_N_UNITS - 1) ? out_dtype : op_dtype;
         const int rc = run_context_unit(u, epi, in, in_ps, B, Hin, Win, Hout, Wout, op_dtype, wp, bp, o, o_ps, od, o2, res,
                                         res_ps, st);

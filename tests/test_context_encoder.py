@@ -4,7 +4,7 @@ BatchNorm folded into tcgen05 convolutions.
 CPU part (-m "not gpu"): parameter tree and strict state_dict round trips against torchvision's class, the refused
 configurations, the host fold + pack evaluated the way the kernels walk it (the stem's polyphase unrolling at odd H and
 W, the 96-channel padding, the fused downsample's slab and bias layout), the packing key, the C ABI's argument errors
-and size queries, the module refusals, the kernels' SASS and their spill-free register allocation.
+and size queries, the module refusals (the kernels' SASS and registers: test_tap_conv.py).
 GPU part (-m gpu): each layer kind against fp64 on the kernel's own inputs (read back from the workspace, which keeps
 every intermediate), the whole module against the fp64 chain and against stock torchvision, NaN-filled workspaces,
 determinism / streams / graphs / batch composition / input layouts, re-packing, and RAFT end to end.  Every test uses
@@ -31,8 +31,6 @@ A wrong tap, phase, channel or slab shows up as an O(1) relative error.
 """
 import ctypes
 import os
-import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -49,12 +47,7 @@ TOL_STOCK = {torch.float32: 2e-2, torch.float16: 2e-2, torch.bfloat16: 1e-1}
 TOL_EPE = 0.05
 DTYPES = [torch.float32, torch.float16, torch.bfloat16]
 ADT = {torch.float32: rc.RDVC_DT_F32, torch.float16: rc.RDVC_DT_F16, torch.bfloat16: rc.RDVC_DT_BF16}
-PKG = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
-                   "pfe-raft-and-hyperprior-based-learned-video-compression_b200")
 SMALL = [(1, 36, 52), (2, 70, 98), (1, 37, 53), (1, 368, 640)]
-# (geometry, N, epilogue) of every kernel instantiation, per operand dtype (csrc/context_encoder_sm100.cuh)
-INSTANCES = [(2, 64, 0, "P"), (0, 64, 0, "P"), (0, 64, 1, "P"), (0, 128, 0, "P"), (0, 128, 1, "P"), (1, 128, 2, "P"),
-             (3, 256, 3, "P"), (3, 256, 3, "float"), (3, 256, 4, "P"), (3, 256, 4, "float")]
 
 
 @pytest.fixture(scope="module")
@@ -315,42 +308,6 @@ def test_module_refusals_on_cpu():
         ce(x)
     with pytest.raises(ValueError, match="hidden_size=128"):
         seeded(4).forward_split(x, hidden_size=96)
-
-
-def test_sass_has_tcgen05_and_tma(lib):
-    """Every instantiation of the context-encoder kernel is Blackwell-native: tcgen05.mma (UTCHMMA), TMA loads
-    (UTMALDG) and TMEM reads (LDTM)."""
-    out = subprocess.run(["cuobjdump", "-sass", rc._cabi.lib_path()], capture_output=True, text=True)
-    if out.returncode != 0:
-        pytest.skip("cuobjdump unavailable")
-    funcs = [f for f in out.stdout.split("Function : ") if f.startswith("_ZN4rdvc19context_conv_kernel")]
-    assert len(funcs) == 2 * len(INSTANCES), len(funcs)
-    for f in funcs:
-        assert "UTCHMMA" in f and "UTMALDG" in f and "LDTM" in f, f.splitlines()[0]
-
-
-def test_no_register_spills():
-    """-Xptxas -v over every instantiation of the context-encoder kernel and the stem pack: no spills."""
-    from rdvc_corr_b200 import _build
-    inst = []
-    for op in ("__half", "__nv_bfloat16"):
-        for g, n, e, o in INSTANCES:
-            inst.append(f"template __global__ void context_conv_kernel<{g}, {n}, {e}, {op if o == 'P' else o}, {op}>"
-                        "(const __grid_constant__ CUtensorMap, const __grid_constant__ CUtensorMap, const CeParams);")
-        for t in ("float", "__half", "__nv_bfloat16"):
-            inst.append(f"template __global__ void ce_stem_pack_kernel<{t}, {op}>(const CeStemParams);")
-    src = '#include "context_encoder_sm100.cuh"\nnamespace rdvc {\n' + "\n".join(inst) + "\n}\n"
-    with tempfile.TemporaryDirectory() as d:
-        cu = os.path.join(d, "spills.cu")
-        with open(cu, "w") as f:
-            f.write(src)
-        res = subprocess.run([_build.nvcc_path(), "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a",
-                              "-Xptxas", "-v", "-I", os.path.join(PKG, "csrc"), "-c", cu, "-o", os.path.join(d, "s.o")],
-                             capture_output=True, text=True)
-    assert res.returncode == 0, res.stderr[-3000:]
-    props = [ln for ln in res.stderr.splitlines() if "spill stores" in ln]
-    assert len(props) == len(inst), res.stderr[-3000:]
-    assert all("0 bytes spill stores, 0 bytes spill loads" in ln for ln in props), props
 
 
 # ------------------------------------------------------------------ GPU

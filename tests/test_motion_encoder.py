@@ -3,7 +3,7 @@ convolutions, and the 1x1 GEMM's NHWC output.
 
 CPU part (-m "not gpu"): parameter trees and strict state_dict round trips against torchvision's classes, the refused
 configurations, each layer's host-packed weights evaluated the way the kernels walk them, the C ABI's argument errors
-and size queries, the module refusals, the kernels' SASS and their spill-free register allocation.
+and size queries, the module refusals (the kernels' SASS and registers: test_tap_conv.py).
 GPU part (-m gpu): every layer against an fp64 evaluation with the kernels' rounding points, input forms, whole modules
 against the stock ones, the 1x1 NHWC output, the flow channels and untouched channel slices, determinism / streams /
 graphs / re-packing, and RAFT end to end.
@@ -26,8 +26,6 @@ Tolerances (absolute, per element):
 """
 import ctypes
 import os
-import subprocess
-import tempfile
 
 import numpy as np
 import pytest
@@ -48,8 +46,6 @@ ADT = {torch.float32: rc.RDVC_DT_F32, torch.float16: rc.RDVC_DT_F16, torch.bfloa
 LAYERS = {_cabi.RDVC_UC_CONVCORR2: (256, 192, 3, 192), _cabi.RDVC_UC_CONVFLOW1: (2, 128, 7, 128),
           _cabi.RDVC_UC_CONVFLOW2: (128, 64, 3, 64), _cabi.RDVC_UC_CONV: (256, 126, 3, 128),
           _cabi.RDVC_UC_FH_CONV1: (128, 256, 3, 256), _cabi.RDVC_UC_FH_CONV2: (256, 2, 3, 16)}
-PKG = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))),
-                   "pfe-raft-and-hyperprior-based-learned-video-compression_b200")
 
 
 @pytest.fixture(scope="module")
@@ -248,52 +244,6 @@ def test_module_refusals_on_cpu():
         me(flow, corr.detach())
     with pytest.raises(RuntimeError, match="forward-only"):
         fh(h.detach())
-
-
-def test_sass_has_tcgen05_and_tma(lib):
-    """Every 3x3 instantiation and the 1x1 GEMM's NHWC variant are Blackwell-native: tcgen05.mma (UTCHMMA), TMA loads
-    (UTMALDG) and TMEM reads (LDTM)."""
-    out = subprocess.run(["cuobjdump", "-sass", rc._cabi.lib_path()], capture_output=True, text=True)
-    if out.returncode != 0:
-        pytest.skip("cuobjdump unavailable")
-    funcs = out.stdout.split("Function : ")
-    uc = [f for f in funcs if f.startswith("_ZN4rdvc18update_conv_kernel")]
-    nhwc = [f for f in funcs if f.startswith("_ZN4rdvc24corr_conv1x1_nhwc_kernel")]
-    assert len(uc) == 14, len(uc)          # (convcorr2, convflow2, fh conv1) x 2 operand dtypes + (conv, fh conv2) x 4
-    assert len(nhwc) == 2, len(nhwc)
-    for f in uc + nhwc:
-        assert "UTCHMMA" in f and "UTMALDG" in f and "LDTM" in f, f.splitlines()[0]
-    assert len([f for f in funcs if f.startswith("_ZN4rdvc16convflow1_kernel")]) == 2
-
-
-def test_no_register_spills():
-    """-Xptxas -v over every new kernel instantiation: no spill stores or loads."""
-    from rdvc_corr_b200 import _build
-    src = """
-#include "update_conv_sm100.cuh"
-#include "corr_conv1x1_sm100.cuh"
-namespace rdvc {
-#define UC(N, E, O, P) template __global__ void update_conv_kernel<N, E, O, P>(const __grid_constant__ CUtensorMap, const __grid_constant__ CUtensorMap, const UcParams);
-UC(192, 0, __half, __half) UC(64, 0, __half, __half) UC(256, 0, __half, __half)
-UC(128, 1, __half, __half) UC(128, 1, float, __half) UC(16, 2, __half, __half) UC(16, 2, float, __half)
-UC(192, 0, __nv_bfloat16, __nv_bfloat16) UC(128, 1, float, __nv_bfloat16) UC(16, 2, __nv_bfloat16, __nv_bfloat16)
-template __global__ void convflow1_kernel<__half>(const Cf1Params);
-template __global__ void convflow1_kernel<__nv_bfloat16>(const Cf1Params);
-template __global__ void corr_conv1x1_nhwc_kernel<__half>(const __grid_constant__ CUtensorMap, const __grid_constant__ CUtensorMap, const Conv1x1Params);
-template __global__ void corr_conv1x1_nhwc_kernel<__nv_bfloat16>(const __grid_constant__ CUtensorMap, const __grid_constant__ CUtensorMap, const Conv1x1Params);
-}
-"""
-    with tempfile.TemporaryDirectory() as d:
-        cu = os.path.join(d, "spills.cu")
-        with open(cu, "w") as f:
-            f.write(src)
-        res = subprocess.run([_build.nvcc_path(), "-std=c++17", "-gencode", "arch=compute_100a,code=sm_100a",
-                              "-Xptxas", "-v", "-I", os.path.join(PKG, "csrc"), "-c", cu, "-o", os.path.join(d, "s.o")],
-                             capture_output=True, text=True)
-    assert res.returncode == 0, res.stderr[-3000:]
-    props = [ln for ln in res.stderr.splitlines() if "spill stores" in ln]
-    assert len(props) >= 14, res.stderr[-3000:]
-    assert all("0 bytes spill stores, 0 bytes spill loads" in ln for ln in props), props
 
 
 # ------------------------------------------------------------------ GPU

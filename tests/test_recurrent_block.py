@@ -2,7 +2,7 @@
 
 CPU part (-m "not gpu"): parameter tree and strict state_dict round trips against torchvision's class, the refused
 configurations, the host-packed tap matrices evaluated as a convolution (both tap axes), the C ABI's argument errors,
-the refusals of the module, and the kernels' SASS.
+and the refusals of the module (the kernels' SASS and registers: test_tap_conv.py).
 GPU part (-m gpu): passes and whole blocks against an fp64 evaluation with the kernel's rounding points and against
 the stock module, guard bands, determinism / streams / graphs, re-packing, and RAFT end to end.
 
@@ -20,7 +20,6 @@ Tolerances (absolute):
 """
 import ctypes
 import os
-import subprocess
 
 import numpy as np
 import pytest
@@ -160,18 +159,6 @@ def test_module_refusals_on_cpu():
     rb.train()
     with pytest.raises(RuntimeError, match="forward-only"):
         rb(h.detach(), x)
-
-
-def test_sass_has_tcgen05_and_tma(lib):
-    """The new kernels are Blackwell-native: tcgen05.mma (UTCHMMA) and TMA loads (UTMALDG) in each of them."""
-    out = subprocess.run(["cuobjdump", "-sass", rc._cabi.lib_path()], capture_output=True, text=True)
-    if out.returncode != 0:
-        pytest.skip("cuobjdump unavailable")
-    funcs = out.stdout.split("Function : ")
-    gru = [f for f in funcs if f.startswith("_ZN4rdvc14convgru_kernel")]
-    assert len(gru) == 8, len(gru)                                      # 2 passes x 4 (activation, operand) dtypes
-    for f in gru:
-        assert "UTCHMMA" in f and "UTMALDG" in f and "LDTM" in f, f.splitlines()[0]
 
 
 # ------------------------------------------------------------------ GPU
