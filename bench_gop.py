@@ -119,6 +119,10 @@ def run_sharded(args, own_process_group=True):
         ce = rc.ContextEncoder()
         ce.load_state_dict(model.context_encoder.state_dict())
         model.context_encoder = ce.to(dev).eval()
+    if getattr(args, "b200_feature_encoder", False):      # same weights, InstanceNorm statistics in tcgen05 epilogues
+        fe = rc.FeatureEncoder()
+        fe.load_state_dict(model.feature_encoder.state_dict())
+        model.feature_encoder = fe.to(dev).eval()
     h, w = args.height, args.width
     g = torch.Generator(device=dev).manual_seed(0)
     base = torch.rand(1, 3, h // 16 + 8, w // 16 + 8, device=dev, generator=g)
@@ -338,6 +342,8 @@ def run_sharded(args, own_process_group=True):
             line["config"]["b200_mask_predictor"] = True
         if getattr(args, "b200_context_encoder", False):
             line["config"]["b200_context_encoder"] = True
+        if getattr(args, "b200_feature_encoder", False):
+            line["config"]["b200_feature_encoder"] = True
         # flow end-point error of this configuration against STOCK torchvision RAFT (same weights, same autocast
         # setting) on one frame pair of the sequence -- outside the timed region
         a, b = frame_at(big, 3, h, w), frame_at(big, 4, h, w)
@@ -428,6 +434,9 @@ def main():
     ap.add_argument("--b200-context-encoder", action="store_true",
                     help="swap rc.ContextEncoder into the model: the context encoder with BatchNorm folded into tcgen05 "
                          "convolutions, RAFT's tanh / relu in its last epilogue")
+    ap.add_argument("--b200-feature-encoder", action="store_true",
+                    help="swap rc.FeatureEncoder into the model: the feature encoder as tcgen05 convolutions whose "
+                         "epilogues write InstanceNorm statistics, one normalising pass per layer")
     args = ap.parse_args()
     if args.cudnn_benchmark:
         torch.backends.cudnn.benchmark = True

@@ -440,6 +440,54 @@ int rdvc_corr_context_encoder(const void* image, const long long* image_strides,
                               int op_dtype, const void* packed_w, const float* biases, int out_form, void* workspace,
                               size_t workspace_bytes, void* out, long long out_pixel_stride, int out_dtype, void* stream);
 
+/* ---- RAFT's feature encoder (torchvision FeatureEncoder, InstanceNorm2d without affine or running statistics,
+ * raft_large's configuration) ---- *
+ * The context encoder's 16 convolutions and units, each of the first 15 followed by InstanceNorm.  Weights: the
+ * context encoder's packing (rdvc_corr_context_encoder_pack_weights) with the identity norm (bn_w = 1, bn_b = 0,
+ * bn_mean = 0, bn_var = 1, eps = 0: s = 1 exactly, each weight rounded once).  The normalised layers' conv biases are
+ * not used: InstanceNorm subtracts each (sample, channel)'s mean, so IN(y + b) = IN(y) exactly.
+ * Per normalised unit (13; a stride-2 unit also carries its block's 1x1 downsample) three launches:
+ *   the convolution (tcgen05, fp32 accumulation) stores its raw output y rounded to op_dtype and, per 16 x 8 tile and
+ *     channel, (mean, M2) of the stored values over the tile's pixels inside the image;
+ *   finalize merges a sample's tiles in a fixed order in fp64 (Chan) -> fp32 mean and rstd = 1 / sqrt(var + eps),
+ *     var biased;
+ *   apply, in fp32, rounded once to op_dtype: relu(IN(y)) (stem, convnormrelu1), relu(x + relu(IN(y))) (convnormrelu2
+ *     of an identity block, x its input) or relu(IN(ds) + relu(IN(y))) (of a stride-2 block, ds its downsample's raw
+ *     output).  layer2's channels 96-127 are written as exact zeros.
+ * No atomics, and tiles never span images: a sample's result does not depend on the batch it is in.
+ *
+ * rdvc_corr_feature_encoder_workspace_bytes: 0 for a non-positive size, an unknown act_dtype or a one-element layer3
+ *   plane (ceil(H / 8) = ceil(W / 8) = 1, which InstanceNorm cannot normalise).
+ * rdvc_corr_feature_encoder: image, image_strides, in_dtype, B, H, W, op_dtype, packed_w, biases: as for
+ *   rdvc_corr_context_encoder; eps: RDVC_FE_NORMS HOST doubles (>= 0, finite), indexed like the pack arrays (layer i <
+ *   15 of the context encoder's list).  out_form:
+ *   RDVC_FE_OUT_FEATURES: FeatureEncoder.forward, NHWC (B, ceil(H / 8), ceil(W / 8), 256) out_dtype (F32 or op_dtype),
+ *     out_pixel_stride >= 256;
+ *   RDVC_FE_OUT_TRUNK: layer3's output, NHWC (B, ceil(H / 8), ceil(W / 8), 128) op_dtype, out_pixel_stride >= 128 (the
+ *     input of the final 1x1, e.g. for TVCorrBlock.build_pyramid_from_encoder).
+ *   out: a multiple of 16 bytes per pixel, 16-byte aligned, overlapping neither the image nor the workspace.
+ *   workspace: DEVICE, rdvc_corr_feature_encoder_workspace_bytes(...), 256-byte aligned; after the call it holds every
+ *   intermediate, each in its own buffer of align256(bytes), in this order:
+ *     at (H1, W1), B * H1 * W1 * 64 16-bit values each: the stem operand, then y and the normalised activation a of
+ *       convnormrelu, layer1.0.convnormrelu1, layer1.0.convnormrelu2 (a = layer1.0's output), layer1.1.convnormrelu1,
+ *       layer1.1.convnormrelu2 (11 buffers);
+ *     at (H2, W2), 128-channel pixels: y, downsample y, a of layer2.0.convnormrelu1, then y, a of
+ *       layer2.0.convnormrelu2, layer2.1.convnormrelu1, layer2.1.convnormrelu2 (9 buffers);
+ *     at (H3, W3): the same for layer3 (with RDVC_FE_OUT_TRUNK the last a goes to out and its buffer is untouched);
+ *     per normalised unit u = 0..12 (stem, layer1 x 4, layer2.0 conv1 + downsample, 3 more of layer2, the same for
+ *       layer3): float2 (mean, M2) partials [B * ceil(w_u / 16) * ceil(h_u / 8)][NT_u], tiles along x first, NT_u =
+ *       64 (layer1), 128, or 256 for a stride-2 unit (channels 128-255: its downsample);
+ *     per normalised unit: fp32 [B][2][NT_u], mean then rstd.
+ *   1 + 13 x 3 launches, + 1 (the 1x1) for RDVC_FE_OUT_FEATURES.                                                    */
+#define RDVC_FE_OUT_FEATURES 0
+#define RDVC_FE_OUT_TRUNK 1
+#define RDVC_FE_NORMS 15
+size_t rdvc_corr_feature_encoder_workspace_bytes(int B, int H, int W, int act_dtype);
+int rdvc_corr_feature_encoder(const void* image, const long long* image_strides, int in_dtype, int B, int H, int W,
+                              int op_dtype, const void* packed_w, const float* biases, const double* eps, int out_form,
+                              void* workspace, size_t workspace_bytes, void* out, long long out_pixel_stride,
+                              int out_dtype, void* stream);
+
 /* ---- next row f-4 (last piece): entropy-coder stand-in (HOST functions) ---- *
  * Stands in for the range coder behind EntropyBottleneck.compress / .decompress (R:codec_processing.py:433,447
  * construction, :488-497 compress, :509-536 decompress; compressai's RansEncoder.encode_with_indexes /

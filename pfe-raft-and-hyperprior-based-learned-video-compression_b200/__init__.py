@@ -24,6 +24,7 @@ from .corr_block import (  # noqa: F401
     index_pyramid,
 )
 from .context_encoder import ContextEncoder  # noqa: F401
+from .feature_encoder import FeatureEncoder  # noqa: F401
 from .mask_predictor import MaskPredictor  # noqa: F401
 from .mcn import MotionCompensationNetwork  # noqa: F401
 from .motion_encoder import FlowHead, MotionEncoder  # noqa: F401
@@ -35,7 +36,7 @@ from .recurrent_block import RecurrentBlock  # noqa: F401
 __all__ = [
     "CorrBlock", "CorrPyramid", "TVCorrBlock", "build_pyramid", "index_pyramid", "raft_flow", "raft_flow_sequence", "GraphedRaftFlow",
     "WarpingLayer", "motion_warp", "resize_flow", "MotionCompensationNetwork", "RecurrentBlock",
-    "MotionEncoder", "FlowHead", "MaskPredictor", "ContextEncoder",
+    "MotionEncoder", "FlowHead", "MaskPredictor", "ContextEncoder", "FeatureEncoder",
     "frame_to_tensor", "preprocess_frame_codec", "preprocess_frame_raft",
     "RDVC_DT_BF16", "RDVC_DT_F16", "RDVC_DT_F32", "RDVC_LAYOUT_ROWMAJOR", "RDVC_LAYOUT_TILED",
 ]

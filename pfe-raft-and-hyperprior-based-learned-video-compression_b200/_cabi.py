@@ -18,6 +18,7 @@ RDVC_GRU_HORIZONTAL, RDVC_GRU_VERTICAL = 0, 1
 RDVC_UC_CONVCORR2, RDVC_UC_CONVFLOW1, RDVC_UC_CONVFLOW2, RDVC_UC_CONV, RDVC_UC_FH_CONV1, RDVC_UC_FH_CONV2 = range(6)
 RDVC_MASK_OUT_UPSAMPLED, RDVC_MASK_OUT_MASK = 0, 1
 RDVC_CE_OUT_RAW, RDVC_CE_OUT_SPLIT = 0, 1
+RDVC_FE_OUT_FEATURES, RDVC_FE_OUT_TRUNK = 0, 1
 
 RDVC_E = {
     -1: "RDVC_E_NULL", -2: "RDVC_E_SHAPE", -3: "RDVC_E_TOO_SMALL", -4: "RDVC_E_DTYPE",
@@ -117,6 +118,10 @@ SYMBOLS = {
     "rdvc_corr_context_encoder": (_c.c_int, [_c.c_void_p, _c.c_void_p] + [_c.c_int] * 5 +
                                   [_c.c_void_p, _c.c_void_p, _c.c_int, _c.c_void_p, _c.c_size_t, _c.c_void_p,
                                    _c.c_longlong, _c.c_int, _c.c_void_p]),
+    "rdvc_corr_feature_encoder_workspace_bytes": (_c.c_size_t, [_c.c_int] * 4),
+    "rdvc_corr_feature_encoder": (_c.c_int, [_c.c_void_p, _c.c_void_p] + [_c.c_int] * 5 +
+                                  [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_int, _c.c_void_p, _c.c_size_t,
+                                   _c.c_void_p, _c.c_longlong, _c.c_int, _c.c_void_p]),
     "rdvc_corr_pair_host_submit": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p] +
                                    [_c.c_int] * 9),
     "rdvc_corr_pair_host_wait": (_c.c_int, [_c.c_int]),

@@ -24,6 +24,7 @@
 #include "corr_pack.cuh"
 #include "mask_upsample_sm100.cuh"
 #include "tap_conv_sm100.cuh"
+#include "instance_norm_sm100.cuh"
 #include "entropy_coder.h"
 #include "mcn_conv_sm100.cuh"
 #include "mcn_convx_sm100.cuh"
@@ -1688,6 +1689,21 @@ int launch_tap_conv(const rdvc::TapMaps<rdvc::TapGeom<G>::MAPS>& maps, const rdv
     return RDVC_OK;
 }
 
+template <int G, int N, int EPI, typename OpT>
+int launch_tap_conv_in(const rdvc::TapMaps<rdvc::TapGeom<G>::MAPS>& maps, const rdvc::TapParams& p, cudaStream_t st) {
+    constexpr int SMEM = rdvc::TapCfg<G, N, EPI>::SMEM_LAUNCH;
+    auto kern = rdvc::tap_conv_in_kernel<G, N, EPI, OpT>;
+    static std::atomic<unsigned long long> attr_done{0};
+    if (int rc = ensure_dynamic_smem(kern, SMEM, attr_done, "cudaFuncSetAttribute(tap_conv_in, max dynamic smem)"))
+        return rc;
+    const int grid = std::min(sm_count(), p.n_super);
+    kern<<<grid, rdvc::TAP_THREADS, SMEM, st>>>(maps, p);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "tap_conv_in_kernel launch");
+    return RDVC_OK;
+}
+
 // Shared memory and TMEM columns of every (geometry, N, epilogue) the dispatch tables instantiate: the tile and ring
 // sizes these kernels are measured with.  A change that moves one of them is a performance change.
 template <int G, int N, int EPI>
@@ -1708,6 +1724,11 @@ static_assert(tap_cfg_is<rdvc::TAP_G_S1, 128, rdvc::TAP_EPI_RES>(148736, 256), "
 static_assert(tap_cfg_is<rdvc::TAP_G_S2, 128, rdvc::TAP_EPI_DS>(140544, 512), "stride 2 + downsample");
 static_assert(tap_cfg_is<rdvc::TAP_G_1X1, 256, rdvc::TAP_EPI_RAW>(197888, 512), "1x1");
 static_assert(tap_cfg_is<rdvc::TAP_G_1X1, 256, rdvc::TAP_EPI_SPLIT>(197888, 512), "1x1 split");
+// the feature encoder's statistics epilogues: the context encoder's rings plus 2 tiles x 4 warps x NT (mean, M2)
+static_assert(tap_cfg_is<rdvc::TAP_G_STEM, 64, rdvc::TAP_EPI_STATS>(128256, 128), "stem, statistics");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 64, rdvc::TAP_EPI_STATS>(120064, 128), "layer1, statistics");
+static_assert(tap_cfg_is<rdvc::TAP_G_S1, 128, rdvc::TAP_EPI_STATS>(156928, 256), "layer2/3, statistics");
+static_assert(tap_cfg_is<rdvc::TAP_G_S2, 128, rdvc::TAP_EPI_DS_STATS>(156928, 512), "stride 2 + downsample, statistics");
 
 // fp32 activations -> 16-bit NHWC operand copies (128 channels of each of the first n_src sources of cp)
 int launch_gru_cast(const rdvc::GruCastParams& cp, int n_src, int op_dtype, cudaStream_t st) {
@@ -2334,18 +2355,27 @@ int dispatch_context_conv(const CeUnit& u, int epi, bool f32_out, const rdvc::Ta
     }
 }
 
+// one unit's tensor maps and tile grid: input NHWC op_dtype (B, Hin, Win, n_kb * 64 of in_ps channels) -> output
+// grid (Hout, Wout)
+int context_unit_setup(const CeUnit& u, const void* in, long long in_ps, int B, int Hin, int Win, int Hout, int Wout,
+                       int op_dtype, const void* w, rdvc::TapMaps<1>& m, rdvc::TapParams& p) {
+    const CUtensorMapDataType dt = op_map_dtype(op_dtype);
+    const CeGeomSizes g = ce_geom(u.geom);
+    const int k = (u.geom == rdvc::TAP_G_S2) ? 2 : 1;      // stride 2: a box of {32, 18} lands 16 x 9 pixels
+    if (int rc = act_map(&m.a[0], dt, in, in_ps, u.n_kb * 64, B, Hin, Win, k * rdvc::TAP_TX, k * g.box_y, false, k == 2))
+        return rc;
+    if (int rc = slab_map(&m.w, dt, w, u.n, u.n_kb * g.slabs)) return rc;
+    p = tap_params(B, Hout, Wout, u.n_kb);
+    return RDVC_OK;
+}
+
 // one unit: input NHWC op_dtype (B, Hin, Win, n_kb * 64 of in_ps channels) -> output grid (Hout, Wout)
 int run_context_unit(const CeUnit& u, int epi, const void* in, long long in_ps, int B, int Hin, int Win, int Hout,
                      int Wout, int op_dtype, const void* w, const float* bias, void* out, long long out_ps,
                      int out_dtype, void* out2, const void* res, long long res_ps, cudaStream_t st) {
-    const CUtensorMapDataType dt = op_map_dtype(op_dtype);
-    const CeGeomSizes g = ce_geom(u.geom);
-    const int k = (u.geom == rdvc::TAP_G_S2) ? 2 : 1;      // stride 2: a box of {32, 18} lands 16 x 9 pixels
     rdvc::TapMaps<1> m;
-    if (int rc = act_map(&m.a[0], dt, in, in_ps, u.n_kb * 64, B, Hin, Win, k * rdvc::TAP_TX, k * g.box_y, false, k == 2))
-        return rc;
-    if (int rc = slab_map(&m.w, dt, w, u.n, u.n_kb * g.slabs)) return rc;
-    rdvc::TapParams p = tap_params(B, Hout, Wout, u.n_kb);
+    rdvc::TapParams p;
+    if (int rc = context_unit_setup(u, in, in_ps, B, Hin, Win, Hout, Wout, op_dtype, w, m, p)) return rc;
     p.bias = bias;
     p.out = out; p.out_ps = out_ps;
     p.out2 = out2;
@@ -2551,6 +2581,215 @@ int rdvc_corr_context_encoder(const void* image, const long long* image_strides,
     if ((rc = unit(11, l3[2], 128, H3, W3, H3, W3, l3[3], 128, nullptr, nullptr, 0))) return rc;
     if ((rc = unit(12, l3[3], 128, H3, W3, H3, W3, l3[4], 128, nullptr, l3[2], 128))) return rc;
     return unit(13, l3[4], 128, H3, W3, H3, W3, out, out_pixel_stride, nullptr, nullptr, 0);
+}
+
+}  // extern "C"
+
+// ---- RAFT's feature encoder: FeatureEncoder with InstanceNorm, statistics in the convolution epilogues ------------
+// The context encoder's units and packed weights (packed with the identity norm); every unit but the final 1x1 runs
+// as tap_conv_in_kernel (raw output + per-tile partials), then in_finalize_kernel and in_apply_kernel.
+namespace {
+
+constexpr int FE_N_NORM_UNITS = CE_N_UNITS - 1;
+
+int fe_unit_nt(int i) { return CE_UNITS[i].n * (CE_UNITS[i].ds >= 0 ? 2 : 1); }
+
+// the workspace of include/rdvc_corr.h; with base == nullptr only .bytes is meaningful
+struct FeLayout {
+    uint8_t* l1[11];                     // S, then Y, A of units 0-4
+    uint8_t* l2[9];                      // Y5 D5 A5 Y6 A6 Y7 A7 Y8 A8
+    uint8_t* l3[9];                      // the same for units 9-12
+    float2* part[FE_N_NORM_UNITS];
+    float* stats[FE_N_NORM_UNITS];
+    size_t bytes;
+};
+
+FeLayout fe_layout(int B, int H, int W, void* base) {
+    const CeSizes s = ce_sizes(B, H, W);
+    FeLayout L;
+    uint8_t* q = static_cast<uint8_t*>(base);
+    size_t off = 0;
+    auto take = [&](size_t n) {
+        uint8_t* r = q ? q + off : nullptr;
+        off += align_up(n, 256);
+        return r;
+    };
+    for (auto& x : L.l1) x = take(s.p1);
+    for (auto& x : L.l2) x = take(s.p2);
+    for (auto& x : L.l3) x = take(s.p3);
+    for (int i = 0; i < FE_N_NORM_UNITS; ++i) {
+        const int Ho = i < 5 ? s.H1 : i < 9 ? s.H2 : s.H3, Wo = i < 5 ? s.W1 : i < 9 ? s.W2 : s.W3;
+        L.part[i] = reinterpret_cast<float2*>(take(static_cast<size_t>(tap_params(B, Ho, Wo, 1).n_tiles) * fe_unit_nt(i) * 8));
+    }
+    for (int i = 0; i < FE_N_NORM_UNITS; ++i)
+        L.stats[i] = reinterpret_cast<float*>(take(static_cast<size_t>(B) * 2 * fe_unit_nt(i) * 4));
+    L.bytes = off;
+    return L;
+}
+
+template <typename OpT>
+int dispatch_feature_conv(const CeUnit& u, const rdvc::TapMaps<1>& m, const rdvc::TapParams& p, cudaStream_t st) {
+    using namespace rdvc;
+    switch (u.geom) {
+        case TAP_G_STEM: return launch_tap_conv_in<TAP_G_STEM, 64, TAP_EPI_STATS, OpT>(m, p, st);
+        case TAP_G_S2: return launch_tap_conv_in<TAP_G_S2, 128, TAP_EPI_DS_STATS, OpT>(m, p, st);
+        default:
+            return u.n == 64 ? launch_tap_conv_in<TAP_G_S1, 64, TAP_EPI_STATS, OpT>(m, p, st)
+                             : launch_tap_conv_in<TAP_G_S1, 128, TAP_EPI_STATS, OpT>(m, p, st);
+    }
+}
+
+template <typename OpT>
+int launch_in_apply(int form, const rdvc::InApplyParams& a, cudaStream_t st) {
+    const unsigned blocks = static_cast<unsigned>((a.n_pix * (a.Cs / 8) + 255) / 256);
+    if (form == rdvc::IN_APPLY_RELU) rdvc::in_apply_kernel<rdvc::IN_APPLY_RELU, OpT><<<blocks, 256, 0, st>>>(a);
+    else if (form == rdvc::IN_APPLY_RES) rdvc::in_apply_kernel<rdvc::IN_APPLY_RES, OpT><<<blocks, 256, 0, st>>>(a);
+    else rdvc::in_apply_kernel<rdvc::IN_APPLY_DS, OpT><<<blocks, 256, 0, st>>>(a);
+    ++g_launches;
+    cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) return cuda_fail(e, "in_apply_kernel launch");
+    return RDVC_OK;
+}
+
+}  // namespace
+
+extern "C" {
+
+size_t rdvc_corr_feature_encoder_workspace_bytes(int B, int H, int W, int act_dtype) {
+    if (B <= 0 || H <= 0 || W <= 0) return 0;
+    if (act_dtype != RDVC_DT_F32 && act_dtype != RDVC_DT_F16 && act_dtype != RDVC_DT_BF16) return 0;
+    if ((H + 7) / 8 == 1 && (W + 7) / 8 == 1) return 0;          // a one-element plane cannot be normalised
+    return fe_layout(B, H, W, nullptr).bytes;
+}
+
+int rdvc_corr_feature_encoder(const void* image, const long long* image_strides, int in_dtype, int B, int H, int W,
+                              int op_dtype, const void* packed_w, const float* biases, const double* eps, int out_form,
+                              void* workspace, size_t workspace_bytes, void* out, long long out_pixel_stride,
+                              int out_dtype, void* stream) {
+    if (!image || !image_strides || !packed_w || !biases || !eps || !workspace || !out)
+        return fail(RDVC_E_NULL, "null pointer argument");
+    if (out_form != RDVC_FE_OUT_FEATURES && out_form != RDVC_FE_OUT_TRUNK)
+        return fail(RDVC_E_UNSUPPORTED, "unknown out_form %d", out_form);
+    if (B <= 0 || H <= 0 || W <= 0) return fail(RDVC_E_SHAPE, "non-positive dimension B=%d H=%d W=%d", B, H, W);
+    if ((H + 7) / 8 == 1 && (W + 7) / 8 == 1)
+        return fail(RDVC_E_SHAPE, "H=%d W=%d: InstanceNorm expects more than 1 spatial element in layer3", H, W);
+    if (in_dtype != RDVC_DT_F32 && in_dtype != RDVC_DT_F16 && in_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "unsupported in_dtype=%d", in_dtype);
+    if (op_dtype != RDVC_DT_F16 && op_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 or BF16, got %d", op_dtype);
+    const bool trunk = out_form == RDVC_FE_OUT_TRUNK;
+    if (trunk ? out_dtype != op_dtype : (out_dtype != RDVC_DT_F32 && out_dtype != op_dtype))
+        return fail(RDVC_E_DTYPE, "out_dtype=%d must be %sop_dtype=%d", out_dtype, trunk ? "" : "F32 or ", op_dtype);
+    for (int i = 0; i < RDVC_FE_NORMS; ++i)
+        if (!(eps[i] >= 0.0) || std::isinf(eps[i])) return fail(RDVC_E_UNSUPPORTED, "eps[%d] = %g", i, eps[i]);
+    for (int i = 0; i < 4; ++i)
+        if (image_strides[i] < 0) return fail(RDVC_E_UNSUPPORTED, "negative image stride %lld", image_strides[i]);
+    if (H >= (1 << 24) || W >= (1 << 24) || static_cast<long long>(B) * ((H + 1) / 2) * ((W + 1) / 2) >= (1LL << 31))
+        return fail(RDVC_E_UNSUPPORTED, "too many pixels for 32-bit TMA coordinates");
+    const size_t in_es = elem_size(in_dtype), out_es = elem_size(out_dtype);
+    if (reinterpret_cast<uintptr_t>(image) % in_es) return fail(RDVC_E_ALIGN, "the image must be aligned to its element size");
+    if ((reinterpret_cast<uintptr_t>(packed_w) & 15) || (reinterpret_cast<uintptr_t>(biases) & 15) ||
+        (reinterpret_cast<uintptr_t>(out) & 15))
+        return fail(RDVC_E_ALIGN, "out, the packed weights and the biases must be 16-byte aligned");
+    const int out_c = trunk ? 128 : 256;
+    if (out_pixel_stride < out_c) return fail(RDVC_E_UNSUPPORTED, "out_pixel_stride %lld < %d", out_pixel_stride, out_c);
+    if ((out_pixel_stride * static_cast<long long>(out_es)) % 16)
+        return fail(RDVC_E_ALIGN, "out_pixel_stride must be a multiple of 16 bytes");
+    const size_t need = rdvc_corr_feature_encoder_workspace_bytes(B, H, W, RDVC_DT_F32);
+    if (workspace_bytes < need) return fail(RDVC_E_WORKSPACE, "workspace %zu < required %zu", workspace_bytes, need);
+    if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(RDVC_E_ALIGN, "the workspace must be 256-byte aligned");
+    const CeSizes s = ce_sizes(B, H, W);
+    const long long dims[4] = {B, 3, H, W};
+    size_t img_elems = 1;
+    for (int i = 0; i < 4; ++i) img_elems += static_cast<size_t>(dims[i] - 1) * static_cast<size_t>(image_strides[i]);
+    const size_t out_bytes = (static_cast<size_t>(B) * s.H3 * s.W3 - 1) * out_pixel_stride * out_es + out_c * out_es;
+    if (ranges_overlap(out, out_bytes, image, img_elems * in_es) || ranges_overlap(out, out_bytes, workspace, need))
+        return fail(RDVC_E_UNSUPPORTED, "out overlaps the image or the workspace");
+
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const FeLayout L = fe_layout(B, H, W, workspace);
+    rdvc::CeStemParams sp;
+    memset(&sp, 0, sizeof(sp));
+    sp.img = image;
+    sp.sb = image_strides[0]; sp.sc = image_strides[1]; sp.sy = image_strides[2]; sp.sx = image_strides[3];
+    sp.H = H; sp.W = W; sp.H1 = s.H1; sp.W1 = s.W1;
+    sp.out = L.l1[0];
+    sp.n_pix = static_cast<long long>(B) * s.H1 * s.W1;
+    if (int rc = op_dtype == RDVC_DT_F16 ? dispatch_ce_stem_pack<__half>(in_dtype, sp, st)
+                                         : dispatch_ce_stem_pack<__nv_bfloat16>(in_dtype, sp, st))
+        return rc;
+
+    const uint8_t* wp = static_cast<const uint8_t*>(packed_w);
+    const float* bp = biases;
+    // unit i: convolution of `in` -> raw y (and the downsample's raw y2), its statistics, then `form` -> a (a_ps);
+    // z / zi: the residual input, or the stride-2 unit whose downsample this block adds
+    auto unit = [&](int i, const void* in, long long in_ps, int Hin, int Win, int Ho, int Wo, void* y, void* y2,
+                    int form, const void* z, long long z_ps, int zi, void* a, long long a_ps) {
+        const CeUnit& u = CE_UNITS[i];
+        const long long ps = u.n;                                   // 64, or 128 (layer2's 96 channels padded)
+        rdvc::TapMaps<1> m;
+        rdvc::TapParams p;
+        if (int rc = context_unit_setup(u, in, in_ps, B, Hin, Win, Ho, Wo, op_dtype, wp, m, p)) return rc;
+        p.out = y; p.out_ps = ps;
+        p.out2 = y2;
+        p.part = L.part[i];
+        if (int rc = op_dtype == RDVC_DT_F16 ? dispatch_feature_conv<__half>(u, m, p, st)
+                                             : dispatch_feature_conv<__nv_bfloat16>(u, m, p, st))
+            return rc;
+        wp += ce_unit_w_elems(u) * 2;
+        bp += ce_unit_b_floats(u);
+        const int nt = fe_unit_nt(i);
+        rdvc::InFinParams f;
+        f.part = L.part[i]; f.stats = L.stats[i];
+        f.NT = nt; f.N = u.n;
+        f.n_tx = p.n_tx; f.n_ty = p.n_ty; f.H = Ho; f.W = Wo;
+        f.eps_lo = eps[u.conv]; f.eps_hi = u.ds >= 0 ? eps[u.ds] : 0.0;
+        rdvc::in_finalize_kernel<<<dim3(nt / 32, B), dim3(32, rdvc::IN_FIN_SLICES), 0, st>>>(f);
+        ++g_launches;
+        if (cudaError_t e = cudaGetLastError()) return cuda_fail(e, "in_finalize_kernel launch");
+        rdvc::InApplyParams ap;
+        memset(&ap, 0, sizeof(ap));
+        ap.y = y; ap.y_ps = ps;
+        ap.z = z; ap.z_ps = ps;
+        ap.st = L.stats[i]; ap.st_nt = nt;
+        if (form == rdvc::IN_APPLY_DS) { ap.zst = L.stats[zi] + CE_UNITS[zi].n; ap.zst_nt = fe_unit_nt(zi); }
+        ap.out = a; ap.out_ps = a_ps;
+        ap.C = CE_LAYERS[u.conv].cout; ap.Cs = u.n;
+        ap.hw = static_cast<long long>(Ho) * Wo;
+        ap.n_pix = B * ap.hw;
+        return op_dtype == RDVC_DT_F16 ? launch_in_apply<__half>(form, ap, st) : launch_in_apply<__nv_bfloat16>(form, ap, st);
+    };
+    using rdvc::IN_APPLY_RELU;
+    using rdvc::IN_APPLY_RES;
+    using rdvc::IN_APPLY_DS;
+    const int H1 = s.H1, W1 = s.W1, H2 = s.H2, W2 = s.W2, H3 = s.H3, W3 = s.W3;
+    uint8_t* const* l1 = L.l1;
+    uint8_t* const* l2 = L.l2;
+    uint8_t* const* l3 = L.l3;
+    void* last = trunk ? out : static_cast<void*>(l3[8]);
+    const long long last_ps = trunk ? out_pixel_stride : 128;
+    int rc = 0;
+    // TV:raft.py:145: convnormrelu; 146: layer1 = two residual blocks relu(x + relu(norm2(conv2(relu(norm1(conv1(x)))))))
+    if ((rc = unit(0, l1[0], 64, H1, W1, H1, W1, l1[1], nullptr, IN_APPLY_RELU, nullptr, 0, 0, l1[2], 64))) return rc;
+    if ((rc = unit(1, l1[2], 64, H1, W1, H1, W1, l1[3], nullptr, IN_APPLY_RELU, nullptr, 0, 0, l1[4], 64))) return rc;
+    if ((rc = unit(2, l1[4], 64, H1, W1, H1, W1, l1[5], nullptr, IN_APPLY_RES, l1[2], 64, 0, l1[6], 64))) return rc;
+    if ((rc = unit(3, l1[6], 64, H1, W1, H1, W1, l1[7], nullptr, IN_APPLY_RELU, nullptr, 0, 0, l1[8], 64))) return rc;
+    if ((rc = unit(4, l1[8], 64, H1, W1, H1, W1, l1[9], nullptr, IN_APPLY_RES, l1[6], 64, 0, l1[10], 64))) return rc;
+    // 147: layer2; its first block's downsample is the second accumulator of its stride-2 convolution, normalised in
+    // the apply of the block's second convolution
+    if ((rc = unit(5, l1[10], 64, H1, W1, H2, W2, l2[0], l2[1], IN_APPLY_RELU, nullptr, 0, 0, l2[2], 128))) return rc;
+    if ((rc = unit(6, l2[2], 128, H2, W2, H2, W2, l2[3], nullptr, IN_APPLY_DS, l2[1], 128, 5, l2[4], 128))) return rc;
+    if ((rc = unit(7, l2[4], 128, H2, W2, H2, W2, l2[5], nullptr, IN_APPLY_RELU, nullptr, 0, 0, l2[6], 128))) return rc;
+    if ((rc = unit(8, l2[6], 128, H2, W2, H2, W2, l2[7], nullptr, IN_APPLY_RES, l2[4], 128, 0, l2[8], 128))) return rc;
+    // 148: layer3
+    if ((rc = unit(9, l2[8], 128, H2, W2, H3, W3, l3[0], l3[1], IN_APPLY_RELU, nullptr, 0, 0, l3[2], 128))) return rc;
+    if ((rc = unit(10, l3[2], 128, H3, W3, H3, W3, l3[3], nullptr, IN_APPLY_DS, l3[1], 128, 9, l3[4], 128))) return rc;
+    if ((rc = unit(11, l3[4], 128, H3, W3, H3, W3, l3[5], nullptr, IN_APPLY_RELU, nullptr, 0, 0, l3[6], 128))) return rc;
+    if ((rc = unit(12, l3[6], 128, H3, W3, H3, W3, l3[7], nullptr, IN_APPLY_RES, l3[4], 128, 0, last, last_ps))) return rc;
+    if (trunk) return RDVC_OK;
+    // 150: conv, the context encoder's 1x1 instantiation
+    return run_context_unit(CE_UNITS[13], rdvc::TAP_EPI_RAW, l3[8], 128, B, H3, W3, H3, W3, op_dtype, wp, bp, out,
+                            out_pixel_stride, out_dtype, nullptr, nullptr, 0, st);
 }
 
 }  // extern "C"

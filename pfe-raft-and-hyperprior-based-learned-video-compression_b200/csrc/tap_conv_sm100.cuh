@@ -1,8 +1,10 @@
 // tap_conv_sm100.cuh -- the tcgen05 tap-convolution engine behind RAFT's recurrent block (ConvGRU, TV:raft.py:214-270),
-// motion encoder and flow head (TV:raft.py:171-211, 272-285) and context encoder (FeatureEncoder with frozen BatchNorm,
-// TV:raft.py:116-168): implicit GEMMs over NHWC 16-bit activations, one kernel with the tap geometry G and the
-// epilogue EPI as template parameters.  The CUDA-core helpers of those modules (convflow1, the fp32 -> 16-bit operand
-// cast, the stem's polyphase pack) are at the end of this file.
+// motion encoder and flow head (TV:raft.py:171-211, 272-285), context encoder (FeatureEncoder with frozen BatchNorm,
+// TV:raft.py:116-168) and feature encoder (the same with InstanceNorm): implicit GEMMs over NHWC 16-bit activations,
+// one pipeline with the tap geometry G and the epilogue EPI as template parameters, entered through tap_conv_kernel or,
+// for the InstanceNorm statistics epilogues, tap_conv_in_kernel.  The CUDA-core helpers of those modules (convflow1,
+// the fp32 -> 16-bit operand cast, the stem's polyphase pack) are at the end of this file; the feature encoder's
+// finalize and apply kernels are in instance_norm_sm100.cuh.
 //
 // Tile.  16 x 8 pixels of the activation map's x and y (M = 128 GEMM rows, row m = pixel (m % 16, m / 16)).  A map is
 // 4-D {C, x, y, B} with the caller's pixel stride, so a channel slice of a channels_last tensor is read in place; one
@@ -67,6 +69,15 @@ constexpr int TAP_EPI_RELU_FLOW = 5;  // relu(acc + bias); channels N-2, N-1 are
 constexpr int TAP_EPI_FLOW2 = 6;      // acc + bias, channels 0-1 -> OutT planes (B, 2, H, W)
 constexpr int TAP_EPI_GRU_ZR = 7;     // N = 256: z = sigmoid(acc + bias) -> out, r * h = sigmoid(acc' + bias_r) * h -> out2
 constexpr int TAP_EPI_GRU_Q = 8;      // N = 128: h' = (1 - z) h + z tanh(acc + bias) -> out (OutT)
+// InstanceNorm statistics epilogues (tap_conv_in_kernel; OutT = OpT).  The conv bias is not added: InstanceNorm
+// subtracts each (sample, channel)'s mean, so a per-channel constant cancels exactly, IN(y + b) = IN(y), and without it
+// the stored values are smaller and rounded more finely.  Per tile and channel the kernel writes (mean, M2 about that
+// mean) of the values AS STORED (rounded to OpT) over the tile's pixels inside the image to part[tile * NT + c]; the
+// 4 lane-quarter warps of a tile merge theirs through shared memory (Chan).  No atomics and no per-CTA sums: a tile
+// never spans images and its partials do not depend on which CTA ran it, so a sample's statistics do not depend on
+// the batch it is in.
+constexpr int TAP_EPI_STATS = 9;      // acc -> out (OpT, out_ps)
+constexpr int TAP_EPI_DS_STATS = 10;  // columns 0..N-1: acc -> out; N..2N-1 (the fused downsample): acc -> out2 (out_ps)
 
 // ConvGRU: hidden = context = motion channels; z, r*h and h' are dense 128-channel NHWC
 constexpr int GRU_C = 128;
@@ -94,6 +105,7 @@ struct TapParams {
     const void* z;              // GRU_Q: z (OpT)
     const float* flow;          // RELU_FLOW: fp32 flow at flow[b * fs_b + c * fs_c + y * fs_y + x * fs_x]
     long long fs_b, fs_c, fs_y, fs_x;
+    float2* part;               // STATS / DS_STATS: per-tile (mean, M2) partials [n_tiles][NT]
 };
 
 template <int G> struct TapGeom;
@@ -159,7 +171,9 @@ template <int NM> struct TapMaps {
 
 template <int G, int N, int EPI>
 struct TapCfg {
-    static constexpr int NT = EPI == TAP_EPI_DS ? 2 * N : N;                // accumulator columns per tile
+    static constexpr bool HAS_DS = EPI == TAP_EPI_DS || EPI == TAP_EPI_DS_STATS;   // fused stride-2 downsample
+    static constexpr bool STATS = EPI == TAP_EPI_STATS || EPI == TAP_EPI_DS_STATS;
+    static constexpr int NT = HAS_DS ? 2 * N : N;                           // accumulator columns per tile
     static constexpr int W_STAGES = EPI == TAP_EPI_GRU_ZR ? 3 : 4;          // z|r: 3 x 32 KB next to its 48 KB A stages
     static constexpr int BOX_BYTES = TAP_TX * TapGeom<G>::BOX_Y * 128;
     static constexpr int W_BYTES = N * 128;
@@ -167,7 +181,9 @@ struct TapCfg {
     static constexpr int SMEM_A = 0;
     static constexpr int SMEM_W = TAP_A_STAGES * A_BYTES;
     static constexpr int SMEM_BAR = SMEM_W + W_STAGES * W_BYTES;
-    static constexpr int SMEM_TOTAL = SMEM_BAR + 256;
+    static constexpr int SMEM_SCR = SMEM_BAR + 256;                         // STATS: per tile [4 warps][NT] (mean, M2)
+    static constexpr int SCR_TILE_BYTES = STATS ? 4 * NT * 8 : 0;
+    static constexpr int SMEM_TOTAL = SMEM_SCR + TAP_P * SCR_TILE_BYTES;
     static constexpr int SMEM_LAUNCH = SMEM_TOTAL + 1024;                   // slack for 1024-byte alignment
     static constexpr int TMEM_COLS = TAP_P * NT <= 32 ? 32 : TAP_P * NT <= 64 ? 64 : TAP_P * NT <= 128 ? 128
                                    : TAP_P * NT <= 256 ? 256 : 512;
@@ -175,7 +191,7 @@ struct TapCfg {
     static_assert(BOX_BYTES % 1024 == 0, "boxes must start on swizzle atoms");
     static_assert(SMEM_LAUNCH <= 227 * 1024, "shared memory");
     static_assert(TAP_P * NT <= 512, "tensor memory");
-    static_assert(EPI != TAP_EPI_DS || G == TAP_G_S2, "the fused downsample rides on the stride-2 centre tap");
+    static_assert(!HAS_DS || G == TAP_G_S2, "the fused downsample rides on the stride-2 centre tap");
     static_assert((EPI != TAP_EPI_GRU_ZR && EPI != TAP_EPI_GRU_Q) || G == TAP_G_GRU5, "GRU epilogues");
 };
 
@@ -355,16 +371,98 @@ __device__ __forceinline__ void tap_epilogue(const TapParams& p, uint32_t taddr,
     }
 }
 
-// G: TAP_G_*; N: GEMM width (output channels padded to a multiple of 16); EPI: TAP_EPI_*; OutT: output dtype (GRU
-// epilogues: the dtype of h and h'); OpT: 16-bit operand dtype.  All maps 128-byte swizzled.
+template <typename OpT>
+__device__ __forceinline__ float tap_round(float v) {
+    if constexpr (std::is_same<OpT, __half>::value) return __half2float(__float2half_rn(v));
+    else return __bfloat162float(__float2bfloat16_rn(v));
+}
+
+// 16 values per lane -> lane l returns the warp's sum of value (l >> 1) & 15.  A halving exchange (16 shuffles instead
+// of 80) in a fixed order, so the sums are the same on every run.
+__device__ __forceinline__ float warp_sum16(float* v, int lane) {
+#pragma unroll
+    for (int o = 16, h = 8; o >= 2; o >>= 1, h >>= 1) {
+        const bool hi = (lane & o) != 0;
+#pragma unroll
+        for (int i = 0; i < h; ++i) {
+            const float send = hi ? v[i] : v[i + h];
+            const float keep = hi ? v[i + h] : v[i];
+            v[i] = keep + __shfl_xor_sync(0xffffffffu, send, o);
+        }
+    }
+    return v[0] + __shfl_xor_sync(0xffffffffu, v[0], 1);
+}
+
+__device__ __forceinline__ void tap_named_sync(int id, int threads) {
+    asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(threads) : "memory");
+}
+
+// STATS / DS_STATS epilogue of one tile (tile < n_tiles) at (x0, y0): store acc rounded to OpT, then per channel the
+// tile's (mean, M2) of the stored values over its pixels inside the image.  Each warp reduces its 32 pixels (lane-
+// quarter q = tile rows 2q and 2q + 1) about its own mean; the 4 warps merge in order through scr ([4][NT] float2).
+template <int N, int NT, typename OpT>
+__device__ __forceinline__ void tap_stats_epilogue(const TapParams& p, uint32_t taddr, long long pix, bool ok, int tile,
+                                                   int x0, int y0, int q, int lane, int bar_id, float2* scr) {
+    const float n_w = static_cast<float>(__popc(__ballot_sync(0xffffffffu, ok)));
+#pragma unroll 1
+    for (int c = 0; c < NT; c += 16) {
+        float v[16], s[16];
+        ptx::tmem_ld_x16(taddr + c, v);
+        ptx::tmem_ld_wait();
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {
+            v[i] = ok ? tap_round<OpT>(v[i]) : 0.f;
+            s[i] = v[i];
+        }
+        if (ok) {
+            OpT* o = c < N ? static_cast<OpT*>(p.out) + pix * p.out_ps + c
+                           : static_cast<OpT*>(p.out2) + pix * p.out_ps + (c - N);
+            GruVec<OpT>::store(o, v);
+        }
+        const float mean = n_w > 0.f ? warp_sum16(s, lane) / n_w : 0.f;
+#pragma unroll
+        for (int i = 0; i < 16; ++i) {      // every lane shuffles (a full-mask shuffle under `ok` would never complete)
+            const float m = __shfl_sync(0xffffffffu, mean, 2 * i);
+            const float d = ok ? v[i] - m : 0.f;
+            s[i] = d * d;
+        }
+        const float m2 = warp_sum16(s, lane);
+        if ((lane & 1) == 0) scr[q * NT + c + (lane >> 1)] = make_float2(mean, m2);
+    }
+    tap_named_sync(bar_id, 128);
+    const float nx = static_cast<float>(min(TAP_TX, p.W - x0));
+#pragma unroll 1
+    for (int c = q * 32 + lane; c < NT; c += 128) {
+        float n = 0.f, mean = 0.f, m2 = 0.f;
+#pragma unroll
+        for (int w = 0; w < 4; ++w) {
+            const float nq = nx * static_cast<float>(max(0, min(2, p.H - y0 - 2 * w)));
+            if (nq == 0.f) continue;
+            const float2 a = scr[w * NT + c];
+            if (n == 0.f) {
+                n = nq; mean = a.x; m2 = a.y;
+            } else {
+                const float nn = n + nq, d = a.x - mean;
+                mean += d * (nq / nn);
+                m2 += a.y + d * d * (n * nq / nn);
+                n = nn;
+            }
+        }
+        p.part[static_cast<long long>(tile) * NT + c] = make_float2(mean, m2);
+    }
+    tap_named_sync(bar_id, 128);                         // scr is free for the next super-tile
+}
+
+// The persistent pipeline shared by tap_conv_kernel and tap_conv_in_kernel.  G: TAP_G_*; N: GEMM width (output
+// channels padded to a multiple of 16); EPI: TAP_EPI_*; OutT: output dtype (GRU epilogues: the dtype of h and h');
+// OpT: 16-bit operand dtype.  All maps 128-byte swizzled.
 template <int G, int N, int EPI, typename OutT, typename OpT>
-__global__ void __launch_bounds__(TAP_THREADS, 1)
-tap_conv_kernel(const __grid_constant__ TapMaps<TapGeom<G>::MAPS> maps, const TapParams p) {
+__device__ __forceinline__ void tap_conv_body(const TapMaps<TapGeom<G>::MAPS>& maps, const TapParams& p) {
     using Geo = TapGeom<G>;
     using Cfg = TapCfg<G, N, EPI>;
     constexpr int NT = Cfg::NT;
     constexpr int WST = Cfg::W_STAGES;
-    constexpr bool DS = (EPI == TAP_EPI_DS);
+    constexpr bool DS = Cfg::HAS_DS;
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>(
         (reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~static_cast<uintptr_t>(1023));
@@ -502,7 +600,14 @@ tap_conv_kernel(const __grid_constant__ TapMaps<TapGeom<G>::MAPS> maps, const Ta
             const uint32_t taddr = tmem_base + (static_cast<uint32_t>(q * 32) << 16) + j * NT;
             ptx::mbar_wait(bar(T_FULL), t_it & 1);
             ptx::tc_fence_after();
-            tap_epilogue<EPI, N, OutT, OpT>(p, taddr, b, x, y, pix, ok);
+            if constexpr (Cfg::STATS) {       // the duplicated last tile of an odd super-tile writes nothing
+                if (tile < p.n_tiles)
+                    tap_stats_epilogue<N, NT, OpT>(p, taddr, pix, ok, tile, x0, y0, q, lane, 1 + j,
+                                                   reinterpret_cast<float2*>(smem + Cfg::SMEM_SCR +
+                                                                             j * Cfg::SCR_TILE_BYTES));
+            } else {
+                tap_epilogue<EPI, N, OutT, OpT>(p, taddr, b, x, y, pix, ok);
+            }
             ptx::tc_fence_before();
             __syncwarp();
             if (lane == 0) ptx::mbar_arrive(bar(T_EMPTY));      // accumulators back to the MMA warp
@@ -512,6 +617,22 @@ tap_conv_kernel(const __grid_constant__ TapMaps<TapGeom<G>::MAPS> maps, const Ta
     ptx::tc_fence_before();
     __syncthreads();
     if (warp == 2) ptx::tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
+}
+
+template <int G, int N, int EPI, typename OutT, typename OpT>
+__global__ void __launch_bounds__(TAP_THREADS, 1)
+tap_conv_kernel(const __grid_constant__ TapMaps<TapGeom<G>::MAPS> maps, const TapParams p) {
+    static_assert(!TapCfg<G, N, EPI>::STATS, "the statistics epilogues run in tap_conv_in_kernel");
+    tap_conv_body<G, N, EPI, OutT, OpT>(maps, p);
+}
+
+// The InstanceNorm layers' convolutions (EPI = TAP_EPI_STATS or TAP_EPI_DS_STATS): the raw output in OpT and per-tile
+// statistics partials, normalised afterwards by in_finalize_kernel and in_apply_kernel.
+template <int G, int N, int EPI, typename OpT>
+__global__ void __launch_bounds__(TAP_THREADS, 1)
+tap_conv_in_kernel(const __grid_constant__ TapMaps<TapGeom<G>::MAPS> maps, const TapParams p) {
+    static_assert(TapCfg<G, N, EPI>::STATS, "tap_conv_in_kernel runs the statistics epilogues");
+    tap_conv_body<G, N, EPI, OpT, OpT>(maps, p);
 }
 
 // ===================== CUDA-core helpers =====================

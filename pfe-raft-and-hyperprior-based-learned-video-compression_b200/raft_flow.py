@@ -31,7 +31,9 @@ reads it in place; :class:`rc.FlowHead` reads the hidden state in place.  With :
 ``model.mask_predictor`` the mask, its softmax and the convex 8x upsampling run as one GEMM epilogue
 (``MaskPredictor.upsample_flow``), in the fused and the unfused path alike.  With :class:`rc.ContextEncoder` as
 ``model.context_encoder`` the hidden state and context come from ``ContextEncoder.forward_split``: RAFT's tanh and
-ReLU run in its last layer's epilogue, and both are channel slices of one NHWC buffer.
+ReLU run in its last layer's epilogue, and both are channel slices of one NHWC buffer.  With :class:`rc.FeatureEncoder`
+as ``model.feature_encoder`` the fused encoder tail reads ``FeatureEncoder.forward_trunk``'s layer3 output, and the
+unfused path calls the module itself.
 
 :class:`GraphedRaftFlow` replays the whole call as ONE CUDA graph per input shape.  At the reference's
 default RAFT size (368x640, R:codec_processing.py:649-650) a P-frame's ~700 kernel launches cost more
@@ -48,6 +50,7 @@ from torch import Tensor
 
 from .context_encoder import ContextEncoder
 from .corr_block import TVCorrBlock, index_pyramid
+from .feature_encoder import FeatureEncoder
 from .mask_predictor import MaskPredictor
 from .motion_encoder import MotionEncoder
 from .recurrent_block import RecurrentBlock
@@ -173,7 +176,10 @@ def _raft_flow_impl(model, enc_in: Tensor, split, image1: Tensor, num_flow_updat
 
     fe = model.feature_encoder
     if fuse_encoder_tail and _can_fuse_encoder_tail(model):
-        x = fe.layer3(fe.layer2(fe.layer1(fe.convnormrelu(enc_in))))   # TV:raft.py:145-149
+        if isinstance(fe, FeatureEncoder):      # layer3's output as a view of one NHWC buffer
+            x = fe.forward_trunk(enc_in)
+        else:
+            x = fe.layer3(fe.layer2(fe.layer1(fe.convnormrelu(enc_in))))   # TV:raft.py:145-149
         fmap1, fmap2 = split(x)                                   # 128-channel activations; fe.conv runs inside the block
         if fmap1.shape[-2:] != (h // 8, w // 8):                  # TV:raft.py:494-495
             raise ValueError("The feature encoder should downsample H and W by 8")
