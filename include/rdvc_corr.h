@@ -191,6 +191,12 @@ int rdvc_corr_lookup_conv1x1_ex(const void* pyramid, int vol_dtype, int layout, 
  * op_dtype: BF16, or F16 when the activations are fp16 (the pack keeps fp16 inputs as fp16).                        */
 int rdvc_corr_pack(const void* x1, const void* x2, int B, int D, int h, int w, int in_dtype, int vol_dtype,
                    int layout, int num_levels, void* workspace, size_t workspace_bytes, void* stream);
+/* rdvc_corr_pack on NHWC maps: pixel (b, y, x) of x1 / x2 at x + ((b * h + y) * w + x) * pixel_stride, channel stride 1
+ * (e.g. rdvc_corr_feature_encoder's RDVC_FE_OUT_TRUNK output, read in place; the two maps may be rows of one buffer).
+ * in_dtype F16 | BF16; bases 16-byte aligned; pixel_stride >= D, a multiple of 8.  Writes the same bytes as
+ * rdvc_corr_pack on the same values.                                                                                */
+int rdvc_corr_pack_nhwc(const void* x1, const void* x2, long long pixel_stride, int B, int D, int h, int w, int in_dtype,
+                        int vol_dtype, int layout, int num_levels, void* workspace, size_t workspace_bytes, void* stream);
 size_t rdvc_linear_packed_weight_bytes(int cout, int cin);
 int rdvc_linear_pack_weights(const float* weight, int cout, int cin, int dtype, void* packed_host);
 int rdvc_corr_encoder_tail(const void* ws_in, size_t ws_in_bytes, int D_in, const void* packed_w, const float* bias,
@@ -487,6 +493,75 @@ int rdvc_corr_feature_encoder(const void* image, const long long* image_strides,
                               int op_dtype, const void* packed_w, const float* biases, const double* eps, int out_form,
                               void* workspace, size_t workspace_bytes, void* out, long long out_pixel_stride,
                               int out_dtype, void* stream);
+
+/* ---- the whole RAFT call: torchvision raft_large's flow, every network on this library's kernels -------------- *
+ * The C counterpart of rc.raft_flow / rc.raft_flow_sequence with all six drop-ins (feature and context encoders,
+ * motion encoder, recurrent block, flow head, mask predictor) and TVCorrBlock: images in, flow_preds[-1] out
+ * (R:codec_processing.py:1442-1444).  Caller-owned memory, the caller's stream, no allocation, no host
+ * synchronisation: a call can be captured into a CUDA graph.  All arguments are checked before the first launch; a
+ * refused call enqueues nothing.
+ *
+ * Weights (HOST, no GPU needed).  rdvc_corr_raft_pack_weights takes raft_large's state_dict(): n (name, contiguous fp32
+ * tensor, ndim, shape) entries in any order, the context encoder's BatchNorm buffers included (num_batches_tracked is
+ * ignored; BatchNorm and InstanceNorm eps are torchvision's 1e-5).  A missing key, a wrong shape (RDVC_E_SHAPE), an
+ * unexpected or duplicate key (RDVC_E_UNSUPPORTED: raft_small's state dict is refused this way) names the key in
+ * rdvc_corr_last_error().  op_dtype: RDVC_DT_F16, the operand type of both activation dtypes.  The blob,
+ * rdvc_corr_raft_packed_weight_bytes(op_dtype) long: a header { uint32 magic 0x54464152 ("RAFT"), uint32 version 1, int32
+ * op_dtype, int32 RDVC_RAFT_SECTIONS, uint64 offset[RDVC_RAFT_SECTIONS], uint64 bytes[RDVC_RAFT_SECTIONS] }, then the
+ * sections, each at a 256-byte aligned offset, written ONLY by the existing pack functions (biases used as they are
+ * are fp32 copies), in this order:
+ *    0, 1  feature encoder: rdvc_corr_context_encoder_pack_weights with the identity norm (weights, biases)
+ *    2, 3  context encoder: the same with its BatchNorm folded (weights, biases)
+ *    4, 5  feature_encoder.conv: rdvc_linear_pack_weights (256, 128), bias
+ *    6, 7  motion_encoder.convcorr1: rdvc_conv1x1_pack_weights (256, 4 levels, radius 4), bias
+ *    8-11  motion_encoder convcorr2, convflow1, convflow2, conv: rdvc_corr_update_conv_pack_weights;  12-15 their biases
+ *   16, 17 flow_head conv1, conv2 (update-conv packing);  18, 19 their biases
+ *   20, 21 recurrent_block convgru1, convgru2: rdvc_corr_convgru_pack_weights;  22-27 biases z, r, q of convgru1, then 2
+ *   28, 29 mask_predictor convrelu (FH_CONV1 packing), conv (rdvc_corr_mask_conv_pack_weights);  30, 31 their biases
+ *          (31: the permuted bias_host of the mask-conv pack)
+ * Copy the blob to the device (cudaMemcpy / cudaMemcpyAsync) at a 256-byte aligned address.
+ *
+ * rdvc_corr_raft_flow: image1, image2 DEVICE (B, 3, H, W) in_dtype (F32 | F16 | BF16) at image[b * s[0] + c * s[1] + y * s[2]
+ *   + x * s[3]], s = image_strides (4 HOST long longs, elements, >= 0, shared by both images).  flow_out: DEVICE
+ *   (B, 2, H, W) contiguous fp32, 16-byte aligned.
+ * rdvc_corr_raft_flow_sequence: frames (n_frames, 3, H, W) at frame_strides: the n_frames - 1 consecutive pairs (frame i,
+ *   frame i + 1); the feature encoder sees each frame once and pair i reads its trunk rows i and i + 1 in place.
+ *   flow_out: (n_frames - 1, 2, H, W).  Bit-identical to rdvc_corr_raft_flow on the same pairs.
+ * Both: H, W multiples of 8 with H / 8, W / 8 >= 16 (RDVC_E_SHAPE / RDVC_E_TOO_SMALL), iters >= 1 (RDVC_E_SHAPE).
+ *   act_dtype F32 (torch's eager fp32) or F16 (fp16 autocast); the operands are fp16 either way, the hidden state,
+ *   context and motion features are act_dtype.  vol_dtype F32 | BF16 (the pyramid).  mask_multiplier: the mask
+ *   predictor's (0.25 for raft_large).  packed_weights / workspace 256-byte aligned; workspace_bytes >=
+ *   rdvc_corr_raft_workspace_bytes(2 B, B, ...) for rdvc_corr_raft_flow, (n_frames, n_frames - 1, ...) for the sequence.
+ *   Images, workspace and flow_out must not overlap.
+ * rdvc_corr_raft_workspace_bytes(n_images, n_pairs, ...): 0 for invalid arguments (n_pairs < n_images <= 2 n_pairs).
+ *   Layout, every buffer at a 256-byte aligned offset, (h, w) = (H, W) / 8, P = n_pairs * h * w pixels:
+ *     persistent: the pyramid (rdvc_corr_pyramid_bytes(n_pairs, h, w, 4, vol_dtype, RDVC_LAYOUT_TILED): the bulk,
+ *       5.7 GB per 1080p pair with an fp32 volume); the context encoder's split output (P x 256 act_dtype: tanh hidden
+ *       state | relu context); coords1 and flow (each (n_pairs, 2, h, w) fp32);
+ *     then one scratch region, reused by three phases whose buffers are dead before the next starts:
+ *       1. the trunk (n_images x h x w x 128 fp16, NHWC), then the feature encoder's workspace (for n_images) or,
+ *          at the same offset, the encoder tail's input and output rows (rdvc_corr_workspace_bytes for D = 128, 256);
+ *       2. the context encoder's workspace;
+ *       3. the K-major lookup features (rdvc_corr_feat_bytes), convcorr1's output (P x 256 fp16), the motion features,
+ *          convgru1's output and the hidden state (P x 128 act_dtype each), and one workspace shared by the motion
+ *          encoder, the ConvGRU, the flow head and the mask predictor (the largest of theirs).
+ * Order: feature encoder (trunk) -> rdvc_corr_pack_nhwc -> rdvc_corr_encoder_tail -> rdvc_corr_build_packed -> context
+ *   encoder (RDVC_CE_OUT_SPLIT) -> coords1 = grid, flow = 0 (one kernel) -> iters x [lookup + convcorr1 (NHWC) ->
+ *   motion encoder -> convgru1 -> convgru2 -> flow head, whose conv2 epilogue rounds delta to act_dtype, adds it to
+ *   coords1 in fp32 and writes flow = coords1 - grid] -> mask predictor + convex upsampling into flow_out.
+ * Launches per call (rdvc_corr_launch_count): 40 x (2 for rdvc_corr_raft_flow, 1 for the sequence) + 3 + 15 + 1
+ *   + iters x (12 for F16, 15 for F32) + (2 for F16, 3 for F32).  Deterministic: no atomics anywhere on the path. */
+#define RDVC_RAFT_SECTIONS 32
+size_t rdvc_corr_raft_packed_weight_bytes(int op_dtype);
+int rdvc_corr_raft_pack_weights(const char* const* names, const float* const* tensors, const int* ndims,
+                           const long long* const* shapes, int n, int op_dtype, void* packed_host, size_t bytes);
+size_t rdvc_corr_raft_workspace_bytes(int n_images, int n_pairs, int H, int W, int act_dtype, int vol_dtype);
+int rdvc_corr_raft_flow(const void* image1, const void* image2, const long long* image_strides, int in_dtype, int B, int H,
+                   int W, int iters, int act_dtype, int vol_dtype, const void* packed_weights, float mask_multiplier,
+                   void* workspace, size_t workspace_bytes, float* flow_out, void* stream);
+int rdvc_corr_raft_flow_sequence(const void* frames, const long long* frame_strides, int in_dtype, int n_frames, int H, int W,
+                            int iters, int act_dtype, int vol_dtype, const void* packed_weights, float mask_multiplier,
+                            void* workspace, size_t workspace_bytes, float* flow_out, void* stream);
 
 /* ---- next row f-4 (last piece): entropy-coder stand-in (HOST functions) ---- *
  * Stands in for the range coder behind EntropyBottleneck.compress / .decompress (R:codec_processing.py:433,447

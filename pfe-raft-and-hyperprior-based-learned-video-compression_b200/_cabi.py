@@ -19,6 +19,7 @@ RDVC_UC_CONVCORR2, RDVC_UC_CONVFLOW1, RDVC_UC_CONVFLOW2, RDVC_UC_CONV, RDVC_UC_F
 RDVC_MASK_OUT_UPSAMPLED, RDVC_MASK_OUT_MASK = 0, 1
 RDVC_CE_OUT_RAW, RDVC_CE_OUT_SPLIT = 0, 1
 RDVC_FE_OUT_FEATURES, RDVC_FE_OUT_TRUNK = 0, 1
+RDVC_RAFT_SECTIONS = 32
 
 RDVC_E = {
     -1: "RDVC_E_NULL", -2: "RDVC_E_SHAPE", -3: "RDVC_E_TOO_SMALL", -4: "RDVC_E_DTYPE",
@@ -122,6 +123,15 @@ SYMBOLS = {
     "rdvc_corr_feature_encoder": (_c.c_int, [_c.c_void_p, _c.c_void_p] + [_c.c_int] * 5 +
                                   [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_int, _c.c_void_p, _c.c_size_t,
                                    _c.c_void_p, _c.c_longlong, _c.c_int, _c.c_void_p]),
+    "rdvc_corr_pack_nhwc": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_longlong] + [_c.c_int] * 8 +
+                            [_c.c_void_p, _c.c_size_t, _c.c_void_p]),
+    "rdvc_corr_raft_packed_weight_bytes": (_c.c_size_t, [_c.c_int]),
+    "rdvc_corr_raft_pack_weights": (_c.c_int, [_c.c_void_p] * 4 + [_c.c_int, _c.c_int, _c.c_void_p, _c.c_size_t]),
+    "rdvc_corr_raft_workspace_bytes": (_c.c_size_t, [_c.c_int] * 6),
+    "rdvc_corr_raft_flow": (_c.c_int, [_c.c_void_p] * 3 + [_c.c_int] * 7 + [_c.c_void_p, _c.c_float, _c.c_void_p, _c.c_size_t,
+                                                                     _c.c_void_p, _c.c_void_p]),
+    "rdvc_corr_raft_flow_sequence": (_c.c_int, [_c.c_void_p] * 2 + [_c.c_int] * 7 + [_c.c_void_p, _c.c_float, _c.c_void_p,
+                                                                              _c.c_size_t, _c.c_void_p, _c.c_void_p]),
     "rdvc_corr_pair_host_submit": (_c.c_int, [_c.c_void_p, _c.c_void_p, _c.c_void_p, _c.c_void_p] +
                                    [_c.c_int] * 9),
     "rdvc_corr_pair_host_wait": (_c.c_int, [_c.c_int]),

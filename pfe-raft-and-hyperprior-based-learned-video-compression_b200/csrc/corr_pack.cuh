@@ -32,6 +32,7 @@ struct PackParams {
     int img[2][4];               // [map][level]: operand rows per batch item (pixels incl. layout padding)
     int f16;                     // operand format: 0 = bf16, 1 = fp16 (fp16 inputs keep their 11-bit mantissa)
     int B, D, h, w;
+    long long ps;                // NHWC sources: pixel stride in elements (a multiple of 8, 16-byte aligned bases)
 };
 
 template <typename T> __device__ __forceinline__ float pack_to_float(T v);
@@ -73,11 +74,13 @@ __device__ __forceinline__ uint32_t pack_pair(float a, float b, int f16) {
 
 // grid: (D/64 * ceil(w/32), ceil(h/8), 2 * B); block: 256 threads; dynamic smem: PACK_SMEM_BYTES.
 // VEC: w % 4 == 0, rows can be fetched as 16-byte vectors.
+// NHWC: the sources are NHWC 16-bit maps, pixel (b, y, x) at src + ((b * h + y) * w + x) * ps (the feature encoder's
+// trunk, read in place); 16-byte loads of 8 channels, 8 lanes per pixel.  Same tile, same stores, same rows.
 // QUICK: the layout is raster order or 4-row tiles 4 / 8 pixels wide (the defaults), so a warp's region maps onto
 // whole layout tiles and pixel addresses are compile-time offsets from one base per level; !QUICK keeps the general
 // per-pixel formula for other (experimental) tile shapes.  Two instantiations instead of a run-time choice: the
 // general formula inlined 43 times made the kernel 4096 instructions long.
-template <typename T, bool QUICK, bool VEC>
+template <typename T, bool QUICK, bool VEC, bool NHWC = false>
 __global__ void __launch_bounds__(PACK_THREADS)
 corr_pack_kernel(const __grid_constant__ PackParams p) {
     extern __shared__ float tile[];  // [64][257], column = yy * 32 + xx
@@ -90,15 +93,40 @@ corr_pack_kernel(const __grid_constant__ PackParams p) {
     const int map = blockIdx.z / p.B;
     const int y0 = blockIdx.y * PACK_TY, x0 = (blockIdx.x / cgn) * PACK_TX;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    const T* src = static_cast<const T*>(p.src[map]) +
-                   (static_cast<size_t>(b) * D + static_cast<size_t>(cg) * PACK_CG) * h * w;
+    const T* src = NHWC ? static_cast<const T*>(p.src[map]) + static_cast<size_t>(cg) * PACK_CG
+                        : static_cast<const T*>(p.src[map]) +
+                              (static_cast<size_t>(b) * D + static_cast<size_t>(cg) * PACK_CG) * h * w;
 
     // load.  Vector path (w % 4 == 0): one warp instruction fetches 4 pixels per lane for 4
     // consecutive channels at one row (4 x 128 B of fp32), PACK_MLP of them in flight per
     // thread before the first is consumed; the 4 channels land 257 floats apart, so the four
     // scalar smem stores are conflict-free.  Scalar path: one 32-pixel row per instruction.
     constexpr int NWARP = PACK_THREADS / 32, PACK_MLP = 8;
-    if constexpr (VEC) {   // w % 4 == 0, chosen by the host: the two load loops are separate instantiations
+    if constexpr (NHWC) {
+        static_assert(sizeof(T) == 2, "NHWC sources are 16-bit");
+        constexpr int CHUNKS = PACK_TY * PACK_TX * (PACK_CG / 8);   // 16-byte pieces: 8 per pixel
+        static_assert(CHUNKS % (PACK_THREADS * PACK_MLP) == 0, "load loop shape");
+        for (int i0 = threadIdx.x; i0 < CHUNKS; i0 += PACK_THREADS * PACK_MLP) {
+            uint4 v[PACK_MLP];
+#pragma unroll
+            for (int u = 0; u < PACK_MLP; ++u) {
+                const int i = i0 + u * PACK_THREADS, q = i >> 3;
+                const int y = y0 + q / PACK_TX, x = x0 + q % PACK_TX;
+                v[u] = make_uint4(0, 0, 0, 0);
+                if (y < h && x < w)
+                    v[u] = __ldg(reinterpret_cast<const uint4*>(
+                        src + ((static_cast<size_t>(b) * h + y) * w + x) * static_cast<size_t>(p.ps) + (i & 7) * 8));
+            }
+#pragma unroll
+            for (int u = 0; u < PACK_MLP; ++u) {
+                const int i = i0 + u * PACK_THREADS, q = i >> 3;
+                const T* e = reinterpret_cast<const T*>(&v[u]);
+                float* t = tile + (i & 7) * 8 * PACK_PITCH + q;
+#pragma unroll
+                for (int k = 0; k < 8; ++k) t[k * PACK_PITCH] = pack_to_float<T>(e[k]);
+            }
+        }
+    } else if constexpr (VEC) {   // w % 4 == 0, chosen by the host: the two load loops are separate instantiations
         constexpr int ROWS4 = PACK_CG * PACK_TY / 4;   // 128 four-channel row groups
         static_assert(ROWS4 % (NWARP * PACK_MLP) == 0, "load loop shape");
         const int cl = lane >> 3, xq = (lane & 7) * 4;

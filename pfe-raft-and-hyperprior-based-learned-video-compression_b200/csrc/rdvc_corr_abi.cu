@@ -10,7 +10,9 @@
 #include <cstdarg>
 #include <cstdio>
 #include <cstring>
+#include <algorithm>
 #include <mutex>
+#include <string>
 #include <vector>
 
 #include "../../include/rdvc_corr.h"
@@ -30,6 +32,7 @@
 #include "mcn_convx_sm100.cuh"
 #include "motion_warp.cuh"
 #include "preprocess.cuh"
+#include "raft_flow.cuh"
 
 #ifndef RDVC_PAIR_DEFAULT
 #define RDVC_PAIR_DEFAULT 0   // the CTA-pair build kernel is opt-in (option key 12 = 2) until it wins
@@ -276,10 +279,11 @@ int launch_build_pair(const CUtensorMap& ta, const CUtensorMap* tb, const CUtens
 #endif
 
 // both feature maps -> K-major bf16 rows (fmap2 at `levels2` pyramid levels), one launch
-template <typename T, bool QUICK, bool VEC>
+template <typename T, bool QUICK, bool VEC, bool NHWC = false>
 int launch_pack_impl(const void* f1, const void* f2, void* a_km, void* const* b_km, int B, int D, int h, int w,
-                int levels2, int layout, int twl, int thl, const size_t* nl_of, int f16, cudaStream_t st) {
-    auto kern = rdvc::corr_pack_kernel<T, QUICK, VEC>;
+                int levels2, int layout, int twl, int thl, const size_t* nl_of, int f16, cudaStream_t st,
+                long long ps = 0) {
+    auto kern = rdvc::corr_pack_kernel<T, QUICK, VEC, NHWC>;
     static std::atomic<unsigned long long> attr_done{0};
     if (int rc = ensure_dynamic_smem(kern, rdvc::PACK_SMEM_BYTES, attr_done, "cudaFuncSetAttribute(pack, max dynamic smem)"))
         return rc;
@@ -293,6 +297,7 @@ int launch_pack_impl(const void* f1, const void* f2, void* a_km, void* const* b_
     pp.tiled[0] = 0; pp.tiled[1] = (layout == RDVC_LAYOUT_TILED);
     pp.twl = twl; pp.thl = thl;
     pp.f16 = f16;
+    pp.ps = ps;
     pp.img[0][0] = h * w;
     for (int l = 0; l < 4; ++l) pp.img[1][l] = static_cast<int>(nl_of[l]);
     dim3 grid((D / rdvc::PACK_CG) * ((w + rdvc::PACK_TX - 1) / rdvc::PACK_TX), (h + rdvc::PACK_TY - 1) / rdvc::PACK_TY,
@@ -318,6 +323,18 @@ int launch_pack(const void* f1, const void* f2, void* a_km, void* const* b_km, i
     if (quick) return launch_pack_impl<T, true, false>(f1, f2, a_km, b_km, B, D, h, w, levels2, layout, twl, thl, nl_of, f16, st);
     if (vec) return launch_pack_impl<T, false, true>(f1, f2, a_km, b_km, B, D, h, w, levels2, layout, twl, thl, nl_of, f16, st);
     return launch_pack_impl<T, false, false>(f1, f2, a_km, b_km, B, D, h, w, levels2, layout, twl, thl, nl_of, f16, st);
+}
+
+// the same rows from NHWC 16-bit maps at pixel stride ps (elements)
+template <typename T>
+int launch_pack_nhwc(const void* f1, const void* f2, long long ps, void* a_km, void* const* b_km, int B, int D, int h,
+                     int w, int levels2, int layout, int twl, int thl, const size_t* nl_of, int f16, cudaStream_t st) {
+    const bool quick = (layout != RDVC_LAYOUT_TILED) || (thl == 2 && (twl == 2 || twl == 3));
+    if (quick)
+        return launch_pack_impl<T, true, false, true>(f1, f2, a_km, b_km, B, D, h, w, levels2, layout, twl, thl, nl_of, f16,
+                                                      st, ps);
+    return launch_pack_impl<T, false, false, true>(f1, f2, a_km, b_km, B, D, h, w, levels2, layout, twl, thl, nl_of, f16,
+                                                   st, ps);
 }
 
 // row-major kernels: KIND 0 / 1 = scalar / 128-bit loads
@@ -880,8 +897,12 @@ int rdvc_corr_build_packed(int B, int D, int h, int w, int op_dtype, void* pyram
                       workspace_bytes, stream);
 }
 
-int rdvc_corr_pack(const void* x1, const void* x2, int B, int D, int h, int w, int in_dtype, int vol_dtype,
-                   int layout, int num_levels, void* workspace, size_t workspace_bytes, void* stream) {
+}  // extern "C"
+
+namespace {
+// pixel_stride 0: NCHW maps (rdvc_corr_pack); > 0: NHWC 16-bit maps at that pixel stride (rdvc_corr_pack_nhwc)
+int pack_impl(const void* x1, const void* x2, long long pixel_stride, int B, int D, int h, int w, int in_dtype,
+              int vol_dtype, int layout, int num_levels, void* workspace, size_t workspace_bytes, void* stream) {
     if (!x1 || !x2 || !workspace) return fail(RDVC_E_NULL, "null pointer argument");
     int rc = check_geometry(B, h, w, num_levels);
     if (rc) return rc;
@@ -896,6 +917,12 @@ int rdvc_corr_pack(const void* x1, const void* x2, int B, int D, int h, int w, i
     if (workspace_bytes < rdvc_corr_workspace_bytes(B, D, h, w))
         return fail(RDVC_E_WORKSPACE, "workspace %zu < required %zu", workspace_bytes, rdvc_corr_workspace_bytes(B, D, h, w));
     if (reinterpret_cast<uintptr_t>(workspace) & 255) return fail(RDVC_E_ALIGN, "workspace must be 256-byte aligned");
+    if (pixel_stride) {
+        if (in_dtype == RDVC_DT_F32) return fail(RDVC_E_DTYPE, "NHWC maps are F16 or BF16, got in_dtype=%d", in_dtype);
+        if (pixel_stride < D) return fail(RDVC_E_UNSUPPORTED, "pixel_stride %lld < D=%d", pixel_stride, D);
+        if ((pixel_stride % 8) || ((reinterpret_cast<uintptr_t>(x1) | reinterpret_cast<uintptr_t>(x2)) & 15))
+            return fail(RDVC_E_ALIGN, "NHWC maps need 16-byte aligned bases and a pixel stride of a multiple of 8");
+    }
     cudaStream_t st = static_cast<cudaStream_t>(stream);
     WorkspaceLayout wl;
     workspace_layout(workspace, B, D, h, w, vol_dtype, layout, num_levels, &wl);
@@ -904,9 +931,29 @@ int rdvc_corr_pack(const void* x1, const void* x2, int B, int D, int h, int w, i
         if (e != cudaSuccess) return cuda_fail(e, "cudaMemsetAsync(padded operand rows)");
     }
     const int f16 = (in_dtype == RDVC_DT_F16) ? 1 : 0;
+    if (pixel_stride)
+        return f16 ? launch_pack_nhwc<__half>(x1, x2, pixel_stride, wl.a_km, wl.b_km, B, D, h, w, num_levels, layout, wl.twl,
+                                              wl.thl, wl.nl_of, f16, st)
+                   : launch_pack_nhwc<__nv_bfloat16>(x1, x2, pixel_stride, wl.a_km, wl.b_km, B, D, h, w, num_levels, layout,
+                                                     wl.twl, wl.thl, wl.nl_of, f16, st);
     if (in_dtype == RDVC_DT_F32) return launch_pack<float>(x1, x2, wl.a_km, wl.b_km, B, D, h, w, num_levels, layout, wl.twl, wl.thl, wl.nl_of, f16, st);
     if (in_dtype == RDVC_DT_BF16) return launch_pack<__nv_bfloat16>(x1, x2, wl.a_km, wl.b_km, B, D, h, w, num_levels, layout, wl.twl, wl.thl, wl.nl_of, f16, st);
     return launch_pack<__half>(x1, x2, wl.a_km, wl.b_km, B, D, h, w, num_levels, layout, wl.twl, wl.thl, wl.nl_of, f16, st);
+}
+}  // namespace
+
+extern "C" {
+
+int rdvc_corr_pack(const void* x1, const void* x2, int B, int D, int h, int w, int in_dtype, int vol_dtype,
+                   int layout, int num_levels, void* workspace, size_t workspace_bytes, void* stream) {
+    return pack_impl(x1, x2, 0, B, D, h, w, in_dtype, vol_dtype, layout, num_levels, workspace, workspace_bytes, stream);
+}
+
+int rdvc_corr_pack_nhwc(const void* x1, const void* x2, long long pixel_stride, int B, int D, int h, int w, int in_dtype,
+                        int vol_dtype, int layout, int num_levels, void* workspace, size_t workspace_bytes, void* stream) {
+    if (pixel_stride <= 0) return fail(RDVC_E_UNSUPPORTED, "pixel_stride must be positive, got %lld", pixel_stride);
+    return pack_impl(x1, x2, pixel_stride, B, D, h, w, in_dtype, vol_dtype, layout, num_levels, workspace, workspace_bytes,
+                     stream);
 }
 
 size_t rdvc_linear_packed_weight_bytes(int cout, int cin) {
@@ -1963,6 +2010,31 @@ int hidden_operand(const void** h, long long* ps, int act_dtype, int op_dtype, l
     return RDVC_OK;
 }
 
+// one 3x3 layer on the tap-convolution engine, arguments checked by the caller.  out2: FH_CONV2's coordinate update
+// (out = coords1, out2 = flow, fp32 (B, 2, H, W); out_dtype is the dtype delta is rounded to), else NULL.
+int launch_update_conv(int layer, const void* in, long long in_pixel_stride, const float* flow,
+                       const long long* flow_strides, int B, int H, int W, int op_dtype, const void* packed_w,
+                       const float* bias, void* out, long long out_pixel_stride, int out_dtype, void* out2,
+                       cudaStream_t st) {
+    const UcLayer& L = UC_LAYERS[layer];
+    const CUtensorMapDataType dt = op_map_dtype(op_dtype);
+    rdvc::TapMaps<1> m;
+    if (int rc = act_map(&m.a[0], dt, in, in_pixel_stride, L.cin, B, H, W, rdvc::TAP_TX,
+                         rdvc::TapGeom<rdvc::TAP_G_S1>::BOX_Y))
+        return rc;
+    if (int rc = slab_map(&m.w, dt, packed_w, L.n, L.cin / 64 * 9)) return rc;
+    rdvc::TapParams p = tap_params(B, H, W, L.cin / 64);
+    p.bias = bias; p.cout = L.cout;
+    p.out = out; p.out_ps = out_pixel_stride;
+    p.out2 = out2;
+    if (flow) {
+        p.flow = flow;
+        p.fs_b = flow_strides[0]; p.fs_c = flow_strides[1]; p.fs_y = flow_strides[2]; p.fs_x = flow_strides[3];
+    }
+    return op_dtype == RDVC_DT_F16 ? dispatch_update_conv<__half>(layer, out_dtype, m, p, st)
+                                   : dispatch_update_conv<__nv_bfloat16>(layer, out_dtype, m, p, st);
+}
+
 }  // namespace
 
 extern "C" {
@@ -2037,21 +2109,8 @@ int rdvc_corr_update_conv(int layer, const void* in, long long in_pixel_stride, 
         p.B = B; p.H = H; p.W = W; p.n_pix = n_pix;
         return op_dtype == RDVC_DT_F16 ? launch_convflow1<__half>(p, st) : launch_convflow1<__nv_bfloat16>(p, st);
     }
-    const CUtensorMapDataType dt = op_map_dtype(op_dtype);
-    rdvc::TapMaps<1> m;
-    if (int rc = act_map(&m.a[0], dt, in, in_pixel_stride, L.cin, B, H, W, rdvc::TAP_TX,
-                         rdvc::TapGeom<rdvc::TAP_G_S1>::BOX_Y))
-        return rc;
-    if (int rc = slab_map(&m.w, dt, packed_w, L.n, L.cin / 64 * 9)) return rc;
-    rdvc::TapParams p = tap_params(B, H, W, L.cin / 64);
-    p.bias = bias; p.cout = L.cout;
-    p.out = out; p.out_ps = out_pixel_stride;
-    if (uses_flow) {
-        p.flow = flow;
-        p.fs_b = flow_strides[0]; p.fs_c = flow_strides[1]; p.fs_y = flow_strides[2]; p.fs_x = flow_strides[3];
-    }
-    return op_dtype == RDVC_DT_F16 ? dispatch_update_conv<__half>(layer, out_dtype, m, p, st)
-                                   : dispatch_update_conv<__nv_bfloat16>(layer, out_dtype, m, p, st);
+    return launch_update_conv(layer, in, in_pixel_stride, uses_flow ? flow : nullptr, flow_strides, B, H, W, op_dtype,
+                              packed_w, bias, out, out_pixel_stride, out_dtype, nullptr, st);
 }
 
 size_t rdvc_corr_motion_encoder_workspace_bytes(int B, int H, int W) {
@@ -2790,6 +2849,455 @@ int rdvc_corr_feature_encoder(const void* image, const long long* image_strides,
     // 150: conv, the context encoder's 1x1 instantiation
     return run_context_unit(CE_UNITS[13], rdvc::TAP_EPI_RAW, l3[8], 128, B, H3, W3, H3, W3, op_dtype, wp, bp, out,
                             out_pixel_stride, out_dtype, nullptr, nullptr, 0, st);
+}
+
+}  // extern "C"
+
+// ---- the whole RAFT call: every network on the library's kernels, caller-owned memory, no allocation ------------
+namespace {
+
+constexpr int RAFT_LEVELS = 4, RAFT_RADIUS = 4;
+constexpr uint32_t RAFT_MAGIC = 0x54464152u;     // "RAFT", little-endian
+constexpr uint32_t RAFT_BLOB_VERSION = 1;
+constexpr double RAFT_NORM_EPS = 1e-5;            // torchvision's BatchNorm2d / InstanceNorm2d default
+
+// sections of the packed blob, in blob order (include/rdvc_corr.h)
+enum {
+    RS_FE_W, RS_FE_B, RS_CE_W, RS_CE_B, RS_TAIL_W, RS_TAIL_B, RS_CC1_W, RS_CC1_B,
+    RS_ME_W, RS_ME_B = RS_ME_W + 4, RS_FH_W = RS_ME_B + 4, RS_FH_B = RS_FH_W + 2, RS_GRU_W = RS_FH_B + 2,
+    RS_GRU_B = RS_GRU_W + 2, RS_MASK_W = RS_GRU_B + 6, RS_MASK_B = RS_MASK_W + 2, RS_COUNT = RS_MASK_B + 2
+};
+static_assert(RS_COUNT == RDVC_RAFT_SECTIONS, "section count of include/rdvc_corr.h");
+
+struct RaftBlobHeader {
+    uint32_t magic, version;
+    int32_t op_dtype, sections;
+    uint64_t offset[RS_COUNT], bytes[RS_COUNT];
+};
+
+constexpr int ME_LAYERS[4] = {RDVC_UC_CONVCORR2, RDVC_UC_CONVFLOW1, RDVC_UC_CONVFLOW2, RDVC_UC_CONV};
+
+size_t raft_sections(uint64_t* off, uint64_t* bytes) {
+    uint64_t b[RS_COUNT];
+    b[RS_FE_W] = b[RS_CE_W] = rdvc_corr_context_encoder_packed_weight_bytes();
+    b[RS_FE_B] = b[RS_CE_B] = rdvc_corr_context_encoder_packed_bias_bytes();
+    b[RS_TAIL_W] = rdvc_linear_packed_weight_bytes(rdvc::ET_N, rdvc::ET_K);
+    b[RS_TAIL_B] = rdvc::ET_N * 4;
+    b[RS_CC1_W] = rdvc_conv1x1_packed_weight_bytes(256, RAFT_LEVELS, RAFT_RADIUS);
+    b[RS_CC1_B] = 256 * 4;
+    for (int i = 0; i < 4; ++i) {
+        b[RS_ME_W + i] = rdvc_corr_update_conv_packed_weight_bytes(ME_LAYERS[i]);
+        b[RS_ME_B + i] = UC_LAYERS[ME_LAYERS[i]].cout * 4;
+    }
+    b[RS_FH_W] = rdvc_corr_update_conv_packed_weight_bytes(RDVC_UC_FH_CONV1);
+    b[RS_FH_W + 1] = rdvc_corr_update_conv_packed_weight_bytes(RDVC_UC_FH_CONV2);
+    b[RS_FH_B] = 256 * 4;
+    b[RS_FH_B + 1] = 2 * 4;
+    b[RS_GRU_W] = b[RS_GRU_W + 1] = rdvc_corr_convgru_packed_weight_bytes();
+    for (int i = 0; i < 6; ++i) b[RS_GRU_B + i] = rdvc::GRU_C * 4;
+    b[RS_MASK_W] = rdvc_corr_update_conv_packed_weight_bytes(RDVC_UC_FH_CONV1);
+    b[RS_MASK_W + 1] = rdvc_corr_mask_conv_packed_weight_bytes();
+    b[RS_MASK_B] = 256 * 4;
+    b[RS_MASK_B + 1] = rdvc::MU_COUT * 4;
+    size_t o = align_up(sizeof(RaftBlobHeader), 256);
+    for (int i = 0; i < RS_COUNT; ++i) {
+        if (off) off[i] = o;
+        if (bytes) bytes[i] = b[i];
+        o = align_up(o + b[i], 256);
+    }
+    return o;
+}
+
+// state_dict keys of torchvision's raft_large and where each one goes
+enum RaftKind { RK_IGNORE, RK_FE_W, RK_FE_B, RK_CE_W, RK_CE_B, RK_BN_W, RK_BN_B, RK_BN_M, RK_BN_V, RK_GRU_W, RK_SECTION };
+struct RaftKey {
+    std::string name;
+    std::vector<long long> shape;
+    int kind, index;              // RK_*; index: encoder layer, 3 * ConvGRU + (z, r, q), or the section of a lone tensor
+};
+
+const std::vector<RaftKey>& raft_keys() {
+    static const std::vector<RaftKey> keys = [] {
+        std::vector<RaftKey> k;
+        // the encoders' 16 convolutions in the order of the context-encoder pack arrays: (module, cout, cin, kernel)
+        struct Conv { const char* name; int cout, cin, ks; };
+        static const Conv enc[RDVC_CE_LAYERS] = {
+            {"convnormrelu", 64, 3, 7},
+            {"layer1.0.convnormrelu1", 64, 64, 3}, {"layer1.0.convnormrelu2", 64, 64, 3},
+            {"layer1.1.convnormrelu1", 64, 64, 3}, {"layer1.1.convnormrelu2", 64, 64, 3},
+            {"layer2.0.convnormrelu1", 96, 64, 3}, {"layer2.0.downsample", 96, 64, 1},
+            {"layer2.0.convnormrelu2", 96, 96, 3}, {"layer2.1.convnormrelu1", 96, 96, 3},
+            {"layer2.1.convnormrelu2", 96, 96, 3},
+            {"layer3.0.convnormrelu1", 128, 96, 3}, {"layer3.0.downsample", 128, 96, 1},
+            {"layer3.0.convnormrelu2", 128, 128, 3}, {"layer3.1.convnormrelu1", 128, 128, 3},
+            {"layer3.1.convnormrelu2", 128, 128, 3},
+            {"conv", 256, 128, 1},
+        };
+        for (int e = 0; e < 2; ++e) {
+            const std::string pre = e == 0 ? "feature_encoder." : "context_encoder.";
+            for (int i = 0; i < RDVC_CE_LAYERS; ++i) {
+                const Conv& c = enc[i];
+                const std::string conv = pre + c.name + (i < RDVC_CE_LAYERS - 1 ? ".0" : "");
+                k.push_back({conv + ".weight", {c.cout, c.cin, c.ks, c.ks}, e ? RK_CE_W : RK_FE_W, i});
+                k.push_back({conv + ".bias", {c.cout}, e ? RK_CE_B : RK_FE_B, i});
+                if (e == 1 && i < RDVC_CE_LAYERS - 1) {
+                    const std::string bn = pre + c.name + ".1";
+                    k.push_back({bn + ".weight", {c.cout}, RK_BN_W, i});
+                    k.push_back({bn + ".bias", {c.cout}, RK_BN_B, i});
+                    k.push_back({bn + ".running_mean", {c.cout}, RK_BN_M, i});
+                    k.push_back({bn + ".running_var", {c.cout}, RK_BN_V, i});
+                    k.push_back({bn + ".num_batches_tracked", {}, RK_IGNORE, i});
+                }
+            }
+        }
+        // single tensors, each packed into (weights) or copied to (biases) one section
+        auto conv = [&](const std::string& name, int cout, int cin, int kh, int kw, int w_section, int b_section,
+                        int w_kind = RK_SECTION) {
+            k.push_back({name + ".weight", {cout, cin, kh, kw}, w_kind, w_section});
+            k.push_back({name + ".bias", {cout}, RK_SECTION, b_section});
+        };
+        const std::string me = "update_block.motion_encoder.";
+        conv(me + "convcorr1.0", 256, RAFT_LEVELS * (2 * RAFT_RADIUS + 1) * (2 * RAFT_RADIUS + 1), 1, 1, RS_CC1_W, RS_CC1_B);
+        const char* me_names[4] = {"convcorr2.0", "convflow1.0", "convflow2.0", "conv.0"};
+        for (int i = 0; i < 4; ++i) {
+            const UcLayer& L = UC_LAYERS[ME_LAYERS[i]];
+            conv(me + me_names[i], L.cout, L.cin, L.k, L.k, RS_ME_W + i, RS_ME_B + i);
+        }
+        for (int g = 0; g < 2; ++g)
+            for (int q = 0; q < 3; ++q) {
+                const std::string name = std::string("update_block.recurrent_block.convgru") + (g ? "2" : "1") + ".conv" + "zrq"[q];
+                conv(name, rdvc::GRU_C, 3 * rdvc::GRU_C, g ? 5 : 1, g ? 1 : 5, 3 * g + q, RS_GRU_B + 3 * g + q, RK_GRU_W);
+            }
+        conv("update_block.flow_head.conv1", 256, 128, 3, 3, RS_FH_W, RS_FH_B);
+        conv("update_block.flow_head.conv2", 2, 256, 3, 3, RS_FH_W + 1, RS_FH_B + 1);
+        conv("mask_predictor.convrelu.0", 256, 128, 3, 3, RS_MASK_W, RS_MASK_B);
+        conv("mask_predictor.conv", rdvc::MU_COUT, rdvc::MU_CIN, 1, 1, RS_MASK_W + 1, RS_MASK_B + 1);
+        return k;
+    }();
+    return keys;
+}
+
+std::string shape_str(const long long* s, int nd) {
+    std::string r = "(";
+    for (int i = 0; i < nd; ++i) r += std::to_string(s[i]) + (i + 1 < nd ? ", " : nd == 1 ? "," : "");
+    return r + ")";
+}
+
+// the workspace: persistent buffers first, then one scratch region shared by the three phases (encoders, context
+// encoder, refinement loop), whose buffers' lifetimes do not overlap
+struct RaftLayout {
+    size_t pyr, hc, coords, flow, scratch;
+    size_t trunk, enc_ws, tail_in, tail_out;          // phase 1: feature encoder, pack, encoder tail, build
+    size_t ce_ws;                                     // phase 2: context encoder
+    size_t feat, c1, motion, g1, hid, loop_ws;        // phase 3: the iterations and the mask predictor
+    size_t total;
+};
+
+RaftLayout raft_layout(int n_images, int B, int H, int W, int act_dtype, int vol_dtype) {
+    RaftLayout L;
+    memset(&L, 0, sizeof(L));
+    const int h = H / 8, w = W / 8;
+    const size_t px = static_cast<size_t>(B) * h * w, aes = elem_size(act_dtype);
+    size_t o = 0;
+    auto take = [&](size_t bytes) { const size_t at = o; o = align_up(o + bytes, 256); return at; };
+    L.pyr = take(rdvc_corr_pyramid_bytes(B, h, w, RAFT_LEVELS, vol_dtype, RDVC_LAYOUT_TILED));
+    L.hc = take(px * 256 * aes);
+    L.coords = take(px * 2 * 4);
+    L.flow = take(px * 2 * 4);
+    L.scratch = o;
+    L.trunk = take(static_cast<size_t>(n_images) * h * w * rdvc::ET_K * 2);
+    const size_t after_trunk = o;
+    L.enc_ws = take(rdvc_corr_feature_encoder_workspace_bytes(n_images, H, W, act_dtype));
+    size_t end1 = o;
+    o = after_trunk;
+    L.tail_in = take(rdvc_corr_workspace_bytes(B, rdvc::ET_K, h, w));
+    L.tail_out = take(rdvc_corr_workspace_bytes(B, rdvc::ET_N, h, w));
+    end1 = std::max(end1, o);
+    o = L.scratch;
+    L.ce_ws = take(rdvc_corr_context_encoder_workspace_bytes(B, H, W, act_dtype));
+    const size_t end2 = o;
+    o = L.scratch;
+    L.feat = take(rdvc_corr_feat_bytes(B, h, w, RAFT_LEVELS, RAFT_RADIUS));
+    L.c1 = take(px * 256 * 2);
+    L.motion = take(px * 128 * aes);
+    L.g1 = take(px * rdvc::GRU_C * aes);
+    L.hid = take(px * rdvc::GRU_C * aes);
+    L.loop_ws = take(std::max(std::max(rdvc_corr_convgru_workspace_bytes(B, h, w, act_dtype),
+                                       rdvc_corr_motion_encoder_workspace_bytes(B, h, w)),
+                              std::max(rdvc_corr_flow_head_workspace_bytes(B, h, w, act_dtype),
+                                       rdvc_corr_mask_predictor_workspace_bytes(B, h, w, act_dtype))));
+    L.total = std::max(std::max(end1, end2), o);
+    return L;
+}
+
+int raft_check_sizes(int n_images, int B, int H, int W, int act_dtype, int vol_dtype) {
+    if (B <= 0 || H <= 0 || W <= 0 || n_images <= B || n_images > 2 * B)
+        return fail(RDVC_E_SHAPE, "bad sizes: %d images, %d pairs, H=%d W=%d", n_images, B, H, W);
+    if (H % 8 || W % 8) return fail(RDVC_E_SHAPE, "input image H and W should be divisible by 8, got H=%d W=%d", H, W);
+    const int min_fmap = 2 << (RAFT_LEVELS - 1);
+    if (H / 8 < min_fmap || W / 8 < min_fmap)
+        return fail(RDVC_E_TOO_SMALL, "feature maps %d x %d are under %d per side: H and W must be at least %d", H / 8, W / 8,
+                    min_fmap, 8 * min_fmap);
+    if (act_dtype != RDVC_DT_F32 && act_dtype != RDVC_DT_F16)
+        return fail(RDVC_E_DTYPE, "act_dtype must be F32 or F16, got %d", act_dtype);
+    if (vol_dtype != RDVC_DT_F32 && vol_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "vol_dtype must be F32 or BF16, got %d", vol_dtype);
+    if (H >= (1 << 24) || W >= (1 << 24) || static_cast<long long>(n_images) * H * W >= (1LL << 31))
+        return fail(RDVC_E_UNSUPPORTED, "too many pixels for 32-bit TMA coordinates");
+    return RDVC_OK;
+}
+
+// one call of either form: the feature encoder sees `images` (one run of n_images frames, or image1 then image2),
+// pair b is (trunk row b, trunk row b + pair_offset)
+int raft_run(const void* image1, const void* image2, const long long* s, int in_dtype, int n_images, int B, int H, int W,
+             int iters, int act_dtype, int vol_dtype, const void* packed_weights, float mask_multiplier, void* workspace,
+             size_t workspace_bytes, float* flow_out, void* stream) {
+    if (!image1 || !s || !packed_weights || !workspace || !flow_out) return fail(RDVC_E_NULL, "null pointer argument");
+    if (int rc = raft_check_sizes(n_images, B, H, W, act_dtype, vol_dtype)) return rc;
+    if (iters < 1) return fail(RDVC_E_SHAPE, "iters must be >= 1, got %d", iters);
+    if (in_dtype != RDVC_DT_F32 && in_dtype != RDVC_DT_F16 && in_dtype != RDVC_DT_BF16)
+        return fail(RDVC_E_DTYPE, "unsupported in_dtype=%d", in_dtype);
+    for (int i = 0; i < 4; ++i)
+        if (s[i] < 0) return fail(RDVC_E_UNSUPPORTED, "negative image stride %lld", s[i]);
+    const size_t in_es = elem_size(in_dtype);
+    if ((reinterpret_cast<uintptr_t>(image1) % in_es) || (reinterpret_cast<uintptr_t>(image2) % in_es))
+        return fail(RDVC_E_ALIGN, "the images must be aligned to their element size");
+    if ((reinterpret_cast<uintptr_t>(packed_weights) & 255) || (reinterpret_cast<uintptr_t>(workspace) & 255) ||
+        (reinterpret_cast<uintptr_t>(flow_out) & 15))
+        return fail(RDVC_E_ALIGN, "packed weights and workspace must be 256-byte aligned, flow_out 16-byte aligned");
+    const RaftLayout L = raft_layout(n_images, B, H, W, act_dtype, vol_dtype);
+    if (workspace_bytes < L.total) return fail(RDVC_E_WORKSPACE, "workspace %zu < required %zu", workspace_bytes, L.total);
+    const long long n_in = image2 ? B : n_images;      // images per feature-encoder call
+    const long long dims[4] = {n_in, 3, H, W};
+    size_t img_elems = 1;
+    for (int i = 0; i < 4; ++i) img_elems += static_cast<size_t>(dims[i] - 1) * static_cast<size_t>(s[i]);
+    const size_t out_bytes = static_cast<size_t>(B) * 2 * H * W * 4;
+    const void* imgs[2] = {image1, image2};
+    for (const void* im : imgs)
+        if (im && (ranges_overlap(im, img_elems * in_es, workspace, L.total) ||
+                   ranges_overlap(im, img_elems * in_es, flow_out, out_bytes)))
+            return fail(RDVC_E_UNSUPPORTED, "an image overlaps the workspace or flow_out");
+    if (ranges_overlap(flow_out, out_bytes, workspace, L.total))
+        return fail(RDVC_E_UNSUPPORTED, "flow_out overlaps the workspace");
+
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    const int h = H / 8, w = W / 8, op = RDVC_DT_F16;
+    const long long hw = static_cast<long long>(h) * w;
+    uint8_t* ws = static_cast<uint8_t*>(workspace);
+    const uint8_t* pk = static_cast<const uint8_t*>(packed_weights);
+    uint64_t off[RS_COUNT];
+    raft_sections(off, nullptr);
+    auto sec = [&](int i) { return static_cast<const void*>(pk + off[i]); };
+    auto fsec = [&](int i) { return reinterpret_cast<const float*>(pk + off[i]); };
+    void* pyr = ws + L.pyr;
+    uint8_t* hc = ws + L.hc;
+    float* coords = reinterpret_cast<float*>(ws + L.coords);
+    float* flow = reinterpret_cast<float*>(ws + L.flow);
+    __half* trunk = reinterpret_cast<__half*>(ws + L.trunk);
+    const size_t enc_ws_bytes = rdvc_corr_feature_encoder_workspace_bytes(n_images, H, W, act_dtype);
+    const size_t tail_in_bytes = rdvc_corr_workspace_bytes(B, rdvc::ET_K, h, w);
+    const size_t tail_out_bytes = rdvc_corr_workspace_bytes(B, rdvc::ET_N, h, w);
+    double eps[RDVC_FE_NORMS];
+    for (double& e : eps) e = RAFT_NORM_EPS;
+
+    // 1. feature encoder -> layer3's trunk, NHWC fp16; the encoder tail (pack + 1x1 GEMM) and the build on it
+    for (int i = 0; i < (image2 ? 2 : 1); ++i)
+        if (int rc = rdvc_corr_feature_encoder(imgs[i], s, in_dtype, static_cast<int>(n_in), H, W, op, sec(RS_FE_W),
+                                               fsec(RS_FE_B), eps, RDVC_FE_OUT_TRUNK, ws + L.enc_ws, enc_ws_bytes,
+                                               trunk + i * n_in * hw * rdvc::ET_K, rdvc::ET_K, op, stream))
+            return rc;
+    const long long pair_offset = (image2 ? B : 1) * hw * rdvc::ET_K;
+    if (int rc = rdvc_corr_pack_nhwc(trunk, trunk + pair_offset, rdvc::ET_K, B, rdvc::ET_K, h, w, op, vol_dtype,
+                                     RDVC_LAYOUT_TILED, RAFT_LEVELS, ws + L.tail_in, tail_in_bytes, stream))
+        return rc;
+    if (int rc = rdvc_corr_encoder_tail(ws + L.tail_in, tail_in_bytes, rdvc::ET_K, sec(RS_TAIL_W), fsec(RS_TAIL_B),
+                                        rdvc::ET_N, B, h, w, op, vol_dtype, RDVC_LAYOUT_TILED, RAFT_LEVELS, ws + L.tail_out,
+                                        tail_out_bytes, stream))
+        return rc;
+    if (int rc = rdvc_corr_build_packed(B, rdvc::ET_N, h, w, op, pyr, vol_dtype, RDVC_LAYOUT_TILED, RAFT_LEVELS,
+                                        ws + L.tail_out, tail_out_bytes, stream))
+        return rc;
+    // 2. context encoder: tanh(hidden) | relu(context), one NHWC buffer in the activation dtype
+    if (int rc = rdvc_corr_context_encoder(image1, s, in_dtype, B, H, W, op, sec(RS_CE_W), fsec(RS_CE_B), RDVC_CE_OUT_SPLIT,
+                                           ws + L.ce_ws, rdvc_corr_context_encoder_workspace_bytes(B, H, W, act_dtype), hc,
+                                           256, act_dtype, stream))
+        return rc;
+    // 3. coords1 = grid, flow = 0; then the iterations
+    {
+        const long long n = B * hw;
+        const unsigned grid = static_cast<unsigned>(std::min<long long>((n + 255) / 256, 4LL * sm_count()));
+        rdvc::raft_coords_init_kernel<<<grid, 256, 0, st>>>(coords, flow, B, h, w);
+        ++g_launches;
+        cudaError_t e = cudaGetLastError();
+        if (e != cudaSuccess) return cuda_fail(e, "raft_coords_init_kernel launch");
+    }
+    const long long fs[4] = {2 * hw, hw, w, 1};
+    const size_t aes = elem_size(act_dtype);
+    const void* me_w[4] = {sec(RS_ME_W), sec(RS_ME_W + 1), sec(RS_ME_W + 2), sec(RS_ME_W + 3)};
+    const float* me_b[4] = {fsec(RS_ME_B), fsec(RS_ME_B + 1), fsec(RS_ME_B + 2), fsec(RS_ME_B + 3)};
+    void* loop_ws = ws + L.loop_ws;
+    const size_t loop_ws_bytes = L.total - L.loop_ws;
+    const void* ctx = hc + 128 * aes;
+    void* hid = ws + L.hid;
+    const void* hcur = hc;                               // iteration 0: the hidden half of the context encoder's output
+    long long hps = 256;
+    for (int it = 0; it < iters; ++it) {
+        if (int rc = rdvc_corr_lookup_conv1x1_ex(pyr, vol_dtype, RDVC_LAYOUT_TILED, coords, B, h, w, RAFT_LEVELS, RAFT_RADIUS,
+                                                 sec(RS_CC1_W), fsec(RS_CC1_B), 256, RDVC_ACT_RELU, op, ws + L.feat,
+                                                 rdvc_corr_feat_bytes(B, h, w, RAFT_LEVELS, RAFT_RADIUS), ws + L.c1, op,
+                                                 256, stream))
+            return rc;
+        if (int rc = rdvc_corr_motion_encoder(ws + L.c1, 256, flow, fs, B, h, w, op, me_w, me_b, loop_ws, loop_ws_bytes,
+                                              ws + L.motion, 128, act_dtype, stream))
+            return rc;
+        for (int g = 0; g < 2; ++g)      // convgru1 (1 x 5) -> g1, convgru2 (5 x 1) -> hid
+            if (int rc = rdvc_corr_convgru(g ? ws + L.g1 : hcur, g ? 128 : hps, ctx, 256, ws + L.motion, 128, act_dtype, op,
+                                           g ? RDVC_GRU_VERTICAL : RDVC_GRU_HORIZONTAL, B, h, w, sec(RS_GRU_W + g),
+                                           fsec(RS_GRU_B + 3 * g), fsec(RS_GRU_B + 3 * g + 1), fsec(RS_GRU_B + 3 * g + 2),
+                                           loop_ws, loop_ws_bytes, g ? hid : ws + L.g1, stream))
+                return rc;
+        hcur = hid;
+        hps = 128;
+        // flow head; its conv2 epilogue adds delta (rounded to act_dtype) to coords1 and writes flow = coords1 - grid
+        const void* h16 = hid;
+        long long h16_ps = 128;
+        uint8_t* fh = static_cast<uint8_t*>(loop_ws);
+        if (int rc = hidden_operand(&h16, &h16_ps, act_dtype, op, B * hw, fh + uc_plane_bytes(B, h, w, 256), stream))
+            return rc;
+        if (int rc = rdvc_corr_update_conv(RDVC_UC_FH_CONV1, h16, h16_ps, nullptr, nullptr, B, h, w, op, sec(RS_FH_W),
+                                           fsec(RS_FH_B), fh, 256, op, stream))
+            return rc;
+        if (int rc = launch_update_conv(RDVC_UC_FH_CONV2, fh, 256, nullptr, nullptr, B, h, w, op, sec(RS_FH_W + 1),
+                                        fsec(RS_FH_B + 1), coords, 0, act_dtype, flow, st))
+            return rc;
+    }
+    // 4. mask predictor + convex 8x upsampling of the last flow, straight into flow_out
+    const void* mw[2] = {sec(RS_MASK_W), sec(RS_MASK_W + 1)};
+    const float* mb[2] = {fsec(RS_MASK_B), fsec(RS_MASK_B + 1)};
+    return rdvc_corr_mask_predictor(hid, 128, act_dtype, B, h, w, op, mw, mb, mask_multiplier, flow, fs,
+                                    RDVC_MASK_OUT_UPSAMPLED, loop_ws, loop_ws_bytes, flow_out, stream);
+}
+
+}  // namespace
+
+extern "C" {
+
+size_t rdvc_corr_raft_packed_weight_bytes(int op_dtype) {
+    return op_dtype == RDVC_DT_F16 ? raft_sections(nullptr, nullptr) : 0;
+}
+
+int rdvc_corr_raft_pack_weights(const char* const* names, const float* const* tensors, const int* ndims,
+                           const long long* const* shapes, int n, int op_dtype, void* packed_host, size_t bytes) {
+    if (!names || !tensors || !ndims || !shapes || !packed_host) return fail(RDVC_E_NULL, "null pointer argument");
+    if (op_dtype != RDVC_DT_F16)
+        return fail(RDVC_E_DTYPE, "op_dtype must be F16 (the operand type of both activation dtypes), got %d", op_dtype);
+    if (n < 0) return fail(RDVC_E_SHAPE, "negative tensor count %d", n);
+    uint64_t off[RS_COUNT], sz[RS_COUNT];
+    const size_t need = raft_sections(off, sz);
+    if (bytes < need) return fail(RDVC_E_WORKSPACE, "packed_host holds %zu bytes < required %zu", bytes, need);
+    const std::vector<RaftKey>& keys = raft_keys();
+    std::vector<const float*> found(keys.size(), nullptr);
+    for (int i = 0; i < n; ++i) {
+        if (!names[i]) return fail(RDVC_E_NULL, "names[%d] is NULL", i);
+        size_t k = 0;
+        while (k < keys.size() && keys[k].name != names[i]) ++k;
+        if (k == keys.size()) return fail(RDVC_E_UNSUPPORTED, "unexpected key %s (not in raft_large's state_dict)", names[i]);
+        const RaftKey& key = keys[k];
+        if (key.kind == RK_IGNORE) continue;
+        if (found[k]) return fail(RDVC_E_UNSUPPORTED, "duplicate key %s", names[i]);
+        if (!tensors[i] || (ndims[i] > 0 && !shapes[i])) return fail(RDVC_E_NULL, "key %s: NULL tensor or shape", names[i]);
+        const int nd = static_cast<int>(key.shape.size());
+        bool same = ndims[i] == nd;
+        for (int d = 0; same && d < nd; ++d) same = shapes[i][d] == key.shape[d];
+        if (!same)
+            return fail(RDVC_E_SHAPE, "key %s has shape %s, raft_large's is %s", names[i],
+                        shape_str(ndims[i] > 0 ? shapes[i] : nullptr, std::max(ndims[i], 0)).c_str(),
+                        shape_str(key.shape.data(), nd).c_str());
+        found[k] = tensors[i];
+    }
+    const float* fe_w[RDVC_CE_LAYERS] = {}; const float* fe_b[RDVC_CE_LAYERS] = {};
+    const float* ce_w[RDVC_CE_LAYERS] = {}; const float* ce_b[RDVC_CE_LAYERS] = {};
+    const float* bn[4][RDVC_CE_LAYERS] = {};
+    const float* single[RS_COUNT] = {};
+    const float* gru[2][3] = {};
+    for (size_t k = 0; k < keys.size(); ++k) {
+        const RaftKey& key = keys[k];
+        if (key.kind == RK_IGNORE) continue;
+        if (!found[k]) return fail(RDVC_E_SHAPE, "missing key %s", key.name.c_str());
+        switch (key.kind) {
+            case RK_FE_W:                // feature_encoder.conv (the last layer) is also the encoder tail's weight
+                fe_w[key.index] = found[k];
+                if (key.index == RDVC_CE_LAYERS - 1) single[RS_TAIL_W] = found[k];
+                break;
+            case RK_FE_B:
+                fe_b[key.index] = found[k];
+                if (key.index == RDVC_CE_LAYERS - 1) single[RS_TAIL_B] = found[k];
+                break;
+            case RK_CE_W: ce_w[key.index] = found[k]; break;
+            case RK_CE_B: ce_b[key.index] = found[k]; break;
+            case RK_BN_W: case RK_BN_B: case RK_BN_M: case RK_BN_V: bn[key.kind - RK_BN_W][key.index] = found[k]; break;
+            case RK_GRU_W: gru[key.index / 3][key.index % 3] = found[k]; break;
+            default: single[key.index] = found[k];
+        }
+    }
+    uint8_t* blob = static_cast<uint8_t*>(packed_host);
+    memset(blob, 0, need);
+    RaftBlobHeader hdr;
+    memset(&hdr, 0, sizeof(hdr));
+    hdr.magic = RAFT_MAGIC; hdr.version = RAFT_BLOB_VERSION; hdr.op_dtype = op_dtype; hdr.sections = RS_COUNT;
+    for (int i = 0; i < RS_COUNT; ++i) { hdr.offset[i] = off[i]; hdr.bytes[i] = sz[i]; }
+    memcpy(blob, &hdr, sizeof(hdr));
+    auto fout = [&](int i) { return reinterpret_cast<float*>(blob + off[i]); };
+    // feature encoder: the context encoder's packing with the identity norm (scale exactly 1, each weight rounded once)
+    std::vector<float> ones(256, 1.f), zeros(256, 0.f);
+    const float* one[RDVC_CE_LAYERS]; const float* zero[RDVC_CE_LAYERS];
+    double eps0[RDVC_CE_LAYERS], eps[RDVC_CE_LAYERS];
+    for (int i = 0; i < RDVC_CE_LAYERS; ++i) {
+        one[i] = ones.data(); zero[i] = zeros.data();
+        eps0[i] = 0.0; eps[i] = RAFT_NORM_EPS;
+    }
+    int rc = rdvc_corr_context_encoder_pack_weights(fe_w, fe_b, one, zero, zero, one, eps0, op_dtype, blob + off[RS_FE_W],
+                                                    fout(RS_FE_B));
+    if (!rc) rc = rdvc_corr_context_encoder_pack_weights(ce_w, ce_b, bn[0], bn[1], bn[2], bn[3], eps, op_dtype,
+                                                         blob + off[RS_CE_W], fout(RS_CE_B));
+    if (!rc) rc = rdvc_linear_pack_weights(single[RS_TAIL_W], rdvc::ET_N, rdvc::ET_K, op_dtype, blob + off[RS_TAIL_W]);
+    if (!rc) rc = rdvc_conv1x1_pack_weights(single[RS_CC1_W], 256, RAFT_LEVELS, RAFT_RADIUS, op_dtype, blob + off[RS_CC1_W]);
+    for (int i = 0; i < 4 && !rc; ++i)
+        rc = rdvc_corr_update_conv_pack_weights(ME_LAYERS[i], single[RS_ME_W + i], op_dtype, blob + off[RS_ME_W + i]);
+    for (int i = 0; i < 2 && !rc; ++i)
+        rc = rdvc_corr_update_conv_pack_weights(i ? RDVC_UC_FH_CONV2 : RDVC_UC_FH_CONV1, single[RS_FH_W + i], op_dtype,
+                                                blob + off[RS_FH_W + i]);
+    for (int g = 0; g < 2 && !rc; ++g)
+        rc = rdvc_corr_convgru_pack_weights(gru[g][0], gru[g][1], gru[g][2], op_dtype, blob + off[RS_GRU_W + g]);
+    if (!rc) rc = rdvc_corr_update_conv_pack_weights(RDVC_UC_FH_CONV1, single[RS_MASK_W], op_dtype, blob + off[RS_MASK_W]);
+    if (!rc) rc = rdvc_corr_mask_conv_pack_weights(single[RS_MASK_W + 1], single[RS_MASK_B + 1], op_dtype,
+                                                   blob + off[RS_MASK_W + 1], fout(RS_MASK_B + 1));
+    if (rc) return rc;
+    // biases used as they are: fp32 copies
+    const int copies[] = {RS_TAIL_B, RS_CC1_B, RS_ME_B, RS_ME_B + 1, RS_ME_B + 2, RS_ME_B + 3, RS_FH_B, RS_FH_B + 1,
+                          RS_GRU_B, RS_GRU_B + 1, RS_GRU_B + 2, RS_GRU_B + 3, RS_GRU_B + 4, RS_GRU_B + 5, RS_MASK_B};
+    for (int i : copies) memcpy(blob + off[i], single[i], sz[i]);
+    return RDVC_OK;
+}
+
+size_t rdvc_corr_raft_workspace_bytes(int n_images, int n_pairs, int H, int W, int act_dtype, int vol_dtype) {
+    if (raft_check_sizes(n_images, n_pairs, H, W, act_dtype, vol_dtype)) return 0;     // the reason: rdvc_corr_last_error
+    return raft_layout(n_images, n_pairs, H, W, act_dtype, vol_dtype).total;
+}
+
+int rdvc_corr_raft_flow(const void* image1, const void* image2, const long long* image_strides, int in_dtype, int B, int H,
+                   int W, int iters, int act_dtype, int vol_dtype, const void* packed_weights, float mask_multiplier,
+                   void* workspace, size_t workspace_bytes, float* flow_out, void* stream) {
+    if (!image2) return fail(RDVC_E_NULL, "null pointer argument");
+    return raft_run(image1, image2, image_strides, in_dtype, 2 * B, B, H, W, iters, act_dtype, vol_dtype, packed_weights,
+                    mask_multiplier, workspace, workspace_bytes, flow_out, stream);
+}
+
+int rdvc_corr_raft_flow_sequence(const void* frames, const long long* frame_strides, int in_dtype, int n_frames, int H, int W,
+                            int iters, int act_dtype, int vol_dtype, const void* packed_weights, float mask_multiplier,
+                            void* workspace, size_t workspace_bytes, float* flow_out, void* stream) {
+    return raft_run(frames, nullptr, frame_strides, in_dtype, n_frames, n_frames - 1, H, W, iters, act_dtype, vol_dtype,
+                    packed_weights, mask_multiplier, workspace, workspace_bytes, flow_out, stream);
 }
 
 }  // extern "C"

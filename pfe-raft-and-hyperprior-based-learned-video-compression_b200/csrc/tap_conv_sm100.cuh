@@ -66,7 +66,8 @@ constexpr int TAP_EPI_DS = 2;         // columns 0..N-1: relu(acc + bias) -> out
 constexpr int TAP_EPI_RAW = 3;        // acc + bias
 constexpr int TAP_EPI_SPLIT = 4;      // tanh(acc + bias) on channels 0-127, relu(acc + bias) on the rest
 constexpr int TAP_EPI_RELU_FLOW = 5;  // relu(acc + bias); channels N-2, N-1 are the flow (fp32, strided) rounded to OutT
-constexpr int TAP_EPI_FLOW2 = 6;      // acc + bias, channels 0-1 -> OutT planes (B, 2, H, W)
+constexpr int TAP_EPI_FLOW2 = 6;      // acc + bias, channels 0-1 -> OutT planes (B, 2, H, W); with out2: the
+                                      // coordinate update (out = coords1, out2 = flow, both fp32 (B, 2, H, W))
 constexpr int TAP_EPI_GRU_ZR = 7;     // N = 256: z = sigmoid(acc + bias) -> out, r * h = sigmoid(acc' + bias_r) * h -> out2
 constexpr int TAP_EPI_GRU_Q = 8;      // N = 128: h' = (1 - z) h + z tanh(acc + bias) -> out (OutT)
 // InstanceNorm statistics epilogues (tap_conv_in_kernel; OutT = OpT).  The conv bias is not added: InstanceNorm
@@ -99,7 +100,7 @@ struct TapParams {
     int cout;                   // RELU_FLOW / FLOW2: real output channels (channel c reads bias[min(c, cout - 1)])
     void* out;                  // OutT NHWC, pixel stride out_ps; FLOW2: planes (B, 2, H, W); GRU_ZR: z (OpT); GRU_Q: h'
     long long out_ps;
-    void* out2;                 // DS: OpT NHWC, pixel stride out_ps; GRU_ZR: r * h (OpT)
+    void* out2;                 // DS: OpT NHWC, pixel stride out_ps; GRU_ZR: r * h (OpT); FLOW2: flow (fp32) or NULL
     const void* res;            // RES: OpT NHWC; GRU_*: h (OutT); pixel stride res_ps
     long long res_ps;
     const void* z;              // GRU_Q: z (OpT)
@@ -284,9 +285,22 @@ __device__ __forceinline__ void tap_epilogue(const TapParams& p, uint32_t taddr,
         ptx::tmem_ld_wait();
         if (ok) {
             const long long plane = static_cast<long long>(p.H) * p.W;
-            OutT* o = static_cast<OutT*>(p.out) + static_cast<long long>(b) * 2 * plane + (pix - b * plane);
-            o[0] = static_cast<OutT>(v[0] + __ldg(p.bias));
-            o[plane] = static_cast<OutT>(v[1] + __ldg(p.bias + min(1, p.cout - 1)));
+            const long long i = static_cast<long long>(b) * 2 * plane + (pix - b * plane);
+            const OutT d0 = static_cast<OutT>(v[0] + __ldg(p.bias));
+            const OutT d1 = static_cast<OutT>(v[1] + __ldg(p.bias + min(1, p.cout - 1)));
+            if (p.out2 == nullptr) {
+                OutT* o = static_cast<OutT*>(p.out) + i;
+                o[0] = d0;
+                o[plane] = d1;
+            } else {    // raft_flow's coords1 = coords1 + delta_flow, then flow = coords1 - coords0, in the same fp32 ops
+                float* c = static_cast<float*>(p.out) + i;
+                float* f = static_cast<float*>(p.out2) + i;
+                const float c0 = c[0] + static_cast<float>(d0), c1 = c[plane] + static_cast<float>(d1);
+                c[0] = c0;
+                c[plane] = c1;
+                f[0] = c0 - static_cast<float>(x);
+                f[plane] = c1 - static_cast<float>(y);
+            }
         }
     } else if constexpr (EPI == TAP_EPI_GRU_ZR || EPI == TAP_EPI_GRU_Q) {
         const OutT* hp = static_cast<const OutT*>(p.res) + pix * p.res_ps;
